@@ -2,6 +2,7 @@
 """bench.py -- Viterbi cells/s of the B200 hot path, one JSON line (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pos|large] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.  Default workload = BASELINE.json
 configs[2], the POS-tagging shape (K=45 tags, 20k vocab, 1M sentences, avg T=25): the batched, sharding
@@ -30,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree the bench runs from may be read-only; it writes nothing there
 
 METRIC = "viterbi_cells_per_s"
 UNIT = "cells/s"
@@ -506,7 +508,34 @@ def parse():
     ap.add_argument("--cp-sharded", default="heavy:2000", metavar="KIND:NODES",
                     help="with --gpus > 1: the constrained decode sharded over the ranks (csrc/cp_dist.cuh) next to the "
                          "single-GPU solve, e.g. heavy:2000 (configs[4], the default) or trucks:0; 'off' skips it")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the decoded scores and paths of the last step as DIR/<name>.npy "
+                         "(see dump_outputs) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_SCORES_MAX = 1 << 21      # 16 MiB of f64
+DUMP_PATHS_MAX = 1 << 22       # 16 MiB of f32
+DUMP_PATHS_SAMPLE = 1 << 21
+
+
+def dump_outputs(out_dir, paths, scores):
+    """The batch-ordered results of the last timed step (what a caller of the decode receives) as .npy files:
+    scores.npy (f64, one per sequence) and paths.npy (f32 states, one per observation).  An array larger than its cap
+    is replaced by a fixed, seeded sample at sorted positions, stored next to it as <name>_index.npy (f64); the
+    sample depends only on the array's length, so runs with the same arguments dump the same positions.  At most
+    56 MiB in all."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x, cap, n_sample, dtype in (("scores", scores, DUMP_SCORES_MAX, DUMP_SCORES_MAX, np.float64),
+                                          ("paths", paths, DUMP_PATHS_MAX, DUMP_PATHS_SAMPLE, np.float32)):
+        if len(x) > cap:
+            idx = np.sort(np.random.default_rng(3019).choice(len(x), n_sample, replace=False))
+            x = x[idx]
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
+        np.save(os.path.join(out_dir, f"{name}.npy"), x.astype(dtype))
 
 
 def build_workload(args, rank=0):
@@ -540,8 +569,10 @@ def run_reference(args, rank, world):
         po.decode_batch(wl["A"], wl["B"], ob, o, nthreads=threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        po.decode_batch(wl["A"], wl["B"], ob, o, nthreads=threads)
+        paths, scores = po.decode_batch(wl["A"], wl["B"], ob, o, nthreads=threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, paths, scores)
     v = cells * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -642,6 +673,8 @@ def main():
     full_paths = sd.paths().cpu().numpy()
     full_paths = full_paths.astype(np.uint32) if sd.narrow_paths else full_paths.view(np.uint32)
     full_scores = sd.scores().cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, full_paths, full_scores)
 
     # ---- share of the collective: the same steps without / with only the all-gather ----
     gather_ms = 0.0
