@@ -76,6 +76,8 @@ SIGNATURES = {
                                 C.c_void_p, _dp, _i64p, _dp]),
     "cv_mle": (C.c_int, [C.c_int, C.c_int, _u64p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                          C.c_void_p, C.c_int64, C.c_int, _dp]),
+    "cv_baum_welch": (C.c_int, [C.c_int, C.c_int, _u64p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_int64, C.c_int, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), _i64p, _dp]),
     "cv_last_error": (C.c_char_p, []),
     "cv_launch_count": (C.c_uint64, []),
     "cv_set_timing": (None, [C.c_int]),

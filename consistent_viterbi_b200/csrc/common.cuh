@@ -14,6 +14,10 @@ constexpr int LARGE_BN = 128;     // target states per work item of the large-K 
 
 __device__ __forceinline__ double neg_inf() { return __longlong_as_double(0xfff0000000000000LL); }
 
+// HMM::log (hmm.rs:192-205) of one probability: 0 -> -inf, else x.log(10.0) = ln(x) / ln(10).  Used by cv_mle on the
+// host and by the Baum-Welch M-step on the device.
+__host__ __device__ inline double hmm_log10(double x) { return x == 0.0 ? -INFINITY : log(x) / log(10.0); }
+
 // ---------------------------------------------------------------------------
 // One max-plus cell: v = d + a; if (v > best) { best = v; idx = j; }
 //

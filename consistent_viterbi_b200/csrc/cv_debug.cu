@@ -54,6 +54,9 @@ extern "C" int cv_debug_probe_fp64(int device, int mode, int iters, double *ops_
         } else if (mode == 1) {
             probe_fp64_kernel<1><<<blocks, threads>>>(d_out, iters, 1.0);
             fp64_ops = 32.0 * iters * threads * blocks;
+        } else if (mode == 25) {
+            probe_fp64_kernel<2><<<blocks, threads>>>(d_out, iters, 1.0);   // independent DFMA chains (Baum-Welch cell)
+            fp64_ops = 16.0 * iters * threads * blocks;                      // FMAs
         } else {
             auto launch = [&](auto kern) -> cudaError_t {
                 cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

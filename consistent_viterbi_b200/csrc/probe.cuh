@@ -67,6 +67,8 @@ __global__ void __launch_bounds__(512, 1) probe_fp64_kernel(double *out, int ite
         for (int c = 0; c < NCH; c++) {
             if constexpr (MODE == 0) {
                 acc[c] += inc;
+            } else if constexpr (MODE == 2) {
+                acc[c] = fma(acc[c], seed, inc);          // DFMA (seed = 1.0 at run time: the compiler cannot fold it)
             } else {
                 acc[c] += inc;
                 pr = pr || (acc[c] > seed);

@@ -72,6 +72,38 @@ class HMM:
         _lib.check(rc)
         return ms.value
 
+    # ---- unsupervised training: Baum-Welch (cv_baum_welch) ----
+    def train(self, sequences, n_iter: int = 10, tol: float = 0.0, device: int = -1):
+        """HMM::train's role (hmm.rs:69-190) with the semantics of cv_baum_welch (include/cv_b200.h), which this
+        library defines and does not restate from hmm.rs: Baum-Welch EM from the current model on the GPU.  Unlike
+        decoding, pi and the first observation of every sequence count.  sequences: list of [T, D] observation arrays.
+        Updates a, b, pi in place; returns what train_arrays returns."""
+        obs = [self.flatten_obs(sq) for sq in sequences]
+        off = np.zeros(len(obs) + 1, dtype=np.int64)
+        off[1:] = np.cumsum([len(o) for o in obs])
+        obs_flat = np.concatenate(obs) if obs else np.zeros(0, dtype=np.uint32)
+        return self.train_arrays(obs_flat, off, n_iter, tol, device)
+
+    def train_arrays(self, obs_flat, seq_off, n_iter: int = 10, tol: float = 0.0, device: int = -1):
+        """cv_baum_welch on flat arrays.  Returns dict(loglik = log10 P(O) before each iteration's update, summed over
+        the contributing sequences; iters = iterations run; skipped = sequences with P(O) = 0 in the last iteration;
+        device_ms)."""
+        self.close()                                                     # device copies become stale
+        obs_flat = np.ascontiguousarray(obs_flat, dtype=np.uint32)
+        seq_off = np.ascontiguousarray(seq_off, dtype=np.int64)
+        K = self.nstates()
+        b2 = np.ascontiguousarray(self.b.reshape(K, -1))
+        bd = (C.c_uint64 * len(self.bdims))(*self.bdims)
+        ll = np.zeros(max(int(n_iter), 1), dtype=np.float64)
+        iters, skipped, ms = C.c_int(0), C.c_int64(0), C.c_double(0.0)
+        rc = _lib.lib().cv_baum_welch(K, len(self.bdims), bd, self.a.ctypes.data, b2.ctypes.data, self.pi.ctypes.data,
+                                      obs_flat.ctypes.data, seq_off.ctypes.data, len(seq_off) - 1, int(n_iter),
+                                      float(tol), int(device), ll.ctypes.data_as(C.POINTER(C.c_double)),
+                                      C.byref(iters), C.byref(skipped), C.byref(ms))
+        _lib.check(rc)
+        self.b = b2.reshape(self.b.shape)
+        return dict(loglik=ll[: iters.value].copy(), iters=iters.value, skipped=skipped.value, device_ms=ms.value)
+
     # ---- reference accessors (host-side, used by SuperSequence.reorder and tests) ----
     def nstates(self) -> int:                       # hmm.rs:207-209
         return self.a.shape[0]

@@ -182,6 +182,33 @@ int cv_mle(int K, int D, const uint64_t *bdims, double *a, double *b, double *pi
            const uint32_t *obs_flat, const int32_t *tags_flat, const int64_t *seq_off,
            int64_t B, int device, double *count_ms_out);
 
+/* ---- unsupervised training: Baum-Welch (EM) ------------------------------------
+ * The counterpart of HMM::train (hmm.rs:69-190).  The semantics below are defined by this library (textbook
+ * Baum-Welch over multiple observation sequences, Rabiner 1989); they are not a restatement of hmm.rs, whose random
+ * start makes bit parity impossible anyway.  One iteration from model theta (probabilities p = 10^log10 entry):
+ *   P(O) = sum over paths of pi[s0] b[s0][o0] prod_{t>=1} a[s_{t-1}][s_t] b[s_t][o_t]   (unlike cv_decode_batch,
+ *          pi and the first observation count)
+ *   gamma_t(i) = P(s_t = i | O), xi_t(i,j) = P(s_{t-1} = i, s_t = j | O), summed over the contributing sequences:
+ *   pi'[i]   = sum gamma_0(i) / (number of contributing sequences)
+ *   a'[i][j] = sum_{t=1..T-1} xi_t(i,j) / sum_{t=0..T-2} gamma_t(i)
+ *   b'[j][m] = sum_{t: o_t = m} gamma_t(j) / sum_t gamma_t(j)
+ * A zero denominator gives a zero row; a zero is written as -inf, anything else as ln(x)/ln(10).  An entry that is
+ * -inf on entry stays -inf.  A sequence with P(O) = 0 under the current model (also: whose scaled forward sum
+ * underflows) is not a contributing sequence: it adds nothing and is counted in *skipped_out (of the last iteration).
+ * loglik_out[k] = log10 P(O | theta_k) summed over the contributing sequences, theta_k = the model BEFORE update k.
+ * Runs n_iter iterations, or stops after iteration k >= 1 (its update kept) when tol > 0 and
+ * loglik[k] - loglik[k-1] < tol * |loglik[k-1]|; *iters_out = iterations run.
+ *   logA, logB, logPi  log10 in, log10 out, in place (layouts as above)
+ *   obs_flat[N], seq_off[B+1] as for cv_decode_batch; device -1 = current device; device_ms_out may be NULL
+ * Two calls with the same inputs on the same GPU return the same bytes.  K <= 64.
+ *   CV_ERR_EMPTY an empty sequence   CV_ERR_ARG observation >= M, n_iter < 1, B < 1, bad sizes   CV_ERR_NAN NaN or
+ *   +inf in the model   CV_ERR_UNSUPPORTED K > 64   CV_ERR_CUDA no device.  HOST pointers. */
+int cv_baum_welch(int K, int D, const uint64_t *bdims, double *logA, double *logB, double *logPi,
+                  const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                  int n_iter, double tol, int device,
+                  double *loglik_out /* [n_iter] */, int *iters_out,
+                  int64_t *skipped_out /* last iteration */, double *device_ms_out /* may be NULL */);
+
 /* ---- plumbing --------------------------------------------------------------*/
 const char *cv_last_error(void);
 /* kernels launched by this library in this process (bench.py "gpu_launches") */

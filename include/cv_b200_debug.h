@@ -63,7 +63,7 @@ int cv_debug_ordered_sum(const double *values, int64_t n, int mode, double *out)
 
 /* FP64 issue-rate probe used as the ALU roofline denominator: runs `iters` dependent-free DADD (mode 0),
  * DADD+DSETP pairs (mode 1) or the decode inner loop body (mode >= 2) on every SM and returns FP64 instructions
- * per second. */
+ * per second.  Mode 25: independent DFMA chains (the Baum-Welch cell), returns FMAs per second. */
 int cv_debug_probe_fp64(int device, int mode, int iters, double *ops_per_s_out, double *ms_out);
 
 #ifdef __cplusplus
