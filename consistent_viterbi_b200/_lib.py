@@ -28,16 +28,13 @@ class CvError(RuntimeError):
         self.code = code
 
 
-def build(force: bool = False, variant: int | None = None) -> str:
+def build(force: bool = False) -> str:
     """Compile csrc/ for sm_100a with nvcc (in-tree, so the .so travels to the GPU box)."""
     srcs = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cu", ".cuh", ".inl"))]
     srcs += [os.path.join(_HERE, "..", "include", f) for f in ("cv_b200.h", "cv_b200_debug.h")]
     stale = (not os.path.exists(SO_PATH)) or any(os.path.getmtime(s) > os.path.getmtime(SO_PATH) for s in srcs)
     if force or stale:
-        cmd = ["make", "-C", CSRC, "-s", "-B", "-j4"]
-        if variant is not None:
-            cmd.append(f"VARIANT={variant}")
-        subprocess.check_call(cmd)
+        subprocess.check_call(["make", "-C", CSRC, "-s", "-B", "-j4"])
     return SO_PATH
 
 
@@ -92,7 +89,6 @@ DEBUG_SIGNATURES = {
     "cv_debug_cp_last_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "cv_debug_cp_last_ub": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, _u64p]),
     "cv_debug_ordered_sum": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _dp]),
-    "cv_debug_set_small_config": (None, [C.c_int]),
     "cv_debug_set_chunks": (None, [C.c_int]),
     "cv_debug_set_chain_max_batch": (None, [C.c_longlong]),
     "cv_debug_set_pipeline": (None, [C.c_int, C.c_int]),
@@ -102,7 +98,6 @@ DEBUG_SIGNATURES = {
     "cv_debug_set_em_light": (None, [C.c_int]),
     "cv_debug_set_bt_split": (None, [C.c_int]),
     "cv_debug_set_uneven_chunks": (None, [C.c_int]),
-    "cv_debug_set_prefilter": (None, [C.c_int]),
     "cv_debug_set_large_group_rb": (None, [C.c_longlong]),
     "cv_debug_set_cp_leaf_batch": (None, [C.c_int]),
 }

@@ -12,7 +12,6 @@
 
 #include "common.cuh"
 #include "decode_small.cuh"
-#include "decode_prefilter.cuh"
 #include "decode_f32.cuh"
 #include "decode_chain.cuh"
 #include "decode_large.cuh"
@@ -43,11 +42,8 @@ static Tuning tuning_from_env()
     Tuning t;
     auto geti = [](const char *name, int dflt) { const char *e = getenv(name); return e ? atoi(e) : dflt; };
     t.chunks = geti("CV_CHUNKS", t.chunks);
-    t.small_cfg = geti("CV_SMALL_CFG", t.small_cfg);
     t.bt_concurrent = geti("CV_BT_CONCURRENT", t.bt_concurrent);
     t.streamed = geti("CV_STREAMED", t.streamed);
-    if (const char *e = getenv("CV_TQ")) t.tq = !strcmp(e, "auto") ? 0 : (atoi(e) == 12 ? 12 : atoi(e) == 6 ? 6 : 8);
-    t.tp = geti("CV_TP", 2) == 4 ? 4 : 2;
     t.balanced_split = geti("CV_BALANCED", t.balanced_split);
     t.fwd_ldc = geti("CV_FWD_LDC", t.fwd_ldc);
     t.em_light = geti("CV_EM_LIGHT", t.em_light);
@@ -55,7 +51,6 @@ static Tuning tuning_from_env()
     t.uneven_chunks = geti("CV_UNEVEN_CHUNKS", t.uneven_chunks);
     t.long_split = geti("CV_LONG_SPLIT", t.long_split);
     t.long_pct = geti("CV_LONG_PCT", t.long_pct);
-    t.prefilter = geti("CV_PREFILTER", t.prefilter);
     t.debug = getenv("CV_DEBUG") != nullptr;
     t.bt_prof = getenv("CV_BT_PROF") != nullptr;
     t.e2e_prof = getenv("CV_E2E_PROF") != nullptr;
@@ -65,7 +60,6 @@ static Tuning tuning_from_env()
     t.cp_sum = geti("CV_CP_SUM", t.cp_sum);
     t.cp_hostpoll = geti("CV_CP_HOSTPOLL", t.cp_hostpoll);
     t.cp_leaf_batch = geti("CV_CP_LEAF_BATCH", t.cp_leaf_batch);
-    t.probe_threads = geti("CV_PROBE_THREADS", t.probe_threads);
     return t;
 }
 Tuning cvb::g_tune = tuning_from_env();
@@ -145,24 +139,6 @@ __global__ void build_f32_kernel(const double *in, float *out, int64_t rows, int
     }
 }
 
-// Operands of the pre-filter forward kernel (decode_prefilter.cuh) from the natural layout A [K][Kp]:
-//   A32 [Kp][Kp] f32: row = predecessor j, column = slot c -> rn32(logA[j][state(c)]), clamped to PF_NEG; padding PF_NEG
-//   A64T [Kp][Kp] f64: row = slot c, column = predecessor j -> logA[j][state(c)]; padding -inf
-// state(c) = first(g) + q for slot c = 8 g + q of the balanced split (base, rem), or c itself when base = 0.
-__global__ void build_prefilter_kernel(const double *A, int K, int Kp, int base, int rem, float *A32, double *A64T)
-{
-    const int n = Kp * Kp;
-    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < n; e += gridDim.x * blockDim.x) {
-        const int j = e / Kp, c = e % Kp, g = c >> 3, q = c & 7;
-        int st = c;
-        if (base) { const int first = g * base + min(g, rem), cnt = base + (g < rem ? 1 : 0); st = q < cnt ? first + q : -1; }
-        const bool real = j < K && st >= 0 && st < K;
-        const double v = real ? A[(size_t)j * Kp + st] : neg_inf();
-        A32[(size_t)j * Kp + c] = fmaxf(__double2float_rn(v), PF_NEG);
-        A64T[(size_t)c * Kp + j] = v;
-    }
-}
-
 extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *logA, const double *logB,
                              const double *logPi, int device, cv_hmm **out)
 {
@@ -194,28 +170,9 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     cv_hmm *h = new cv_hmm();
     struct Guard { cv_hmm *h; ~Guard() { if (h) cv_hmm_destroy(h); } } guard{h};   // released on every early return
     h->device = device; h->K = K; h->D = D; h->M = M;
-    // tile shape of the forward kernel: TQT target states per warp, G = ceil(K/TQT) state groups.  Pick the
-    // shape with the least padded work among those whose warps per CTA (G*S, S in {1,2,4}) divide by 4.
-    {
-        double best_eff = -1.0; int best_tq = 8;
-        for (int tq : {8, 12}) {
-            const int g = (K + tq - 1) / tq;
-            double eff = 0.0;
-            for (int s : {1, 2, 4}) {
-                if (g * s * 32 > 512) continue;
-                const int w = g * s;
-                const double bal = (double)w / (4.0 * ((w + 3) / 4));
-                // wide CTAs (one per SM) lose to the per-step barrier: mild penalty so that S = 1 wins ties
-                eff = std::max(eff, bal * (s == 1 ? 1.0 : 0.93) * (double)K / (g * tq));
-            }
-            if (eff > best_eff + 1e-9) { best_eff = eff; best_tq = tq; }
-        }
-        // measured on B200 (POS shape): TQ = 8 with two 6-warp CTAs per SM beats the balanced TQ = 12 shape
-        // (12 vs 8 resident warps), so 8 stays the default; CV_TQ=12 / 6 / auto select the alternatives
-        h->TQT = g_tune.tq == 0 ? best_tq : g_tune.tq;
-    }
-    h->G = (K + h->TQT - 1) / h->TQT;
-    h->Kp = ((std::max(h->G * h->TQT, K) + 7) / 8) * 8;
+    // state groups of the forward tile kernel: G = ceil(K/8) warps of TQ = 8 target states, Kp = 8 G
+    h->G = (K + TQ - 1) / TQ;
+    h->Kp = h->G * TQ;
     h->hA.assign(logA, logA + (size_t)K * K);
     h->hB.assign(logB, logB + (size_t)K * M);
     h->hPi.assign(logPi, logPi + K);
@@ -263,7 +220,7 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     if (K <= SMALL_K_MAX) { h->dA = pA; h->dBT = pBT; h->dPi = pPi; }
     else { h->dAl = pA; h->dBTl = pBT; h->dPi = pPi; }
     pA = pBT = pPi = nullptr;                      // owned by the handle now (cv_hmm_destroy)
-    if (K <= SMALL_K_MAX && h->TQT == 8 && K % 8 != 0 && K / h->G >= 5) {
+    if (K <= SMALL_K_MAX && K % 8 != 0 && K / h->G >= 5) {
         // balanced state split of the forward tile kernel: no padded target states (K = 45: 8,8,8,7,7,7 instead of 5 x 8 + 5)
         CUDA_TRY(cudaMalloc(&h->dAb, sizeof(double) * (size_t)K * Kp));
         CUDA_TRY(cudaMalloc(&h->dBTb, sizeof(double) * (size_t)M * Kp));
@@ -273,7 +230,7 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaDeviceSynchronize());
     }
-    if (K <= SMALL_K_MAX && h->TQT == 8 && Kp % 8 == 0) {
+    if (K <= SMALL_K_MAX) {
         // optional f32 mode (cv_decode_batch_f32): f32 copies of the model
         const bool bal = h->dAb != nullptr;
         const int base = bal ? K / h->G : 0, rem = bal ? K % h->G : 0;
@@ -284,19 +241,6 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
         build_f32_kernel<<<32, 256>>>(h->dA, h->dA32f, K, K, Kp, base, rem);
         build_f32_kernel<<<std::max(1, h->num_sms) * 4, 256>>>(h->dBT, h->dBT32, M, K, Kp, base, rem);
         g_launches += 3;
-        CUDA_TRY(cudaGetLastError());
-        CUDA_TRY(cudaDeviceSynchronize());
-    }
-    // every finite entry of logA / logB <= 0 (log-probabilities): the f32 pre-filter's error bound needs it
-    h->nonpositive = true;
-    for (int64_t i = 0; i < (int64_t)K * K && h->nonpositive; i++) if (logA[i] > 0.0) h->nonpositive = false;
-    for (int64_t i = 0; i < (int64_t)K * M && h->nonpositive; i++) if (logB[i] > 0.0) h->nonpositive = false;
-    if (K <= SMALL_K_MAX && h->TQT == 8 && h->nonpositive && K >= 17 && Kp % 8 == 0) {
-        CUDA_TRY(cudaMalloc(&h->dA32, sizeof(float) * (size_t)Kp * Kp));
-        CUDA_TRY(cudaMalloc(&h->dA64T, sizeof(double) * (size_t)Kp * Kp));
-        const bool bal = h->dAb != nullptr;
-        build_prefilter_kernel<<<32, 256>>>(h->dA, K, Kp, bal ? K / h->G : 0, bal ? K % h->G : 0, h->dA32, h->dA64T);
-        g_launches++;
         CUDA_TRY(cudaGetLastError());
         CUDA_TRY(cudaDeviceSynchronize());
     }
@@ -317,8 +261,8 @@ extern "C" void cv_hmm_destroy(cv_hmm *h)
     if (!h) return;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
-    for (double *p : {h->dA, h->dBT, h->dPi, h->dAl, h->dBTl, h->dATl, h->dAb, h->dBTb, h->dA64T}) if (p) cudaFree(p);
-    for (float *p : {h->dA32, h->dA32n, h->dA32f, h->dBT32}) if (p) cudaFree(p);
+    for (double *p : {h->dA, h->dBT, h->dPi, h->dAl, h->dBTl, h->dATl, h->dAb, h->dBTb}) if (p) cudaFree(p);
+    for (float *p : {h->dA32n, h->dA32f, h->dBT32}) if (p) cudaFree(p);
     for (DevBuf *b : {&h->obs, &h->seq_off, &h->path, &h->score}) b->release();
     for (auto &w : h->ws) {
         for (DevBuf *b : {&w.order, &w.keys_in, &w.keys_out, &w.vals_in, &w.cub_tmp, &w.hist, &w.tmax, &w.base, &w.misc,
@@ -549,27 +493,11 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
 {
     const int G = h->G;
     const uint32_t *d_order = (const uint32_t *)w.order.p, *d_sorted_len = (const uint32_t *)w.keys_out.p;
-    // Launch shape: S sequence groups of 64 per CTA, and which register budget (kernel instantiation) to use.
-    int S = 1, variant = 1;
-    if (g_tune.small_cfg >= 0) { S = std::max(1, std::min(4, g_tune.small_cfg / 10)); variant = std::max(1, g_tune.small_cfg % 10); }
-    int tpt = g_tune.tp;
-    if (h->TQT != 8) tpt = 2;
-    // forward kernel with the f32 pre-filter (decode_prefilter.cuh): non-positive models, 64 sequences per tile
-    const bool pf = !h->f32mode && g_tune.prefilter && h->dA32 && h->TQT == 8 && g_tune.small_cfg < 0 && tpt == 2 && 32 * G <= 256 &&
-                    decode_pf_smem_bytes(h->Kp) <= 113 * 1024;
     // optional f32 mode (decode_f32.cuh): its own forward kernel, f32 history, f32 backtrace
-    const bool f32 = h->f32mode && h->dA32f && h->TQT == 8 && g_tune.small_cfg < 0 && tpt == 2 && 32 * G <= 256;
-    if (h->f32mode && !f32) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs the default tile shape (K <= 64)");
-    if (pf || f32) S = 1;
-    while (S > 1 && (B + 32 * tpt * S - 1) / (32 * tpt * S) < 4 * (int64_t)h->num_sms) S--;
-    size_t smem = f32 ? decode_f32_smem_bytes(h->K, h->Kp) : pf ? decode_pf_smem_bytes(h->Kp) : decode_small_smem_bytes(h->K, h->Kp, 32 * tpt * S);
-    while (smem > 220 * 1024 && S > 1) { S--; smem = decode_small_smem_bytes(h->K, h->Kp, 32 * tpt * S); }
-    if (smem > 220 * 1024 && tpt == 4) { tpt = 2; smem = decode_small_smem_bytes(h->K, h->Kp, 32 * tpt * S); }
-    const int NS = 32 * tpt * S;
-    const int threads = 32 * G * S;
-    if (variant == 3 && threads > 256) variant = 2;
-    if (variant == 2 && threads > 384) variant = 1;
-    if (threads > 512) return fail(CV_ERR_UNSUPPORTED, "small-K launch shape needs %d threads", threads);
+    const bool f32 = h->f32mode != 0;
+    // tiles of NS = 64 sequences (TP = 2 per lane), one warp per state group
+    const int NS = 32 * TP, threads = 32 * G;
+    size_t smem = f32 ? decode_f32_smem_bytes(h->K, h->Kp) : decode_small_smem_bytes(h->K, h->Kp, NS);
     const int64_t ntiles64 = (B + NS - 1) / NS;
     if (ntiles64 > 0x7fffffffLL) return fail(CV_ERR_UNSUPPORTED, "batch too large");
     const int ntiles = (int)ntiles64;
@@ -588,7 +516,7 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     // also checks every tile against hist_cap_rows and reports CV_ERR_UNSUPPORTED instead of storing past the end.
     const size_t stairs = sio ? 2 * (size_t)sio->cbs.nch - 1 : 1;
     const size_t hist_rows = (size_t)N + (size_t)NS * (size_t)max_len * stairs;     // in units of K doubles
-    const size_t hist_elems = hist_rows * (size_t)(pf ? pf_pitch(h->Kp) : h->K);    // pre-filter kernel: rows of Kp + 2 doubles
+    const size_t hist_elems = hist_rows * (size_t)h->K;
     if ((rc = w.hist.ensure(hist_elems * (f32 ? sizeof(float) : sizeof(double))))) return rc;
     if ((rc = w.tmax.ensure(sizeof(long long) * (size_t)ntiles))) return rc;
     if ((rc = w.base.ensure(sizeof(long long) * (size_t)ntiles))) return rc;
@@ -609,37 +537,29 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     p.At = h->dA; p.BTt = h->dBT; p.nq_base = p.nq_rem = 0;
     p.obs16 = h->obs16; p.path8 = h->path8; p.em_light = g_tune.em_light;
     p.is_long = (ls && ls->lstar) ? ls->is_long : nullptr;
-    p.A32s = f32 ? h->dA32f : h->dA32; p.A64Ts = h->dA64T; p.A32n = h->dA32n; p.BT32 = h->dBT32;
-    if ((pf || f32 || g_tune.balanced_split) && h->dAb && h->TQT == 8 && tpt == 2) {     // (the pre-filter operands are built for the balanced split)
+    p.A32s = h->dA32f; p.A32n = h->dA32n; p.BT32 = h->dBT32;
+    if ((f32 || g_tune.balanced_split) && h->dAb) {
         p.At = h->dAb; p.BTt = h->dBTb; p.nq_base = h->K / G; p.nq_rem = h->K % G;
     }
     p.tile_base = (const long long *)w.base.p;
     p.hist = (double *)w.hist.p; p.hist_cap_slabs = (long long)(hist_rows / (size_t)NS); p.path = d_path; p.score = d_score; p.tile_counter = d_counter; p.status = d_status;
-    p.M = h->M; p.B = B; p.K = h->K; p.Kp = h->Kp; p.G = G; p.S = S; p.NS = NS; p.ntiles = ntiles;
+    p.M = h->M; p.B = B; p.K = h->K; p.Kp = h->Kp; p.G = G; p.NS = NS; p.ntiles = ntiles;
     p.tile_tmax = nullptr; p.tile_chunk = nullptr; p.arrived = nullptr; p.chunk_done = nullptr; p.nch = 0;
     if (sio) {
         p.tile_tmax = (const long long *)w.tmax.p; p.tile_chunk = (const int *)w.delta_g.p;
         p.arrived = sio->d_arrived; p.chunk_done = sio->d_chunk_done; p.nch = sio->cbs.nch;
         for (int c = 0; c <= sio->cbs.nch; c++) p.cb[c] = sio->cbs.cb[c];
     }
-    void (*kern)(DecodeSmallParams);
-    if (f32) kern = decode_f32_fwd_kernel;
-    else if (pf) kern = decode_pf_fwd_kernel;
-    else if (h->TQT == 12) kern = variant == 1 ? decode_small_fwd_kernel<12, 512, 1> : decode_small_fwd_kernel<12, 256, 2>;
-    else if (h->TQT == 6) kern = variant == 1 ? decode_small_fwd_kernel<6, 512, 1> : decode_small_fwd_kernel<6, 256, 2>;
-    else if (tpt == 4 && threads <= 256) kern = decode_small_fwd_kernel<8, 256, 1, 4>;
-    else if (tpt == 4) kern = decode_small_fwd_kernel<8, 512, 1, 4>;
-    else kern = variant == 1 ? decode_small_fwd_kernel<8, 512, 1>
-              : variant == 2 ? decode_small_fwd_kernel<8, 384, 2> : decode_small_fwd_kernel<8, 256, 3>;
+    void (*kern)(DecodeSmallParams) = f32 ? decode_f32_fwd_kernel : decode_small_fwd_kernel<0>;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     int occ = 1;
     CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
     occ = std::max(1, occ);
-    if (!f32 && !pf && h->TQT == 8 && tpt == 2 && S == 1 && variant == 1 && g_tune.fwd_ldc) {
-        // Default shape: the same kernel with compile-time row pitches (tiles of 64 sequences, logA rows at a pitch of
-        // 64 doubles in shared memory) -- unless the wider logA costs a resident CTA per SM.
-        void (*kc)(DecodeSmallParams) = decode_small_fwd_kernel<8, 512, 1, 2, FWD_LDC>;
+    if (!f32 && g_tune.fwd_ldc) {
+        // The same kernel with compile-time row pitches (tiles of 64 sequences, logA rows at a pitch of 64 doubles in
+        // shared memory) -- unless the wider logA costs a resident CTA per SM.
+        void (*kc)(DecodeSmallParams) = decode_small_fwd_kernel<FWD_LDC>;
         const size_t smem_c = decode_small_smem_bytes(h->K, h->Kp, NS, FWD_LDC);
         int occ_c = 0;
         if (smem_c <= 220 * 1024) {
@@ -651,8 +571,8 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     }
     const int grid = (int)std::min<int64_t>((int64_t)h->num_sms * occ, ntiles);
     if (g_tune.debug)
-        fprintf(stderr, "[cv] decode_small: K=%d TQ=%d TP=%d G=%d S=%d variant=%d prefilter=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
-                h->K, h->TQT, tpt, G, S, variant, (int)pf, threads, smem, occ, grid, ntiles);
+        fprintf(stderr, "[cv] decode_small: K=%d G=%d f32=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
+                h->K, G, (int)f32, threads, smem, occ, grid, ntiles);
     // Concurrent backtrace: the backtrace kernel runs next to the forward kernel on a second stream and follows
     // it tile by tile (tile_done flags).  It is released only when every forward CTA is resident (stream wait on
     // the `started` counter), so its spinning CTAs can never keep a forward CTA off an SM; it then lives on the
@@ -698,15 +618,15 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     if (timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev1, st));
     // end state + backtrace with lazy backpointers: one thread per sequence
     const size_t smem_bt = (size_t)h->K * (h->K | 1) * 8 + 16 * 8;      // + one chunk of padding behind the last row
-    void (*bt_seq)(DecodeSmallParams) = f32 ? backtrace_small_kernel<16, 4, 64, 0, float> : pf ? backtrace_small_kernel<16, 4, 64, 1> : NS == 64 ? backtrace_small_kernel<16, 4, 64> : backtrace_small_kernel<16, 4, 0>;
-    void (*bt_con)(DecodeSmallParams) = f32 ? backtrace_small_kernel<8, 8, 64, 0, float> : pf ? backtrace_small_kernel<8, 8, 64, 1> : NS == 64 ? backtrace_small_kernel<8, 8, 64> : backtrace_small_kernel<8, 8, 0>;
-    // Four lanes per sequence (backtrace_split_kernel): f64, history layout 0, tiles of 64 sequences -- for batches that do
+    void (*bt_seq)(DecodeSmallParams) = f32 ? backtrace_small_kernel<16, 4, float> : backtrace_small_kernel<16, 4>;
+    void (*bt_con)(DecodeSmallParams) = f32 ? backtrace_small_kernel<8, 8, float> : backtrace_small_kernel<8, 8>;
+    // Four lanes per sequence (backtrace_split_kernel, f64 only) -- for batches that do
     // not fill the GPU for long (a rank's slice of a sharded batch): there the one-thread-per-sequence kernel is latency
     // bound and most of its work is still open when the forward kernel ends.  Measured, device step with the concurrent
     // backtrace, split vs. one thread per sequence: 125 k sentences 1.51 vs 1.74 ms, 250 k 2.83 vs 2.79 ms, 500 k 5.59 vs
     // 5.29 ms, 1 M 11.20 vs 10.56 ms (four times the threads re-stage logA four times as often and execute ~15 % more
     // instructions next to an issue-bound forward kernel).  bt_split = 2 forces it for every size.
-    bool bt_split = g_tune.bt_split && !f32 && !pf && NS == 64 && (g_tune.bt_split >= 2 || B <= (int64_t)1300 * h->num_sms);
+    bool bt_split = g_tune.bt_split && !f32 && (g_tune.bt_split >= 2 || B <= (int64_t)1300 * h->num_sms);
     size_t smem_bt_use = smem_bt;
     if (bt_split) {
         const int JP = h->K <= 16 ? 4 : h->K <= 32 ? 8 : h->K <= 48 ? 12 : 16;
@@ -747,6 +667,15 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     return CV_OK;
 }
 
+// Batches of up to 8192 sequences with K <= 64 go to the warp-per-sequence kernel; cv_debug_set_chain_max_batch moves
+// that bound for the exact mode.  The f32 mode keeps it whatever the override says: cv_b200.h promises such batches
+// the exact f64 kernel.
+static bool chain_batch(const cv_hmm *h, int64_t B)
+{
+    const long long bound = (g_tune.chain_max_b < 0 || h->f32mode) ? 8192 : g_tune.chain_max_b;
+    return h->K <= SMALL_K_MAX && B <= bound;
+}
+
 // One chunk of sequences [0, B) of d_off (offsets are absolute into d_obs / d_path): order by length,
 // forward, backtrace; everything enqueued on `st` with workspace set `w`.
 static int decode_chunk(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
@@ -762,7 +691,7 @@ static int decode_chunk(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int
     unsigned int *d_counter = (unsigned int *)w.misc.p;
     int *d_status = (int *)w.misc.p + 16;
     CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, 256, st));
-    const bool chain_all = h->K <= SMALL_K_MAX && (g_tune.chain_max_b < 0 ? B <= 8192 : B <= g_tune.chain_max_b);
+    const bool chain_all = chain_batch(h, B);
     LongSplit ls{0u, 0u, nullptr, nullptr, nullptr};
     if (!chain_all && (rc = long_split_setup(h, w, B, N, max_len, st, ls))) return rc;
     // order sequences by length, longest first (stable radix sort => deterministic)
@@ -947,7 +876,7 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     StreamWaitValue32Fn wait32 = stream_wait_value32();
     StreamWriteValue32Fn write32 = stream_write_value32();
     if (!g_tune.streamed || !g_tune.bt_concurrent || !wait32 || !write32 || nch < 2 || nch > STREAM_MAX_CHUNKS) return CV_OK;
-    if (h->K > SMALL_K_MAX || (g_tune.chain_max_b < 0 ? B <= 8192 : B <= g_tune.chain_max_b) || B > 0x7fffffffLL) return CV_OK;
+    if (h->K > SMALL_K_MAX || chain_batch(h, B) || B > 0x7fffffffLL) return CV_OK;
     const int64_t N = seq_off[B];
     DecodeWs &w = h->ws[0];
     cudaStream_t sk = w.st, s_in = h->ws[1].st, s_out = h->ws[1].st_bt;

@@ -41,26 +41,21 @@ int check_device(int device);
 // Defaults are what the library ships with.  The environment is read ONCE, when the library is loaded (never on a
 // launch path); tests and bench.py change single fields through include/cv_b200_debug.h.
 struct Tuning {
-    int small_cfg = -1;            // small-K launch shape 10*S + MINB, -1 = automatic          (cv_debug_set_small_config)
     int chunks = -1;               // chunks a host batch is cut into, -1 = automatic             (cv_debug_set_chunks, CV_CHUNKS)
     long long chain_max_b = -1;    // batches up to this size use the warp-per-sequence kernel, -1 = 8192
     int bt_concurrent = 1;         // backtrace next to the forward kernel                        (CV_BT_CONCURRENT)
     int streamed = 1;              // host copies streamed past one launch                        (CV_STREAMED)
-    int tq = 8;                    // target states per warp of the forward tile kernel: 6, 8, 12, 0 = auto (CV_TQ)
-    int tp = 2;                    // sequences per lane: 2 or 4                                  (CV_TP)
     int balanced_split = 1;        // forward tile kernel: state groups of near-equal size, no padded states (CV_BALANCED)
     int fwd_ldc = 1;               // forward tile kernel with compile-time row pitches (tiles of 64, logA pitch 64) when it costs no occupancy (CV_FWD_LDC)
     int em_light = 1;              // uneven balanced split: only the lighter state groups fetch the emission rows (CV_EM_LIGHT)
     int bt_split = 1;              // backtrace with four lanes per sequence (backtrace_split_kernel) where it applies (CV_BT_SPLIT)
     int uneven_chunks = 1;         // streamed host path, automatic chunking: 10/25/25/20/12/8 % with the last chunk's long sequences promoted (CV_UNEVEN_CHUNKS)
     int long_pct = 0;              // long-sequence split: limit in % of the tile-steps per resident CTA, 0 = automatic (70 / 45) (CV_LONG_PCT)
-    int prefilter = 0;             // forward tile kernel with the f32 pre-filter (decode_prefilter.cuh) when the model allows it (CV_PREFILTER)
     int long_split = 1;            // very long sequences of a short batch go to the warp-per-sequence kernel (CV_LONG_SPLIT)
     int debug = 0;                 // print launch shapes                                         (CV_DEBUG)
     int bt_prof = 0, e2e_prof = 0; // print pipeline timelines                                    (CV_BT_PROF, CV_E2E_PROF)
     long long large_group_rb = 0;  // row blocks per group of the large-K kernel, 0 = automatic    (CV_LARGE_GROUP_RB)
     int cp_fullwarp = 0, cp_prof = 0, cp_sum = -1, cp_hostpoll = 1, cp_leaf_batch = 1;   // constrained solver (CV_CP_*)
-    int probe_threads = 384;       // CV_PROBE_THREADS
 };
 extern Tuning g_tune;
 
@@ -91,17 +86,14 @@ struct DevBuf {
 
 // ---- model handle (opaque in the ABI) ------------------------------------------------------------------------------
 struct cv_hmm {
-    int device = 0, K = 0, Kp = 0, G = 0, D = 0, num_sms = 0, TQT = 8;
+    int device = 0, K = 0, Kp = 0, G = 0, D = 0, num_sms = 0;
     int64_t M = 1;
-    bool nonpositive = false;   // every finite model entry is <= 0 (true for log-probabilities)
     // device model
     double *dA = nullptr;    // [K][Kp]   small-K layout (Kp = 8*ceil(K/8)), pad = -inf
     double *dBT = nullptr;   // [M][Kp]
     double *dPi = nullptr;   // [Kp]
-    // slot-permuted copies for the balanced state split of the forward tile kernel (TQT = 8, K % 8 != 0), else null
+    // slot-permuted copies for the balanced state split of the forward tile kernel (K % 8 != 0), else null
     double *dAb = nullptr, *dBTb = nullptr;
-    // pre-filter forward kernel (decode_prefilter.cuh): f32 logA with slot-permuted columns, f64 logA transposed per slot
-    float *dA32 = nullptr; double *dA64T = nullptr;
     // f32 mode (decode_f32.cuh): rn32(logA) natural [K][Kp] and slot-permuted [K][Kp], rn32(logB^T) slot-permuted [M][Kp]
     float *dA32n = nullptr, *dA32f = nullptr, *dBT32 = nullptr;
     int f32mode = 0;                          // the call in progress is cv_decode_batch_f32 / cv_decode_batch_dev_f32

@@ -16,9 +16,17 @@
 #pragma once
 
 #include "decode_small.cuh"
-#include "decode_prefilter.cuh"      // fadd2
 
 namespace cvb {
+
+// packed f32 add (FADD2): two cells per instruction
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b)
+{
+    float2 r;
+    asm("{ .reg .b64 ra, rb, rc; mov.b64 ra, {%2, %3}; mov.b64 rb, {%4, %5}; add.rn.f32x2 rc, ra, rb; mov.b64 {%0, %1}, rc; }"
+        : "=f"(r.x), "=f"(r.y) : "f"(a.x), "f"(a.y), "f"(b.x), "f"(b.y));
+    return r;
+}
 
 __host__ __device__ inline int f32_em_pitch(int Kp) { return Kp + 4; }   // floats; rows stay 16-byte aligned
 __host__ __device__ inline size_t decode_f32_smem_bytes(int K, int Kp)

@@ -13,7 +13,7 @@
 //    logA[j][s]) is a pure function of the stored row, so the backtrace recomputes
 //    it only for the one state per step on the decoded path (K cells, not K*K).
 //
-//    Mapping: persistent CTAs pull tiles of NS = 64*S sequences (pre-sorted by
+//    Mapping: persistent CTAs pull tiles of NS = 64 sequences (pre-sorted by
 //    length, longest first, so a tile runs in lock step).  Shared memory holds
 //      sA  [K][Kp]      logA, staged once per CTA by a TMA bulk copy
 //      sD  [2][K][NS]   delta, double buffered, [state][sequence slot]
@@ -22,7 +22,7 @@
 //    A lane owns TP=2 adjacent sequences (one conflict-free LDS.128 per j), a warp
 //    owns TQ=8 adjacent target states (four broadcast LDS.128 per j): 16 cells per
 //    thread per predecessor from 5 shared loads.  Warps = G state groups
-//    (G = ceil(K/8)) x S sequence groups.  After the j loop the thread adds the
+//    (G = ceil(K/8)).  After the j loop the thread adds the
 //    emission ((delta + a) + b, viterbi.rs:17; an emission of -inf gives -inf,
 //    viterbi.rs:19-21) and stores 8 x double2 into the other buffer; after the
 //    step barrier one thread writes the whole [K][NS] slab to the history with a
@@ -40,28 +40,15 @@
 
 #include "common.cuh"
 
-#ifndef CVB_FWD_UNROLL
-// predecessors per unrolled iteration of the forward tile loop.  Measured at the POS shape (K = 45: predecessor 0 is
-// peeled, 44 remain), forward kernel alone / whole step: 2: 10.94 / 11.49 ms, 4: 10.63 / 11.36 ms, 11: 10.27 / 12.64 ms
-// -- the loop-carried register moves at the back edge (22 IMAD.MOV per iteration) amortise with the unroll factor, but
-// the 13 KB loop bodies (one per state-group width) then fight the concurrent backtrace for the instruction cache.
-// With CVB_FWD_TREE (default) the loop takes the predecessors in pairs, two pairs per iteration: 10.60 / 11.30 ms.
-#define CVB_FWD_UNROLL 4
-#endif
-#ifndef CVB_FWD_TREE
-#define CVB_FWD_TREE 1        // 1: two predecessors are reduced before they meet the running maximum (see maxplus_tile_val)
-#endif
-
 namespace cvb {
 
 struct DecodeSmallParams {
     const double *A;         // [K][Kp]   logA, columns >= K padded with -inf (natural column order: the backtrace)
     const double *BT;        // [M][Kp]   logB transposed (obs-major), padded -inf
     const double *At, *BTt;  // what the forward tile kernel reads: A / BT, or their slot-permuted copies (balanced split)
-    const float *A32n;       // f32 mode (decode_f32.cuh): rn32(logA) [K][Kp], natural columns (backtrace); A32s/BT32 below for its forward kernel
+    const float *A32n;       // f32 mode (decode_f32.cuh): rn32(logA) [K][Kp], natural columns (backtrace)
+    const float *A32s;       //                            rn32(logA) [K][Kp], slot-permuted like At (forward kernel)
     const float *BT32;       //                            rn32(logB^T) [M][Kp], slot-permuted like BTt
-    const float *A32s;       // pre-filter kernel (decode_prefilter.cuh): [Kp][Kp] f32, rows = predecessors, slot-permuted columns
-    const double *A64Ts;     //                                           [Kp][Kp] f64, rows = slots, columns = predecessors
     const uint32_t *obs;     // [N]
     const int64_t *seq_off;  // [B+1]
     const uint32_t *order;   // [B] sequence ids, longest first
@@ -89,8 +76,8 @@ struct DecodeSmallParams {
     int nch;
     int64_t cb[18];                  // chunk boundaries: chunk c = sequences [cb[c], cb[c+1])
     int64_t M, B;
-    int K, Kp, G, S, NS, ntiles;   // NS = sequences per tile = 32 * TPT * S
-    // balanced state split (TQT = 8 only): state group g owns nq_base + (g < nq_rem) states starting at state
+    int K, Kp, G, NS, ntiles;      // NS = sequences per tile (64)
+    // balanced state split: state group g owns nq_base + (g < nq_rem) states starting at state
     // g * nq_base + min(g, nq_rem); the columns of A / BT are permuted into 8-wide slots per group (slot 8g + q holds
     // that group's q-th state, unused slots -inf).  nq_base = 0: the plain layout (group g = states 8g .. 8g+7).
     int nq_base, nq_rem;
@@ -127,22 +114,22 @@ __host__ __device__ inline size_t decode_small_smem_bytes(int K, int Kp, int NS,
     return (size_t)K * (lda ? lda : Kp) * 8 + (size_t)2 * K * NS * 8 + (size_t)NS * em_pitch(Kp) * 8 + (size_t)NS * (8 + 4) + 32 + 16;
 }
 
-// value-only TP x TQ micro-tile: best[p][q] = max_j ( dcol[j*ldd + p] + arow[j*lda + q] )
+// value-only TP x TQ micro-tile over predecessors [0, nj), nj >= 1: best[p][q] = max_j ( dcol[j*ldd + p] + arow[j*lda + q] )
 // (strict > keeps the first maximum's bits, e.g. the sign of a zero, as the reference does).
-// NQ <= TQT: only the first NQ target states of the slot group are computed (balanced split: the slots behind them
+// NQ <= TQ: only the first NQ target states of the slot group are computed (balanced split: the slots behind them
 // are padding); the operand loads stay 16-byte pairs.
 // LDC > 0: both row pitches are the compile-time constant LDC (doubles) -- every operand load of an unrolled iteration is
 // base + immediate off two pointers that advance once per iteration (with run-time pitches: two IMADs per predecessor)
-template <int TQT, int UNR = 2, int TPT = TP, int NQ = TQT, bool FIRST = false, int LDC = 0>
+template <int NQ, int LDC>
 __device__ __forceinline__ void maxplus_tile_val(const double *__restrict__ dcol, int ldd_rt,
                                                  const double *__restrict__ arow, int lda_rt, int nj,
-                                                 double (&best)[TPT][TQT])
+                                                 double (&best)[TP][TQ])
 {
     const int ldd = LDC ? LDC : ldd_rt, lda = LDC ? LDC : lda_rt;
     // operands of one predecessor: dp / ap point at its delta row and its logA row
-    auto load = [&](const double *dp, const double *ap, double (&dd)[TPT], double (&a)[TQT]) {
+    auto load = [&](const double *dp, const double *ap, double (&dd)[TP], double (&a)[TQ]) {
 #pragma unroll
-        for (int p = 0; p < TPT / 2; p++) {
+        for (int p = 0; p < TP / 2; p++) {
             const double2 d = *reinterpret_cast<const double2 *>(dp + 2 * p);
             dd[2 * p] = d.x; dd[2 * p + 1] = d.y;
         }
@@ -155,28 +142,31 @@ __device__ __forceinline__ void maxplus_tile_val(const double *__restrict__ dcol
     // the two row pointers walk the predecessors (no index arithmetic in the loop)
     const double *dp = dcol, *ap = arow;
     const double *const dend = dcol + (size_t)nj * ldd;
-    if (FIRST) {
+    {
         // predecessor 0 starts the running maximum: `best = -inf; if (v > best) best = v` leaves best = v for every v
         // that can occur (v is never NaN), so the initialisation and the first compare/select are dropped
-        double dd[TPT], a[TQT];
+        double dd[TP], a[TQ];
         load(dp, ap, dd, a);
 #pragma unroll
-        for (int p = 0; p < TPT; p++)
+        for (int p = 0; p < TP; p++)
 #pragma unroll
             for (int q = 0; q < NQ; q++) best[p][q] = dd[p] + a[q];
         dp += ldd; ap += lda;
     }
-#if CVB_FWD_TREE
     // two predecessors are reduced before they meet the running maximum: the dependent chain on `best` is one
     // compare/select per two predecessors.  `b > a ? b : a` keeps the EARLIER value on a tie at
     // every level, so the result carries the bits of the first maximum exactly as the sequential scan does.
-    const double *const dend2 = dp + (size_t)((nj - (FIRST ? 1 : 0)) & ~1) * ldd;      // an even number of predecessors
+    // Measured at the POS shape (K = 45), forward kernel alone / whole step: pairs, two per iteration, 10.60 / 11.30 ms;
+    // one predecessor at a time unrolled 2: 10.94 / 11.49 ms, 4: 10.63 / 11.36 ms, 11: 10.27 / 12.64 ms -- the
+    // loop-carried register moves at the back edge amortise with the unroll factor, but the 13 KB loop bodies (one per
+    // state-group width) then fight the concurrent backtrace for the instruction cache.
+    const double *const dend2 = dp + (size_t)((nj - 1) & ~1) * ldd;      // an even number of predecessors
 #pragma unroll 2
     for (; dp != dend2; dp += 2 * ldd, ap += 2 * lda) {
-        double d0[TPT], d1[TPT], a0[TQT], a1[TQT];
+        double d0[TP], d1[TP], a0[TQ], a1[TQ];
         load(dp, ap, d0, a0); load(dp + ldd, ap + lda, d1, a1);
 #pragma unroll
-        for (int p = 0; p < TPT; p++)
+        for (int p = 0; p < TP; p++)
 #pragma unroll
             for (int q = 0; q < NQ; q++) {
                 const double v0 = d0[p] + a0[q], v1 = d1[p] + a1[q];
@@ -185,14 +175,11 @@ __device__ __forceinline__ void maxplus_tile_val(const double *__restrict__ dcol
             }
     }
 #pragma unroll 1
-#else
-#pragma unroll UNR
-#endif
-    for (; dp != dend; dp += ldd, ap += lda) {                       // (with the pair loop above: at most one predecessor is left)
-        double dd[TPT], a[TQT];
+    for (; dp != dend; dp += ldd, ap += lda) {                       // at most one predecessor is left
+        double dd[TP], a[TQ];
         load(dp, ap, dd, a);
 #pragma unroll
-        for (int p = 0; p < TPT; p++)
+        for (int p = 0; p < TP; p++)
 #pragma unroll
             for (int q = 0; q < NQ; q++) {
                 const double v = dd[p] + a[q];
@@ -222,29 +209,29 @@ __device__ __forceinline__ void fence_proxy_async_smem()
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
 
-// One step of one thread: its TPT sequences x NQ target states.  best = max_j (delta[t-1][j] + a[j][i]) over all
+// One step of one thread: its TP sequences x NQ target states.  best = max_j (delta[t-1][j] + a[j][i]) over all
 // predecessors (value only), then (.. + b) (viterbi.rs:17) into the other delta buffer.  `row0` points at the row of the
 // group's first state in that buffer, `nreal` = how many of the NQ states exist (the last group of the plain layout
 // may reach past K).
-template <int TQT, int TPT, int NQ, int LDC = 0>
+template <int NQ, int LDC>
 __device__ __forceinline__ void fwd_step(const double *__restrict__ dcur, double *__restrict__ row0, int NS_rt,
                                          const double *__restrict__ arow, int lda, int K, const double *__restrict__ e0, int EP,
                                          uint64_t *em_bar, uint32_t em_phase, int nreal)
 {
     const int NS = LDC ? LDC : NS_rt;
-    double best[TPT][TQT];
-    maxplus_tile_val<TQT, CVB_FWD_UNROLL, TPT, NQ, true, LDC>(dcur, NS, arow, lda, K, best);     // K >= 1: predecessor 0 exists
+    double best[TP][TQ];
+    maxplus_tile_val<NQ, LDC>(dcur, NS, arow, lda, K, best);     // K >= 1: predecessor 0 exists
 
     mbar_wait(em_bar, em_phase);      // emission rows of step t have landed
 #pragma unroll
     for (int k = 0; k < (NQ + 1) / 2; k++) {
-        double2 x[TPT];
+        double2 x[TP];
 #pragma unroll
-        for (int q = 0; q < TPT; q++) x[q] = *reinterpret_cast<const double2 *>(e0 + (size_t)q * EP + 2 * k);
+        for (int q = 0; q < TP; q++) x[q] = *reinterpret_cast<const double2 *>(e0 + (size_t)q * EP + 2 * k);
         // (delta + a) + b (viterbi.rs:17).  Sequences that already ended compute garbage in their
         // own column only; their last row is already in the history.
 #pragma unroll
-        for (int q = 0; q < TPT; q += 2) {
+        for (int q = 0; q < TP; q += 2) {
             if (2 * k < nreal)
                 *reinterpret_cast<double2 *>(row0 + (size_t)(2 * k) * NS + q) =
                     make_double2(best[q][2 * k] + x[q].x, best[q + 1][2 * k] + x[q + 1].x);
@@ -255,14 +242,12 @@ __device__ __forceinline__ void fwd_step(const double *__restrict__ dcur, double
     }
 }
 
-// TQT = target states per thread (8 or 12; a warp owns TQT adjacent states); MAXT/MINB only set the register
-// budget (launch bounds).  The host picks TQT and S so that a CTA has a multiple of 4 warps: warps map to the
-// four SM sub-partitions by warp id, and with the per-step barrier an uneven split leaves sub-partitions idle.
+// One warp per state group of TQ = 8 target states, TP = 2 sequences per lane: 32 * G threads per CTA.
 // LDC > 0 (= FWD_LDC = 64): tiles of exactly LDC sequences and logA rows at a pitch of LDC doubles in shared memory,
 // both known at compile time (see maxplus_tile_val); 0: run-time NS and pitch Kp.
 constexpr int FWD_LDC = 64;
-template <int TQT, int MAXT, int MINB, int TPT = TP, int LDC = 0>
-__global__ void __launch_bounds__(MAXT, MINB) decode_small_fwd_kernel(const DecodeSmallParams p)
+template <int LDC>
+__global__ void __launch_bounds__(512, 1) decode_small_fwd_kernel(const DecodeSmallParams p)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int K = p.K, Kp = p.Kp, NS = LDC ? LDC : p.NS, EP = em_pitch(Kp);
@@ -277,14 +262,14 @@ __global__ void __launch_bounds__(MAXT, MINB) decode_small_fwd_kernel(const Deco
 
     const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
     const int g = w % p.G, sg = w / p.G;
-    const int i0 = g * TQT;                                  // first column slot of the group in sA / sEm
-    // first state (= delta row) of the group and how many of its TQT slots are real states
+    const int i0 = g * TQ;                                   // first column slot of the group in sA / sEm
+    // first state (= delta row) of the group and how many of its TQ slots are real states
     const int srow0 = p.nq_base ? g * p.nq_base + min(g, p.nq_rem) : i0;
-    const int nreal = p.nq_base ? p.nq_base + (g < p.nq_rem ? 1 : 0) : max(0, min(TQT, K - i0));
-    const int s0 = sg * (32 * TPT) + lane * TPT;
+    const int nreal = p.nq_base ? p.nq_base + (g < p.nq_rem ? 1 : 0) : max(0, min(TQ, K - i0));
+    const int s0 = sg * (32 * TP) + lane * TP;
     const uint32_t slab_bytes = (uint32_t)((size_t)K * NS * 8);
     const uint32_t row_bytes = (uint32_t)(Kp * 8);
-    constexpr int EMK = 2 * TPT;   // emission slots a lane may serve: NS / (32 * warps) <= 32 * TPT * S / (32 * S) = TPT, x2 slack
+    constexpr int EMK = 2 * TP;    // emission slots a lane may serve: NS / (32 * warps) <= TP, x2 slack
 
     // Who fetches the emission rows.  The per-step barrier makes the slowest warp's step the CTA's, so the fetch work
     // (one elected-lane TMA issue per row, ~10 instructions) is dealt out by how much tile work a warp has: with an
@@ -295,7 +280,7 @@ __global__ void __launch_bounds__(MAXT, MINB) decode_small_fwd_kernel(const Deco
     const int nwarps = (int)blockDim.x >> 5;
     int em_beg = 0, em_cnt = 0, n_fetch = 0;
     {
-        const bool uneven = p.em_light && p.nq_base && p.nq_rem && p.S == 1;
+        const bool uneven = p.em_light && p.nq_base && p.nq_rem;
         const int nlight = uneven ? p.G - p.nq_rem : 0;
         const int extra = uneven ? min(NS / nlight, (9 * K + 5) / 10) : 0;      // additional rows per lighter warp
         const int rest = NS - extra * nlight, base = rest / nwarps, left = rest - base * nwarps;
@@ -309,7 +294,7 @@ __global__ void __launch_bounds__(MAXT, MINB) decode_small_fwd_kernel(const Deco
         }
     }
     const int emk = (em_cnt + 31) / 32;                                                            // slots per lane that exist
-    const int st_tid = (p.em_light && p.nq_base && p.nq_rem && p.S == 1) ? 32 * p.nq_rem : 0;      // the thread that issues (and waits for) the history slab stores: one of a lighter warp
+    const int st_tid = (p.em_light && p.nq_base && p.nq_rem) ? 32 * p.nq_rem : 0;      // the thread that issues (and waits for) the history slab stores: one of a lighter warp
     // ---- stage logA once per CTA (TMA bulk copy, UBLKCP) ----
     if (tid == 0) {
         if (p.started) atomicAdd(p.started, 1u);   // the backtrace kernel is released once every forward CTA is resident
@@ -423,20 +408,18 @@ __global__ void __launch_bounds__(MAXT, MINB) decode_small_fwd_kernel(const Deco
             double *row0 = sD + (size_t)(t & 1) * K * NS + (size_t)srow0 * NS + s0;
             const double *e0 = sEm + (size_t)s0 * EP + i0;
             bool done = false;
-            if constexpr (TQT == 8 && TPT == 2) {
-                if (p.nq_base != 0) {
-                    // balanced split: this group's state count (warp-uniform); groups of fewer than 5 states take the
-                    // full-width path below (their unused slots hold -inf and are not stored)
-                    done = true;
-                    switch (nreal) {
-                        case 7: fwd_step<8, 2, 7, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
-                        case 6: fwd_step<8, 2, 6, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
-                        case 5: fwd_step<8, 2, 5, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
-                        default: done = false;
-                    }
+            if (p.nq_base != 0) {
+                // balanced split: this group's state count (warp-uniform); groups of fewer than 5 states take the
+                // full-width path below (their unused slots hold -inf and are not stored)
+                done = true;
+                switch (nreal) {
+                    case 7: fwd_step<7, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
+                    case 6: fwd_step<6, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
+                    case 5: fwd_step<5, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal); break;
+                    default: done = false;
                 }
             }
-            if (!done) fwd_step<TQT, TPT, TQT, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal);
+            if (!done) fwd_step<TQ, LDC>(dcur, row0, NS, sA + i0, lda, K, e0, EP, sBar + 1, em_phase, nreal);
             em_phase ^= 1;
             fence_proxy_async_smem();           // make this thread's delta writes visible to the TMA store
             if (tid == st_tid) tma_store_wait_read_all();   // slab t-1 has left the buffer step t+1 will overwrite
@@ -509,19 +492,17 @@ __device__ __forceinline__ void bt_mark_done_warp(const DecodeSmallParams &p, in
 template <typename T>
 __device__ __forceinline__ T bt_ld(const T *q) { return __ldcg(q); }
 
-// NSC = sequences per tile when known at compile time (64: the load offsets become immediates), 0 = p.NS
-// LAYOUT = 0: history slabs [K][NS] (decode_small_fwd_kernel); 1: [NS][Kp + 2] (decode_pf_fwd_kernel: a sequence's
-// row is contiguous and read as 16-byte vectors)
+// History slabs [K][64] (decode_small_fwd_kernel, decode_f32_fwd_kernel); the tile size is a compile-time constant
+// so that the load offsets become immediates.
 // T = double (exact, the reference's arithmetic) or float (cv_decode_batch_f32: the f32 history of decode_f32.cuh and
 // rn32(logA), same first-maximum rule on fl32 sums)
-template <int BT_CHUNK, int MINB, int NSC, int LAYOUT = 0, typename T = double>
+template <int BT_CHUNK, int MINB, typename T = double>
 __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const DecodeSmallParams p)
 {
     const T NEG = (T)neg_inf();
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int K = p.K, Kp = p.Kp, NS = NSC ? NSC : p.NS;
-    const size_t JS = LAYOUT ? 1 : (size_t)NS;                // distance between consecutive states of one sequence
-    const size_t SS = LAYOUT ? (size_t)(Kp + 2) : 1;          // distance between consecutive sequences of one state
+    constexpr int NS = 64;
+    const int K = p.K, Kp = p.Kp;
     const int ATP = K | 1;                                   // odd pitch: rows of different states spread over banks
     T *sAT = reinterpret_cast<T *>(smem_raw);               // sAT[s*ATP + j] = logA[j][s]
     for (int e = threadIdx.x; e < K * Kp; e += blockDim.x) {
@@ -530,7 +511,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
     }
     __syncthreads();
 
-    const size_t sl = LAYOUT ? (size_t)NS * (Kp + 2) : (size_t)K * NS;
+    const size_t sl = (size_t)K * NS;
     const int nfull = K / BT_CHUNK, ktail = K - nfull * BT_CHUNK;   // full chunks, predecessors of the partial last chunk
     const int nchunk = nfull + (ktail ? 1 : 0);
     const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
@@ -566,13 +547,13 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
         const int64_t off = p.seq_off[b];
         const int len = (int)(p.seq_off[b + 1] - off);
         if (len <= 0 || p.tile_base[tile] + (long long)len > p.hist_cap_slabs) return my_chunk;   // tile refused by the forward kernel (status 7)
-        const T *col = reinterpret_cast<const T *>(p.hist) + (size_t)p.tile_base[tile] * sl + (size_t)s * SS;   // sequence s of slab 0
+        const T *col = reinterpret_cast<const T *>(p.hist) + (size_t)p.tile_base[tile] * sl + (size_t)s;   // sequence s of slab 0
 
         // end state: argmax of the last row (viterbi.rs:24)
         const T *row = col + (size_t)(len - 1) * sl;
         T bv = bt_ld(row); int cur = 0;
         for (int j = 1; j < K; j++) {
-            const T v = bt_ld(row + (size_t)j * JS);
+            const T v = bt_ld(row + (size_t)j * NS);
             if (v > bv) { bv = v; cur = j; }
         }
         if (p.score) p.score[b] = (double)bv;
@@ -587,19 +568,13 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
         const T *rowp = col + (size_t)(len - 2) * sl;         // row tt-1
         int64_t pout = off + (len - 2);
         auto load_chunk = [&](const T *prow, int c, T (&dst)[BT_CHUNK]) {
-            const T *q = prow + (size_t)c * (BT_CHUNK * JS);
-            if (LAYOUT && sizeof(T) == 8 && c < nfull) {
+            const T *q = prow + (size_t)c * (BT_CHUNK * NS);
+            if (c < nfull) {
 #pragma unroll
-                for (int k = 0; k < BT_CHUNK; k += 2) {
-                    const double2 v = __ldcs(reinterpret_cast<const double2 *>(q + k));
-                    dst[k] = (T)v.x; dst[k + 1] = (T)v.y;
-                }
-            } else if (c < nfull) {
-#pragma unroll
-                for (int k = 0; k < BT_CHUNK; k++) dst[k] = bt_ld(q + (size_t)k * JS);
+                for (int k = 0; k < BT_CHUNK; k++) dst[k] = bt_ld(q + (size_t)k * NS);
             } else {
 #pragma unroll
-                for (int k = 0; k < BT_CHUNK; k++) dst[k] = (k < ktail) ? bt_ld(q + (size_t)k * JS) : NEG;
+                for (int k = 0; k < BT_CHUNK; k++) dst[k] = (k < ktail) ? bt_ld(q + (size_t)k * NS) : NEG;
             }
         };
         T mv = 0; int mi = 0;
@@ -643,7 +618,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
             }
             // psi = 0 when delta[tt][cur] = -inf (emission -inf or all candidates -inf; see header comment)
             cur = (dcur > NEG) ? mi : 0;
-            dcur = __ldcg(rowp + (size_t)cur * JS);              // delta[tt-1][cur]
+            dcur = __ldcg(rowp + (size_t)cur * NS);              // delta[tt-1][cur]
             store_path_at(p, pout, (uint32_t)cur);
             pout--; rowp -= sl;
         };
@@ -662,7 +637,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
 }
 
 // ---------------------------------------------------------------------------
-// The same end state + backtrace with FOUR lanes per sequence (history layout 0, tiles of 64 sequences, f64).
+// The same end state + backtrace with FOUR lanes per sequence (f64).
 //
 // One thread per sequence is bound by memory latency: a lane has one chunk of 8 predecessors in flight and a step costs
 // six dependent round trips (6-10 us per step; 0.41 ms for the 125 k sentences a rank of an 8-GPU run decodes, most of

@@ -1,7 +1,7 @@
 /*
  * cv_b200_debug.h -- test / bench hooks of libcv_b200.so.  NOT part of the drop-in boundary (cv_b200.h is):
  * a Rust binding of the reference's interface never needs anything declared here.  tests/, tools/ and bench.py
- * use these to force launch shapes, to dump solver state for parity checks and to measure the FP64 issue peak
+ * use these to force reachable launch paths, to dump solver state for parity checks and to measure the FP64 issue peak
  * that the roofline is quoted against.  Implemented in csrc/cv_debug.cu (setters, probe) and csrc/cv_cp.cu
  * (state dumps, ordered sum).
  */
@@ -16,13 +16,10 @@
 extern "C" {
 #endif
 
-/* force the small-K launch shape, cfg = 10*S + MINB (S sequence groups of 64 per CTA, MINB co-resident CTAs per
- * SM); -1 = automatic */
-void cv_debug_set_small_config(int cfg);
 /* number of chunks a batch is cut into (chunks overlap on two internal streams); -1 = automatic */
 void cv_debug_set_chunks(int n);
 /* batches of at most b sequences (K <= 64) use the warp-per-sequence kernel; -1 = default (8192), 0 = always the
- * tile kernel */
+ * tile kernel.  Exact mode only: the f32 mode always sends batches of <= 8192 sequences to that (f64) kernel. */
 void cv_debug_set_chain_max_batch(long long b);
 /* bt_concurrent = 1 runs the backtrace kernel next to the forward kernel (tile by tile), streamed = 1 lets
  * cv_decode_batch stream its copies past ONE launch instead of launching once per chunk; -1 = leave as is */
@@ -44,9 +41,6 @@ void cv_debug_set_bt_split(int on);
  * sequences of the last chunk are ordered with the chunk before it, 0 = equal chunks, 2 = the uneven cut for every
  * streamed call (tests) */
 void cv_debug_set_uneven_chunks(int on);
-/* forward tile kernel with the f32 pre-filter (csrc/decode_prefilter.cuh) for models whose entries are all <= 0:
- * 1 = on, 0 = the plain f64 tile kernel */
-void cv_debug_set_prefilter(int on);
 /* row blocks per group of the large-K kernel (0 = automatic: as many as the delta history fits) */
 void cv_debug_set_large_group_rb(long long rb);
 /* constrained solver: 1 = the K sibling leaves of the last component are evaluated by one batched launch, 0 = node by node */
@@ -61,9 +55,9 @@ int cv_debug_cp_last_ub(cv_hmm *h, double *ub_out, uint64_t cap, uint64_t *n_out
  * mode 0 = one-thread loop, mode 1 = the parallel exact-order kernel; both must agree bit for bit. */
 int cv_debug_ordered_sum(const double *values, int64_t n, int mode, double *out);
 
-/* FP64 issue-rate probe used as the ALU roofline denominator: runs `iters` dependent-free DADD (mode 0),
- * DADD+DSETP pairs (mode 1) or the decode inner loop body (mode >= 2) on every SM and returns FP64 instructions
- * per second.  Mode 25: independent DFMA chains (the Baum-Welch cell), returns FMAs per second. */
+/* FP64 issue-rate probe used as the ALU roofline denominator: runs `iters` dependent-free DADD (mode 0) or
+ * DADD+DSETP pairs (mode 1) on every SM and returns FP64 instructions per second.  Mode 25: independent DFMA chains
+ * (the Baum-Welch cell), returns FMAs per second.  Any other mode is CV_ERR_ARG. */
 int cv_debug_probe_fp64(int device, int mode, int iters, double *ops_per_s_out, double *ms_out);
 
 #ifdef __cplusplus

@@ -1,7 +1,5 @@
 """GPU parity tests (mode R1): cv_decode_batch through the C ABI against the C
 oracle, bit-exact on paths (u32) and scores (f64 bit patterns)."""
-import os
-
 import numpy as np
 import pytest
 
@@ -545,10 +543,9 @@ def test_long_sequence_split_equals_oracle(K):
 
 
 @pytest.mark.parametrize("K,ties,zero_frac", [(45, False, 0.15), (45, True, 0.0), (24, True, 0.0), (33, False, 0.5), (64, False, 0.05), (17, False, 0.1), (61, True, 0.0)])
-def test_prefilter_forward_kernel_equals_oracle(K, ties, zero_frac):
-    """decode_pf_fwd_kernel (f32 pre-filter + exact f64 pass over the winning block of predecessors) against the
-    oracle: models full of exact ties / +-0.0 / -inf (the "runner-up too close" full-scan path), sparse models (half
-    of the entries -inf), long sequences (delta grows, so does the f32 error), streamed and device-resident paths."""
+def test_tile_path_equals_oracle_on_ties_zeros_and_sparse_models(K, ties, zero_frac):
+    """The tile path (forward tile kernel + backtrace) against the oracle: models full of exact ties / +-0.0 / -inf,
+    sparse models (half of the entries -inf), long sequences (delta in the thousands), u32 and narrow formats."""
     rng = np.random.default_rng(6600 + K)
     M = 40
     A, B, pi = random_hmm(rng, K, M, zero_frac=zero_frac, ties=ties)
@@ -562,23 +559,18 @@ def test_prefilter_forward_kernel_equals_oracle(K, ties, zero_frac):
     L = cv._lib.lib()
     try:
         L.cv_debug_set_chain_max_batch(0)
-        for split in (1, 0):                                      # with and without the long-sequence split
-            L.cv_debug_set_prefilter(1)
-            os.environ  # noqa: B018
-            p, s = cv.decode_batch(h, obs, off)
-            assert (p == rp).all(), "paths"
-            assert s.tobytes() == rs.tobytes(), "score bits"
-            p8, s8 = cv.decode_batch_narrow(h, obs, off)
-            assert (p8 == rp).all() and s8.tobytes() == rs.tobytes()
+        p, s = cv.decode_batch(h, obs, off)
+        assert (p == rp).all(), "paths"
+        assert s.tobytes() == rs.tobytes(), "score bits"
+        p8, s8 = cv.decode_batch_narrow(h, obs, off)
+        assert (p8 == rp).all() and s8.tobytes() == rs.tobytes()
     finally:
-        L.cv_debug_set_prefilter(0)
         L.cv_debug_set_chain_max_batch(-1)
     h.close()
 
 
-def test_prefilter_is_skipped_for_models_with_positive_entries():
-    """The pre-filter's error bound needs every entry <= 0; a model with a positive log-score takes the plain kernel
-    (and still equals the oracle)."""
+def test_tile_path_equals_oracle_with_positive_log_scores():
+    """A model with positive log-scores (not log-probabilities) on the tile path still equals the oracle."""
     rng = np.random.default_rng(12)
     K, M = 40, 30
     A, B, pi = random_hmm(rng, K, M, zero_frac=0.1)
@@ -590,11 +582,9 @@ def test_prefilter_is_skipped_for_models_with_positive_entries():
     L = cv._lib.lib()
     try:
         L.cv_debug_set_chain_max_batch(0)
-        L.cv_debug_set_prefilter(1)
         p, s = cv.decode_batch(h, obs, off)
         assert (p == rp).all() and s.tobytes() == rs.tobytes()
     finally:
-        L.cv_debug_set_prefilter(0)
         L.cv_debug_set_chain_max_batch(-1)
     h.close()
 
@@ -659,15 +649,21 @@ def test_f32_mode_within_tolerance(K, zero_frac):
 
 def test_f32_mode_small_batches_take_the_exact_kernel():
     """Batches of <= 8192 sequences go to the warp-per-sequence kernel, which is f64: in f32 mode they simply return the
-    exact result (documented in include/cv_b200.h)."""
+    exact result (documented in include/cv_b200.h), also while cv_debug_set_chain_max_batch forces the tile kernel."""
     rng = np.random.default_rng(41)
     K, M = 30, 20
     A, B, pi = random_hmm(rng, K, M, zero_frac=0.1)
     obs, off = random_batch(rng, 500, M, 1, 50)
     rp, rs = po.decode_batch(A, B, obs, off, nthreads=4)
     h = cv.HMM(A, B, pi)
-    p, s = cv.decode_batch_f32(h, obs, off)
-    assert (p == rp).all() and s.tobytes() == rs.tobytes()
+    L = cv._lib.lib()
+    try:
+        for chain_max in (-1, 0):
+            L.cv_debug_set_chain_max_batch(chain_max)
+            p, s = cv.decode_batch_f32(h, obs, off)
+            assert (p == rp).all() and s.tobytes() == rs.tobytes(), f"chain_max={chain_max}"
+    finally:
+        L.cv_debug_set_chain_max_batch(-1)
     A2, B2, pi2 = random_hmm(rng, 70, 5)
     h2 = cv.HMM(A2, B2, pi2)
     with pytest.raises(cv.CvError) as e:                              # K > 64: no f32 mode

@@ -2,12 +2,11 @@
 
     python tools/fwd_variants.py [nseq] [variants...]        e.g.  python tools/fwd_variants.py 1000000 1 0
 
-variant: 1 = balanced state split (default), 0 = groups of 8 states (last one padded), 2 = the pre-filter kernel
-(decode_prefilter.cuh), 3 = the optional f32 mode (cv_decode_batch_dev_f32; results differ by design), 4 = default but
+variant: 1 = balanced state split (default), 0 = groups of 8 states (last one padded), 3 = the optional f32 mode (cv_decode_batch_dev_f32; results differ by design), 4 = default but
 run-time row pitches in the forward kernel (cv_debug_set_fwd_ldc(0)), 5 = default but every warp fetches emission rows
 (cv_debug_set_em_light(0)), 6 = default but the one-thread-per-sequence backtrace (cv_debug_set_bt_split(0)), 7 = the four-lane backtrace at
 every batch size (cv_debug_set_bt_split(2); the default uses it up to ~1300 sequences per SM).  Prints the forward kernel alone (CUDA events, timing mode), and the device-resident step (forward +
-concurrent backtrace) for each variant, plus the extra `CV_*` launch-shape settings given in the environment."""
+concurrent backtrace) for each variant, plus the extra `CV_*` settings given in the environment."""
 import ctypes as C
 import json
 import os
@@ -23,6 +22,7 @@ import consistent_viterbi_b200 as cv  # noqa: E402
 
 nseq = int(sys.argv[1]) if len(sys.argv) > 1 else 1_000_000
 variants = [int(v) for v in sys.argv[2:]] or [1, 0]
+assert all(v in (0, 1, 3, 4, 5, 6, 7) for v in variants), "unknown variant"
 wl = bench.workload_pos(0, nseq)
 L = cv._lib.lib()
 hmm = cv.HMM(wl["A"], wl["B"], wl["pi"])
@@ -51,7 +51,6 @@ ref = None
 out = []
 for v in variants:
     L.cv_debug_set_balanced_split(1 if v else 0)
-    L.cv_debug_set_prefilter(1 if v == 2 else 0)
     L.cv_debug_set_fwd_ldc(0 if v == 4 else 1)
     L.cv_debug_set_em_light(0 if v == 5 else 1)
     L.cv_debug_set_bt_split(0 if v == 6 else 2 if v == 7 else 1)
@@ -82,7 +81,6 @@ for v in variants:
     out.append(rec)
     print(json.dumps(rec), flush=True)
 L.cv_debug_set_balanced_split(1)
-L.cv_debug_set_prefilter(0)
 L.cv_debug_set_fwd_ldc(1)
 L.cv_debug_set_em_light(1)
 L.cv_debug_set_bt_split(1)

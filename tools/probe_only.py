@@ -1,4 +1,4 @@
-"""Run one probe mode (for ncu): python tools/probe_only.py MODE ITERS"""
+"""Run one FP64 probe mode (cv_debug_probe_fp64: 0, 1 or 25) in a process of its own: python tools/probe_only.py MODE ITERS"""
 import ctypes as C
 import os
 import sys
