@@ -158,6 +158,15 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     };
     if (bad(logA, (int64_t)K * K) || bad(logB, (int64_t)K * M) || bad(logPi, K))
         return fail(CV_ERR_NAN, "model contains NaN or +inf");
+    // Finite entries beyond 2^900 are refused (cv_b200.h): below it no sum of fewer than 2^63 entries can overflow, so
+    // every kernel's -inf means "impossible" exactly as in the reference.  The f32 mode has the same guarantee below 2^64.
+    auto beyond = [](const double *v, int64_t n, double lim) {
+        for (int64_t i = 0; i < n; i++) if (std::isfinite(v[i]) && std::fabs(v[i]) > lim) return true;
+        return false;
+    };
+    auto model_beyond = [&](double lim) { return beyond(logA, (int64_t)K * K, lim) || beyond(logB, (int64_t)K * M, lim) || beyond(logPi, K, lim); };
+    if (model_beyond(0x1p900)) return fail(CV_ERR_UNSUPPORTED, "model entry with |x| > 2^900 (sums could overflow)");
+    const bool f32_range_ok = !model_beyond(0x1p64);
     if (device < 0) {
         int rc = check_device(0);
         if (rc) return rc;
@@ -170,6 +179,7 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     cv_hmm *h = new cv_hmm();
     struct Guard { cv_hmm *h; ~Guard() { if (h) cv_hmm_destroy(h); } } guard{h};   // released on every early return
     h->device = device; h->K = K; h->D = D; h->M = M;
+    h->f32_range_ok = f32_range_ok;
     // state groups of the forward tile kernel: G = ceil(K/8) warps of TQ = 8 target states, Kp = 8 G
     h->G = (K + TQ - 1) / TQ;
     h->Kp = h->G * TQ;
@@ -668,11 +678,13 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
 }
 
 // Batches of up to 8192 sequences with K <= 64 go to the warp-per-sequence kernel; cv_debug_set_chain_max_batch moves
-// that bound for the exact mode.  The f32 mode keeps it whatever the override says: cv_b200.h promises such batches
-// the exact f64 kernel.
+// that bound for the exact mode.  The f32 mode keeps it whatever the override says, and applies it to the whole call,
+// not to one chunk: cv_b200.h promises such calls the exact f64 kernel, and every larger call the f32 kernels in all
+// its chunks (a forced small chunk count must not hand part of an f32 call to the f64 kernel).
 static bool chain_batch(const cv_hmm *h, int64_t B)
 {
-    const long long bound = (g_tune.chain_max_b < 0 || h->f32mode) ? 8192 : g_tune.chain_max_b;
+    if (h->f32mode) return h->K <= SMALL_K_MAX && h->f32_call_B <= 8192;
+    const long long bound = g_tune.chain_max_b < 0 ? 8192 : g_tune.chain_max_b;
     return h->K <= SMALL_K_MAX && B <= bound;
 }
 
@@ -791,7 +803,8 @@ extern "C" int cv_decode_batch_dev_f32(cv_hmm *h, const uint32_t *d_obs, const i
 {
     if (!h) return fail(CV_ERR_ARG, "NULL model");
     if (!h->dA32f) return fail(CV_ERR_UNSUPPORTED, "the f32 mode is implemented for K <= %d", SMALL_K_MAX);
-    h->f32mode = 1;
+    if (!h->f32_range_ok) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs every finite model entry within |x| <= 2^64");
+    h->f32mode = 1; h->f32_call_B = B;
     const int rc = decode_batch_dev_impl(h, d_obs, d_off, B, N, max_len, d_path, d_score, stream, sync_status);
     h->f32mode = 0;
     return rc;
@@ -1036,7 +1049,8 @@ extern "C" int cv_decode_batch_f32(cv_hmm *h, const uint32_t *obs_flat, const in
 {
     if (!h) return fail(CV_ERR_ARG, "NULL model");
     if (!h->dA32f) return fail(CV_ERR_UNSUPPORTED, "the f32 mode is implemented for K <= %d", SMALL_K_MAX);
-    h->f32mode = 1;
+    if (!h->f32_range_ok) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs every finite model entry within |x| <= 2^64");
+    h->f32mode = 1; h->f32_call_B = B;
     const int rc = decode_batch_host(h, obs_flat, seq_off, B, path_out, score_out, nullptr, nullptr);
     h->f32mode = 0;
     return rc;

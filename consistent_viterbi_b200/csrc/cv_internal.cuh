@@ -97,6 +97,8 @@ struct cv_hmm {
     // f32 mode (decode_f32.cuh): rn32(logA) natural [K][Kp] and slot-permuted [K][Kp], rn32(logB^T) slot-permuted [M][Kp]
     float *dA32n = nullptr, *dA32f = nullptr, *dBT32 = nullptr;
     int f32mode = 0;                          // the call in progress is cv_decode_batch_f32 / cv_decode_batch_dev_f32
+    int64_t f32_call_B = 0;                   // its batch size: the kernel choice is made once per call (chain_batch)
+    bool f32_range_ok = false;                // every finite model entry has |x| <= 2^64 (cv_hmm_create)
     // large-K layout
     int Kl = 0;              // K padded to a multiple of LARGE_BN
     double *dAl = nullptr;   // [Kl][Kl]

@@ -457,7 +457,9 @@ __global__ void __launch_bounds__(512, 1) decode_small_fwd_kernel(const DecodeSm
 // Why no emission lookup is needed: the reference leaves psi[t][s] = 0 when b[s][o_t] = -inf
 // (viterbi.rs:7,19-21) and otherwise stores argmax_j(delta[t-1][j] + a[j][s]).  If delta[t][s] > -inf the
 // emission was finite and the argmax is recomputed here.  If delta[t][s] = -inf then either the emission was
-// -inf (psi = 0) or every candidate was -inf (argmax of an all -inf vector = 0): psi = 0 both ways.
+// -inf (psi = 0) or every candidate was -inf (argmax of an all -inf vector = 0): psi = 0 both ways.  That needs
+// finite sums never to round to -inf: cv_hmm_create refuses finite entries beyond 2^900 (the f32 mode: 2^64), which
+// keeps every sum of fewer than 2^63 entries finite.
 // ---------------------------------------------------------------------------
 // BT_CHUNK = predecessors per prefetch chunk: 16 when the kernel has the GPU to itself (124 registers), 8 with at most
 // 64 registers for the concurrent mode, where it lives on the 16 K registers per SM two forward CTAs leave free

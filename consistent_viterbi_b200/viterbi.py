@@ -34,9 +34,10 @@ def decode_batch(hmm: HMM, obs_flat, seq_off, device: int = -1, want_scores: boo
 
 
 def decode_batch_f32(hmm: HMM, obs_flat, seq_off, device: int = -1):
-    """OPTIONAL f32 mode (cv_decode_batch_f32): the recurrence in IEEE binary32, scores within 1e-5 relative of the
-    exact mode, paths = the optimum of the f32 recurrence (may differ from the f64 path at near-ties).  Not the
-    parity path."""
+    """OPTIONAL f32 mode (cv_decode_batch_f32): the recurrence in IEEE binary32, paths = the optimum of the f32
+    recurrence (may differ from the f64 path at near-ties).  For models with every entry <= 0 a score is within about
+    2 T 2^-24 relative of the exact mode for a sequence of T steps (measured: 4.8e-7 at T = 80, 9.5e-6 at T = 20 000).
+    Not the parity path."""
     obs_flat = np.ascontiguousarray(obs_flat, dtype=np.uint32)
     seq_off = np.ascontiguousarray(seq_off, dtype=np.int64)
     B, N = seq_off.shape[0] - 1, obs_flat.shape[0]

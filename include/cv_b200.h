@@ -45,7 +45,11 @@ typedef struct cv_hmm cv_hmm;   /* device-resident model + its workspaces, one d
  * (hmm.rs:242-245).  Uploads the model to `device` (-1 = current device),
  * builds the padded/transposed device layouts the kernels read.  NaN or +inf
  * entries are rejected with CV_ERR_NAN (the reference would panic later inside
- * argmax). */
+ * argmax).  A finite entry with |x| > 2^900 is rejected with CV_ERR_UNSUPPORTED:
+ * with |x| <= 2^900 no sum of fewer than 2^63 entries reaches 2^1024, so no
+ * finite sum a kernel forms (decode, CP, CFN) overflows to +-inf and every -inf
+ * means an impossible event, as the backtraces rely on.  Real log10
+ * probabilities are >= -324, far inside the bound. */
 int  cv_hmm_create(int K, int D, const uint64_t *bdims, const double *logA,
                    const double *logB, const double *logPi, int device,
                    cv_hmm **out);
@@ -74,10 +78,13 @@ int cv_decode_batch_u16u8(cv_hmm *h, const uint16_t *obs_flat, const int64_t *se
 
 /* OPTIONAL f32 mode -- not the parity path.  The same recurrence with the model rounded to f32 once and every add an
  * IEEE binary32 add; the returned path is the exact optimum of that f32 recurrence (first-maximum backpointers),
- * score_out[b] its f32 score widened to double: within 1e-5 relative of the f64 score of cv_decode_batch, and the
- * path can differ from the f64 path where candidates are within f32 rounding of each other.  About 3-4x the
- * throughput of the exact mode (packed FADD2 / 3-input FMNMX3).  K <= 64; batches of <= 8192 sequences are decoded
- * by the exact f64 warp-per-sequence kernel.  HOST pointers / DEVICE pointers as for cv_decode_batch(_dev). */
+ * score_out[b] its f32 score widened to double (the sign of a zero score is unspecified).  The path can differ from
+ * the f64 path where candidates are within f32 rounding of each other.  For models whose entries are all <= 0 the
+ * score of a sequence of T steps is within about 2T * 2^-24 relative of the f64 score of cv_decode_batch (measured on
+ * random models, K = 45: 4.8e-7 at T = 80, 1.9e-6 at T = 2000, 9.5e-6 at T = 20000).  About 3-4x the throughput of the
+ * exact mode (packed FADD2 / 3-input FMNMX3).  K <= 64; a model with a finite entry |x| > 2^64 is CV_ERR_UNSUPPORTED
+ * (f32 sums could reach FLT_MAX).  A call of <= 8192 sequences is decoded by the exact f64 warp-per-sequence kernel,
+ * a larger call in f32 throughout.  HOST pointers / DEVICE pointers as for cv_decode_batch(_dev). */
 int cv_decode_batch_f32(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off,
                         int64_t B, uint32_t *path_out, double *score_out);
 int cv_decode_batch_dev_f32(cv_hmm *h, const uint32_t *d_obs_flat, const int64_t *d_seq_off,
