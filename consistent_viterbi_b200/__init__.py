@@ -8,8 +8,9 @@ from . import _lib
 from ._lib import CvError
 from .hmm import HMM
 from .viterbi import decode, decode_batch, decode_batch_f32, decode_batch_narrow
+from .posterior import loglik_batch, posterior_batch, score
 from .cp import CPSolver, CpDistGroup, Solver, cfn_tables, cp_solve_arrays, plan_cuts
 from .superseq import Constraints, SuperSequence, load_sequences, load_tags
 
-__all__ = ["HMM", "decode", "decode_batch", "decode_batch_narrow", "decode_batch_f32", "CPSolver", "Solver", "cp_solve_arrays", "CpDistGroup", "plan_cuts", "cfn_tables", "Constraints",
+__all__ = ["HMM", "decode", "decode_batch", "decode_batch_narrow", "decode_batch_f32", "loglik_batch", "posterior_batch", "score", "CPSolver", "Solver", "cp_solve_arrays", "CpDistGroup", "plan_cuts", "cfn_tables", "Constraints",
            "SuperSequence", "load_sequences", "load_tags", "CvError", "_lib"]

@@ -75,6 +75,9 @@ SIGNATURES = {
                          C.c_void_p, C.c_int64, C.c_int, _dp]),
     "cv_baum_welch": (C.c_int, [C.c_int, C.c_int, _u64p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_int64, C.c_int, C.c_double, C.c_int, _dp, C.POINTER(C.c_int), _i64p, _dp]),
+    "cv_loglik_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "cv_posterior_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p]),
     "cv_last_error": (C.c_char_p, []),
     "cv_launch_count": (C.c_uint64, []),
     "cv_set_timing": (None, [C.c_int]),
@@ -100,6 +103,7 @@ DEBUG_SIGNATURES = {
     "cv_debug_set_uneven_chunks": (None, [C.c_int]),
     "cv_debug_set_large_group_rb": (None, [C.c_longlong]),
     "cv_debug_set_cp_leaf_batch": (None, [C.c_int]),
+    "cv_debug_set_fb_chunk_seqs": (None, [C.c_int64]),
 }
 
 

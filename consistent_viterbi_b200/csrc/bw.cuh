@@ -101,6 +101,8 @@ __global__ void bw_prep_kernel(const BwParams p)
 
 // Forward pass.  Warp g owns states [8g, 8g+8), lane l the sequences 2l, 2l+1 of the tile: 16 cells per thread,
 // K DFMAs each per step, operands from shared memory (r_{t-1}: one LDS.128 per predecessor, a: four broadcast LDS.128).
+// HIST = false (cv_loglik_batch, fb.cuh) skips the stores of r_t and e_t to the history; the arithmetic is the same.
+template <bool HIST>
 __global__ void __launch_bounds__(32 * BW_KMAX / 8) bw_fwd_kernel(const BwParams p)
 {
     extern __shared__ __align__(16) unsigned char bw_smem[];
@@ -139,7 +141,7 @@ __global__ void __launch_bounds__(32 * BW_KMAX / 8) bw_fwd_kernel(const BwParams
                     const int e = bw_exponent(S);
                     e_prev[q] = e;
                     if (t - 1 < len[q]) {
-                        if (g == 0) p.ehist[(size_t)(slab0 + t - 1) * BW_NS + s0 + q] = e;
+                        if (HIST && g == 0) p.ehist[(size_t)(slab0 + t - 1) * BW_NS + s0 + q] = e;
                         if (t - 1 == len[q] - 1) {
                             if (g == 0) {
                                 const int64_t r = (int64_t)tile * BW_NS + s0 + q;
@@ -198,7 +200,7 @@ __global__ void __launch_bounds__(32 * BW_KMAX / 8) bw_fwd_kernel(const BwParams
             for (int k = 0; k < 8; k++) {
                 const double2 v = make_double2(acc[0][k], acc[1][k]);
                 *reinterpret_cast<double2 *>(dn + (size_t)(i0 + k) * BW_NS) = v;
-                if (i0 + k < K) *reinterpret_cast<double2 *>(hp + (size_t)(i0 + k) * BW_NS) = v;
+                if (HIST && i0 + k < K) *reinterpret_cast<double2 *>(hp + (size_t)(i0 + k) * BW_NS) = v;
             }
             *reinterpret_cast<double2 *>(sP + (size_t)(t & 1) * G * BW_NS + (size_t)g * BW_NS + s0) = make_double2(ps[0], ps[1]);
             __syncthreads();

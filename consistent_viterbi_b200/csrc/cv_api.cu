@@ -271,7 +271,7 @@ extern "C" void cv_hmm_destroy(cv_hmm *h)
     if (!h) return;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
-    for (double *p : {h->dA, h->dBT, h->dPi, h->dAl, h->dBTl, h->dATl, h->dAb, h->dBTb}) if (p) cudaFree(p);
+    for (double *p : {h->dA, h->dBT, h->dPi, h->dAl, h->dBTl, h->dATl, h->dAb, h->dBTb, h->fbA, h->fbAT, h->fbBT, h->fbPi}) if (p) cudaFree(p);
     for (float *p : {h->dA32n, h->dA32f, h->dBT32}) if (p) cudaFree(p);
     for (DevBuf *b : {&h->obs, &h->seq_off, &h->path, &h->score}) b->release();
     for (auto &w : h->ws) {

@@ -21,6 +21,7 @@ extern "C" void cv_debug_set_bt_split(int on) { g_tune.bt_split = on; }
 extern "C" void cv_debug_set_uneven_chunks(int on) { g_tune.uneven_chunks = on; }
 extern "C" void cv_debug_set_large_group_rb(long long rb) { g_tune.large_group_rb = rb; }
 extern "C" void cv_debug_set_cp_leaf_batch(int on) { g_tune.cp_leaf_batch = on; }
+extern "C" void cv_debug_set_fb_chunk_seqs(int64_t n) { g_tune.fb_chunk_seqs = n; }
 
 // ---------------------------------------------------------------------------
 // FP64 probe

@@ -55,6 +55,7 @@ struct Tuning {
     int debug = 0;                 // print launch shapes                                         (CV_DEBUG)
     int bt_prof = 0, e2e_prof = 0; // print pipeline timelines                                    (CV_BT_PROF, CV_E2E_PROF)
     long long large_group_rb = 0;  // row blocks per group of the large-K kernel, 0 = automatic    (CV_LARGE_GROUP_RB)
+    long long fb_chunk_seqs = 0;   // sequences per chunk of cv_loglik_batch / cv_posterior_batch, 0 = automatic (cv_debug_set_fb_chunk_seqs)
     int cp_fullwarp = 0, cp_prof = 0, cp_sum = -1, cp_hostpoll = 1, cp_leaf_batch = 1;   // constrained solver (CV_CP_*)
 };
 extern Tuning g_tune;
@@ -104,7 +105,13 @@ struct cv_hmm {
     double *dAl = nullptr;   // [Kl][Kl]
     double *dATl = nullptr;  // [Kl][Kl] transposed (lazy-psi backtrace)
     double *dBTl = nullptr;  // [M][Kl]
-    // host copy (control logic of the CP solver)
+    // forward-backward (fb_host.inl): probabilities (10^x, -inf -> 0) in the layouts of bw_prep_kernel, built on the
+    // first cv_loglik_batch / cv_posterior_batch call
+    double *fbA = nullptr;   // [K][Kp]
+    double *fbAT = nullptr;  // [K][Kp] transposed
+    double *fbBT = nullptr;  // [M][Kp]
+    double *fbPi = nullptr;  // [Kp]
+    // host copy (control logic of the CP solver, range check of the forward-backward calls)
     std::vector<double> hA, hB, hPi;
     // workspaces
     cvb::DevBuf obs, seq_off, path, score;   // device copies of the host-API buffers

@@ -216,6 +216,33 @@ int cv_baum_welch(int K, int D, const uint64_t *bdims, double *logA, double *log
                   double *loglik_out /* [n_iter] */, int *iters_out,
                   int64_t *skipped_out /* last iteration */, double *device_ms_out /* may be NULL */);
 
+/* ---- forward-backward inference: log-likelihood, posterior marginals, posterior decoding --------
+ * The model is the handle's log10 entries read as probabilities 10^x; as in cv_baum_welch (and unlike
+ * cv_decode_batch) pi and the first observation count.  For sequence b with positions x = seq_off[b] + t:
+ *   loglik_out[b]  = log10 P(O_b), P(O) as defined at cv_baum_welch
+ *   post_out[x*K + i] = gamma_t(i) = P(s_t = i | O_b)        (row x = position x, in the caller's order)
+ *   path_out[x]    = the lowest i at which row x of the posterior reaches its maximum (maximum posterior marginal)
+ *   pmax_out[x]    = that maximum
+ * path and pmax are taken from the same values post_out receives, so a call with post_out = NULL returns the same
+ * path.  Any output of cv_posterior_batch may be NULL; cv_loglik_batch needs loglik_out.
+ * A sequence with P(O) = 0 (also: whose scaled forward sum underflows, the rule by which cv_baum_welch skips a
+ * sequence) gets loglik -inf, posterior rows of 0.0, path 0 and pmax 0.0; the other sequences are unaffected.
+ * A sequence's outputs are the same bytes whatever batch it is in, wherever it is in that batch and however the call
+ * cuts the batch into chunks: nothing is reduced across sequences.  Two calls with the same inputs return the same
+ * bytes, and the loglik_out of cv_posterior_batch is the same bytes as that of cv_loglik_batch.
+ * Probabilities 10^x must not overflow: a model with a finite entry x > 64 is CV_ERR_UNSUPPORTED.  With every entry
+ * <= x the scaled forward rows sum to < K 10^(2x), the scaled backward vectors stay < 10^x and the normaliser
+ * Z_t = sum_i r_t(i) beta_t(i) < K 10^(3x); at x = 64, K = 64 these are < 1e130 and < 1e194.  Models of
+ * log-probabilities (entries <= 0) are never refused.
+ *   B = 0: CV_OK, nothing written   CV_ERR_EMPTY an empty sequence   CV_ERR_ARG NULL model / obs_flat / seq_off
+ *   (/ loglik_out for cv_loglik_batch), observation >= M (checked on the host before any launch)
+ *   CV_ERR_UNSUPPORTED K > 64 or an entry beyond the bound above.  HOST pointers, as for cv_decode_batch. */
+int cv_loglik_batch(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                    double *loglik_out /* [B] */);
+int cv_posterior_batch(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                       uint32_t *path_out /* [N] may be NULL */, double *pmax_out /* [N] may be NULL */,
+                       double *post_out /* [N*K] may be NULL */, double *loglik_out /* [B] may be NULL */);
+
 /* ---- plumbing --------------------------------------------------------------*/
 const char *cv_last_error(void);
 /* kernels launched by this library in this process (bench.py "gpu_launches") */

@@ -45,6 +45,9 @@ void cv_debug_set_uneven_chunks(int on);
 void cv_debug_set_large_group_rb(long long rb);
 /* constrained solver: 1 = the K sibling leaves of the last component are evaluated by one batched launch, 0 = node by node */
 void cv_debug_set_cp_leaf_batch(int on);
+/* cv_loglik_batch / cv_posterior_batch: cut the batch into chunks of n sequences (0 = automatic: chunks whose history
+ * and device outputs fit half the free device memory) */
+void cv_debug_set_fb_chunk_seqs(int64_t n);
 
 /* Parity hooks for the CP path: after cv_cp_solve, copy out the final delta[N*K] / psi[N*K] state and the per-node
  * upper bounds (first `cap` nodes). */
