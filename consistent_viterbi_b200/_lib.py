@@ -104,6 +104,9 @@ DEBUG_SIGNATURES = {
     "cv_debug_set_large_group_rb": (None, [C.c_longlong]),
     "cv_debug_set_cp_leaf_batch": (None, [C.c_int]),
     "cv_debug_set_fb_chunk_seqs": (None, [C.c_int64]),
+    "cv_debug_set_certified": (None, [C.c_int]),
+    "cv_debug_set_cert_tolerance": (None, [C.c_double]),
+    "cv_debug_last_flagged": (C.c_int64, [C.c_void_p]),
 }
 
 

@@ -167,6 +167,13 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     auto model_beyond = [&](double lim) { return beyond(logA, (int64_t)K * K, lim) || beyond(logB, (int64_t)K * M, lim) || beyond(logPi, K, lim); };
     if (model_beyond(0x1p900)) return fail(CV_ERR_UNSUPPORTED, "model entry with |x| > 2^900 (sums could overflow)");
     const bool f32_range_ok = !model_beyond(0x1p64);
+    auto nonpositive = [](const double *v, int64_t n) {
+        for (int64_t i = 0; i < n; i++) if (std::isfinite(v[i]) && v[i] > 0.0) return false;
+        return true;
+    };
+    // log-probabilities (every finite entry <= 0, -0.0 included) within the f32 range: the exact decode may certify an
+    // f32 forward pass (decode_small.cuh, certified backtrace); any other model keeps the f64 forward pass
+    const bool cert_ok = K <= SMALL_K_MAX && f32_range_ok && nonpositive(logA, (int64_t)K * K) && nonpositive(logB, (int64_t)K * M);
     if (device < 0) {
         int rc = check_device(0);
         if (rc) return rc;
@@ -180,6 +187,7 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     struct Guard { cv_hmm *h; ~Guard() { if (h) cv_hmm_destroy(h); } } guard{h};   // released on every early return
     h->device = device; h->K = K; h->D = D; h->M = M;
     h->f32_range_ok = f32_range_ok;
+    h->cert_ok = cert_ok;
     // state groups of the forward tile kernel: G = ceil(K/8) warps of TQ = 8 target states, Kp = 8 G
     h->G = (K + TQ - 1) / TQ;
     h->Kp = h->G * TQ;
@@ -276,7 +284,7 @@ extern "C" void cv_hmm_destroy(cv_hmm *h)
     for (DevBuf *b : {&h->obs, &h->seq_off, &h->path, &h->score}) b->release();
     for (auto &w : h->ws) {
         for (DevBuf *b : {&w.order, &w.keys_in, &w.keys_out, &w.vals_in, &w.cub_tmp, &w.hist, &w.tmax, &w.base, &w.misc,
-                          &w.lg_arr, &w.lg_start, &w.lg_done, &w.delta_g, &w.is_long, &w.long_list, &w.long_psi})
+                          &w.lg_arr, &w.lg_start, &w.lg_done, &w.delta_g, &w.is_long, &w.long_list, &w.long_psi, &w.cert_list})
             b->release();
         if (w.st) cudaStreamDestroy(w.st);
         if (w.done) cudaEventDestroy(w.done);
@@ -498,13 +506,14 @@ static int launch_chain_kernel(const cv_hmm *h, const DecodeChainParams &p, int 
 
 static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, int64_t B,
                                int64_t N, uint32_t *d_path, double *d_score, unsigned int *d_counter, int *d_status,
-                               int64_t max_len, cudaStream_t st, bool timing, const StreamedIO *sio = nullptr,
+                               int64_t max_len, cudaStream_t st, bool timing, bool cert, const StreamedIO *sio = nullptr,
                                const LongSplit *ls = nullptr)
 {
     const int G = h->G;
     const uint32_t *d_order = (const uint32_t *)w.order.p, *d_sorted_len = (const uint32_t *)w.keys_out.p;
-    // optional f32 mode (decode_f32.cuh): its own forward kernel, f32 history, f32 backtrace
-    const bool f32 = h->f32mode != 0;
+    // optional f32 mode (decode_f32.cuh): its own forward kernel, f32 history, f32 backtrace.  cert: the same forward
+    // kernel and history, then the certified backtrace (decode_small.cuh) -- the exact decode of an eligible model
+    const bool f32 = h->f32mode != 0 || cert;
     // tiles of NS = 64 sequences (TP = 2 per lane), one warp per state group
     const int NS = 32 * TP, threads = 32 * G;
     size_t smem = f32 ? decode_f32_smem_bytes(h->K, h->Kp) : decode_small_smem_bytes(h->K, h->Kp, NS);
@@ -548,6 +557,9 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     p.obs16 = h->obs16; p.path8 = h->path8; p.em_light = g_tune.em_light;
     p.is_long = (ls && ls->lstar) ? ls->is_long : nullptr;
     p.A32s = h->dA32f; p.A32n = h->dA32n; p.BT32 = h->dBT32;
+    p.cert_list = cert ? (uint32_t *)w.cert_list.p : nullptr;
+    p.cert_count = cert ? (unsigned int *)w.misc.p + 10 : nullptr;      // zeroed by the caller with the rest of misc
+    p.cert_tol = g_tune.cert_tol;
     if ((f32 || g_tune.balanced_split) && h->dAb) {
         p.At = h->dAb; p.BTt = h->dBTb; p.nq_base = h->K / G; p.nq_rem = h->K % G;
     }
@@ -581,8 +593,8 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     }
     const int grid = (int)std::min<int64_t>((int64_t)h->num_sms * occ, ntiles);
     if (g_tune.debug)
-        fprintf(stderr, "[cv] decode_small: K=%d G=%d f32=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
-                h->K, G, (int)f32, threads, smem, occ, grid, ntiles);
+        fprintf(stderr, "[cv] decode_small: K=%d G=%d f32=%d cert=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
+                h->K, G, (int)f32, (int)cert, threads, smem, occ, grid, ntiles);
     // Concurrent backtrace: the backtrace kernel runs next to the forward kernel on a second stream and follows
     // it tile by tile (tile_done flags).  It is released only when every forward CTA is resident (stream wait on
     // the `started` counter), so its spinning CTAs can never keep a forward CTA off an SM; it then lives on the
@@ -628,8 +640,10 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     if (timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev1, st));
     // end state + backtrace with lazy backpointers: one thread per sequence
     const size_t smem_bt = (size_t)h->K * (h->K | 1) * 8 + 16 * 8;      // + one chunk of padding behind the last row
-    void (*bt_seq)(DecodeSmallParams) = f32 ? backtrace_small_kernel<16, 4, float> : backtrace_small_kernel<16, 4>;
-    void (*bt_con)(DecodeSmallParams) = f32 ? backtrace_small_kernel<8, 8, float> : backtrace_small_kernel<8, 8>;
+    void (*bt_seq)(DecodeSmallParams) = cert ? backtrace_small_kernel<16, 4, float, true>
+                                      : f32 ? backtrace_small_kernel<16, 4, float> : backtrace_small_kernel<16, 4>;
+    void (*bt_con)(DecodeSmallParams) = cert ? backtrace_small_kernel<8, 8, float, true>
+                                      : f32 ? backtrace_small_kernel<8, 8, float> : backtrace_small_kernel<8, 8>;
     // Four lanes per sequence (backtrace_split_kernel, f64 only) -- for batches that do
     // not fill the GPU for long (a rank's slice of a sharded batch): there the one-thread-per-sequence kernel is latency
     // bound and most of its work is still open when the forward kernel ends.  Measured, device step with the concurrent
@@ -681,17 +695,75 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
 // that bound for the exact mode.  The f32 mode keeps it whatever the override says, and applies it to the whole call,
 // not to one chunk: cv_b200.h promises such calls the exact f64 kernel, and every larger call the f32 kernels in all
 // its chunks (a forced small chunk count must not hand part of an f32 call to the f64 kernel).
+constexpr int64_t CHAIN_BATCH_MAX = 8192;
 static bool chain_batch(const cv_hmm *h, int64_t B)
 {
-    if (h->f32mode) return h->K <= SMALL_K_MAX && h->f32_call_B <= 8192;
-    const long long bound = g_tune.chain_max_b < 0 ? 8192 : g_tune.chain_max_b;
+    if (h->f32mode) return h->K <= SMALL_K_MAX && h->f32_call_B <= CHAIN_BATCH_MAX;
+    const long long bound = g_tune.chain_max_b < 0 ? CHAIN_BATCH_MAX : g_tune.chain_max_b;
     return h->K <= SMALL_K_MAX && B <= bound;
 }
 
+// sort keys of the sequences in list[0, n): length, id
+__global__ void listed_len_keys_kernel(const int64_t *seq_off, const uint32_t *list, int64_t n, uint32_t *keys, uint32_t *vals)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t b = list[i];
+    keys[i] = (uint32_t)(seq_off[b + 1] - seq_off[b]);
+    vals[i] = b;
+}
+
+// Exact f64 re-decode of the sequences the certified backtrace could not certify (launch_decode_small with cert): their
+// paths and scores are overwritten.  This is the one host round trip of a certified call: the flagged count, their
+// longest length and their elements are read back, and decide the kernel -- the warp-per-sequence kernel for as many
+// sequences as a batch would give it (chain_batch), else the f64 tile path over the flagged sequences ordered by length.
+static int certified_fallback(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, uint32_t *d_path,
+                              double *d_score, int *d_status, cudaStream_t st)
+{
+    unsigned int *d_count = (unsigned int *)w.misc.p + 10;                  // cert_count of launch_decode_small
+    unsigned int *hc = (unsigned int *)((char *)h->pinned_status + 64);
+    CUDA_TRY(cudaMemcpyAsync(hc, d_count, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    const int64_t n = hc[0], lmax = hc[1];
+    const int64_t nel = (int64_t)*reinterpret_cast<const unsigned long long *>(hc + 2);
+    h->last_flagged = n;
+    if (n == 0) return CV_OK;
+    const uint32_t *list = (const uint32_t *)w.cert_list.p;
+    int rc;
+    if (n <= CHAIN_BATCH_MAX) {
+        // the f32 history is no longer needed: its buffer takes the backpointer rows
+        if ((rc = w.hist.ensure((size_t)n * (size_t)lmax * h->Kp + 64))) return rc;
+        DecodeChainParams q;
+        q.A = h->dA; q.BT = h->dBT; q.obs = d_obs; q.seq_off = d_off; q.order = list;
+        q.psi = (uint8_t *)w.hist.p; q.path = d_path; q.score = d_score;
+        q.counter = (unsigned int *)w.misc.p + 14; q.status = d_status;
+        q.M = h->M; q.B = n; q.K = h->K; q.Kp = h->Kp;
+        q.bt_in_smem = ((size_t)h->M * h->Kp * 8 <= CHAIN_BT_SMEM_MAX) ? 1 : 0;
+        q.obs16 = h->obs16; q.path8 = h->path8;
+        q.B_dev = d_count; q.psi_stride = lmax;
+        q.chunk_done = nullptr; q.nch = 0;
+        const int grid = (int)std::min<int64_t>((n + DC_WARPS - 1) / DC_WARPS, (int64_t)h->num_sms * 8);
+        return launch_chain_kernel(h, q, grid, st);
+    }
+    listed_len_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, list, n, (uint32_t *)w.keys_in.p, (uint32_t *)w.vals_in.p);
+    g_launches++;
+    const int end_bit = key_bits(lmax);
+    size_t tmp_bytes = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
+                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
+    if ((rc = w.cub_tmp.ensure(tmp_bytes))) return rc;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
+                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
+    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, sizeof(unsigned int), st));        // tile counter
+    return launch_decode_small(h, w, d_obs, d_off, n, nel, d_path, d_score, (unsigned int *)w.misc.p, d_status, lmax, st,
+                               false, false);
+}
+
 // One chunk of sequences [0, B) of d_off (offsets are absolute into d_obs / d_path): order by length,
-// forward, backtrace; everything enqueued on `st` with workspace set `w`.
+// forward, backtrace; everything enqueued on `st` with workspace set `w`.  can_certify: the chunk is the whole call
+// (certified_fallback's host round trip is made once per call).
 static int decode_chunk(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                        int64_t max_len, uint32_t *d_path, double *d_score, cudaStream_t st, bool timing)
+                        int64_t max_len, uint32_t *d_path, double *d_score, cudaStream_t st, bool timing, bool can_certify)
 {
     int rc;
     if (B > 0x7fffffffLL) return fail(CV_ERR_UNSUPPORTED, "more than 2^31 sequences in one chunk");
@@ -736,8 +808,16 @@ static int decode_chunk(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int
         if (timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
         return CV_OK;
     }
-    if (h->K <= SMALL_K_MAX)
-        return launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, st, timing, nullptr, &ls);
+    if (h->K <= SMALL_K_MAX) {
+        const bool cert = can_certify && h->cert_ok && !h->f32mode && g_tune.certified;
+        if (cert && (rc = w.cert_list.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
+        if ((rc = launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, st, timing, cert, nullptr, &ls)))
+            return rc;
+        if (!cert) return CV_OK;
+        if ((rc = certified_fallback(h, w, d_obs, d_off, d_path, d_score, d_status, st))) return rc;
+        if (timing) CUDA_TRY(cudaEventRecord(h->ev2, st));               // backtrace time = backtrace + fallback
+        return CV_OK;
+    }
     if (timing) CUDA_TRY(cudaEventRecord(h->ev0, st));
     if ((rc = launch_decode_large(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, st))) return rc;
     if (timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
@@ -818,12 +898,13 @@ static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t
     if (B == 0) return CV_OK;
     if (!d_obs || !d_off || !d_path) return fail(CV_ERR_ARG, "NULL buffer");
     CUDA_TRY(cudaSetDevice(h->device));
+    h->last_flagged = -1;
     cudaStream_t user = (cudaStream_t)stream;
     const bool timing = g_timing.load() != 0;
     const int nch = chunk_count(h, B, timing, false);
     int rc;
     if (nch == 1) {
-        if ((rc = decode_chunk(h, h->ws[0], d_obs, d_off, B, N, max_len, d_path, d_score, user, timing))) return rc;
+        if ((rc = decode_chunk(h, h->ws[0], d_obs, d_off, B, N, max_len, d_path, d_score, user, timing, true))) return rc;
     } else {
         // fork: chunk k runs on internal stream k % 2 so that backtrace(k) overlaps forward(k+1)
         if (max_len <= 0) return fail(CV_ERR_ARG, "max_len is required for the chunked device path");
@@ -833,7 +914,7 @@ static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t
             const int64_t b0 = B * k / nch, b1 = B * (k + 1) / nch;
             DecodeWs &w = h->ws[k & 1];
             if ((rc = decode_chunk(h, w, d_obs, d_off + b0, b1 - b0, N, max_len, d_path,
-                                   d_score ? d_score + b0 : nullptr, w.st, false)))
+                                   d_score ? d_score + b0 : nullptr, w.st, false, false)))
                 return rc;
         }
         for (int k = 0; k < 2; k++) {
@@ -997,7 +1078,7 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
                                                        (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)B, 0, end_bit, sk));
     if (prof) cudaEventRecord(pe[2], sk);
-    if ((rc = launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, sk, false, &sio, &ls))) return rc;
+    if ((rc = launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, sk, false, false, &sio, &ls))) return rc;
     if (prof) cudaEventRecord(pe[3], sk);
     // paths / scores of chunk c leave as soon as the backtrace has counted all its sequences
     CUDA_TRY(cudaStreamWaitEvent(s_out, w.ev_pre, 0));
@@ -1080,6 +1161,7 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
     if (seq_off[0] != 0) return fail(CV_ERR_ARG, "seq_off[0] must be 0");
     const int64_t N = seq_off[B];
     CUDA_TRY(cudaSetDevice(h->device));
+    h->last_flagged = -1;
     int rc;
     if ((rc = h->obs.ensure(sizeof(uint32_t) * (size_t)N))) return rc;
     if ((rc = h->seq_off.ensure(sizeof(int64_t) * (size_t)(B + 1)))) return rc;
@@ -1122,7 +1204,7 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
         mark(st);
         CUDA_TRY(cudaMemcpyAsync((char *)d_obs + ob * e0, (const char *)obs_flat + ob * e0, ob * (size_t)(e1 - e0), cudaMemcpyHostToDevice, st));
         mark(st);
-        if ((rc = decode_chunk(h, w, d_obs, d_off + b0, b1 - b0, e1 - e0, max_len, d_path, d_score + b0, st, timing))) return rc;
+        if ((rc = decode_chunk(h, w, d_obs, d_off + b0, b1 - b0, e1 - e0, max_len, d_path, d_score + b0, st, timing, nck == 1))) return rc;
         mark(st);
         CUDA_TRY(cudaMemcpyAsync((char *)path_out + pb * e0, (const char *)d_path + pb * e0, pb * (size_t)(e1 - e0), cudaMemcpyDeviceToHost, st));
         if (score_out)

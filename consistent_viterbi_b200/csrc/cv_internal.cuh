@@ -57,6 +57,8 @@ struct Tuning {
     long long large_group_rb = 0;  // row blocks per group of the large-K kernel, 0 = automatic    (CV_LARGE_GROUP_RB)
     long long fb_chunk_seqs = 0;   // sequences per chunk of cv_loglik_batch / cv_posterior_batch, 0 = automatic (cv_debug_set_fb_chunk_seqs)
     int cp_fullwarp = 0, cp_prof = 0, cp_sum = -1, cp_hostpoll = 1, cp_leaf_batch = 1;   // constrained solver (CV_CP_*)
+    int certified = 1;             // eligible models: f32 forward pass + certified backtrace + exact fallback (cv_debug_set_certified)
+    double cert_tol = 1.0;         // scale of the certified backtrace's error bound (cv_debug_set_cert_tolerance)
 };
 extern Tuning g_tune;
 
@@ -100,6 +102,10 @@ struct cv_hmm {
     int f32mode = 0;                          // the call in progress is cv_decode_batch_f32 / cv_decode_batch_dev_f32
     int64_t f32_call_B = 0;                   // its batch size: the kernel choice is made once per call (chain_batch)
     bool f32_range_ok = false;                // every finite model entry has |x| <= 2^64 (cv_hmm_create)
+    // the exact decode may run the f32 forward pass and certify it (decode_small.cuh, certified backtrace): K <= 64,
+    // f32_range_ok and every finite entry of logA / logB <= 0
+    bool cert_ok = false;
+    int64_t last_flagged = -1;                // sequences the last decode call re-decoded in f64; -1: not certified
     // large-K layout
     int Kl = 0;              // K padded to a multiple of LARGE_BN
     double *dAl = nullptr;   // [Kl][Kl]
@@ -120,6 +126,7 @@ struct cv_hmm {
     struct DecodeWs {
         cvb::DevBuf order, keys_in, keys_out, vals_in, cub_tmp, hist, tmax, base, misc, lg_arr, lg_start, lg_done, delta_g;
         cvb::DevBuf is_long, long_list, long_psi;          // long-sequence split of the tile path (cv_api.cu)
+        cvb::DevBuf cert_list;                             // sequences the certified backtrace could not certify
         cudaStream_t st = nullptr;
         cudaEvent_t done = nullptr;
         cudaStream_t st_bt = nullptr;                      // concurrent backtrace (launch_decode_small)

@@ -13,6 +13,10 @@
 // decode_small_fwd_kernel (persistent CTAs, tiles of 64 sequences, a lane owns 2 adjacent sequences, a warp one group
 // of <= 8 target states of the balanced split, emission rows by TMA, one TMA bulk store of the [K][64] slab per step),
 // at half the shared memory (46 KB at K = 45: four CTAs per SM).
+//
+// The exact decode of an eligible model (cv_hmm_create: every finite entry <= 0 and |x| <= 2^64) runs this kernel as
+// well: backtrace_small_kernel<.., float, true> then certifies every backpointer against the f64 recurrence (the
+// bound is derived above that kernel) and the sequences it cannot certify are decoded again in f64.
 #pragma once
 
 #include "decode_small.cuh"
@@ -107,6 +111,7 @@ __global__ void __launch_bounds__(256, 3) decode_f32_fwd_kernel(const DecodeSmal
                 const uint32_t b = p.order[r];
                 off = p.seq_off[b];
                 len = (int)(p.seq_off[b + 1] - off);
+                if (p.is_long && p.is_long[b]) len = 0;              // decoded by the warp-per-sequence kernel
             }
             sOff[s] = off; sLen[s] = len;
         }

@@ -87,6 +87,12 @@ struct DecodeSmallParams {
     // long-sequence split: sequences flagged here are decoded by the warp-per-sequence kernel, the tile kernels treat
     // them as inactive slots (nullptr: no split)
     const uint8_t *is_long;
+    // certified backtrace (backtrace_small_kernel<.., float, true>): the ids of the sequences it could not certify are
+    // appended to cert_list; cert_count[0] = how many, [1] = their longest length, [2..3] = their elements (u64).
+    // cert_tol scales the error bound: 1 = the derived bound, 0 = certify every decision, inf = none.
+    uint32_t *cert_list;
+    unsigned int *cert_count;
+    double cert_tol;
 };
 
 // element `idx` of the observation array (u32, or u16 when obs16); `coherent`: the copy engine is still writing the
@@ -103,6 +109,11 @@ __device__ __forceinline__ void store_path_at(const DecodeSmallParams &p, int64_
 {
     if (p.path8) reinterpret_cast<uint8_t *>(p.path)[idx] = (uint8_t)state;
     else p.path[idx] = state;
+}
+// reads back a state this thread stored (plain load: the read-only path could serve a stale line)
+__device__ __forceinline__ uint32_t load_path_at(const DecodeSmallParams &p, int64_t idx)
+{
+    return p.path8 ? (uint32_t)reinterpret_cast<const uint8_t *>(p.path)[idx] : p.path[idx];
 }
 
 __host__ __device__ inline int em_pitch(int Kp) { return Kp + 2; }   // doubles; bank-conflict-free row pitch
@@ -494,22 +505,66 @@ __device__ __forceinline__ void bt_mark_done_warp(const DecodeSmallParams &p, in
 template <typename T>
 __device__ __forceinline__ T bt_ld(const T *q) { return __ldcg(q); }
 
+// ---------------------------------------------------------------------------
+// Certified backtrace (CERT = true, T = float): the exact f64 decode from the f32 history of decode_f32_fwd_kernel.
+//
+// Model (cv_hmm_create, cv_hmm::cert_ok): every finite entry of logA / logB is <= 0 and has |x| <= 2^64.  Then every
+// delta and every candidate is <= 0, no finite sum of fewer than 2^63 entries overflows in f32 or f64, and the f32 and
+// f64 recurrences have the same -inf pattern (a cell is -inf iff every path into it holds a -inf entry).  On values of
+// one sign fl(x + y) and max are monotone, so with C = the exact max-plus value of a cell (real arithmetic on the f64
+// entries) and n roundings along the way, a rounded result lies in [C (1+u)^n, C (1-u)^n], plus an absolute term for
+// entries that rn32 puts in the f32 subnormal range (|error| <= 2^-150 each; an add whose result is subnormal is exact).
+//
+// Decision at step t (t = tt for the backpointer of step tt, whose candidates fl(delta[tt-1][j] + a[j][cur]) take 2tt-1
+// adds; t = len-1 for the end state): the f32 candidate carries <= 2t roundings of u32 = 2^-24 (adds plus the one
+// rounding of the entries), the f64 candidate <= 2t of u64 = 2^-53.  Let v = the f32 first maximum (index m) and
+// r = the largest other f32 candidate.  For j != m: c64[j] <= c32[j] (1-e64)/(1+e32) <= r + |r| E, and
+// c64[m] >= v - |v| E, with E = (1+u32)^(2t) (1+u64)^(2t) / (1 - ...) - 1 <= (2t+2) u32 while (2t+2) u32 < 1/2.  So
+//     v - r > E (|v| + |r|) + 2 eta,   eta = 2t 2^-150 (times at most 2 for the relative factors),
+// makes c64[m] strictly the largest f64 candidate: the f64 first-argmax is m as well.  The test below uses
+//     v - r > s ((2t+4) 2^-23 (|v| + |r|) + (2t+2) 2^-148),   s = cert_tol (1 by default),
+// a factor of 2 over E and 2 eta, which also absorbs the f64 rounding of the test itself (a few 2^-53 relative);
+// the gap is evaluated in f64.  A runner-up of -inf (one finite candidate) always passes: the f64 row has the same single
+// finite candidate.  A decision with delta[tt][cur] = -inf is psi = 0 in both recurrences and needs no test.
+//
+// If every decision of a path passes, the f32 path is the f64 path, and along it every f64 maximum is the path's own
+// candidate, so the f64 score is the chain  d = fl(fl(d + a[p(t-1)][p(t)]) + b[p(t)][o(t)])  from d = 0.0 -- bit for bit
+// what the f64 forward kernel computes (a -inf along the way stays -inf: the -inf => psi = 0 rule puts a -inf term in the
+// chain).  A sequence with a failed test is appended to cert_list and decoded again by the exact f64 kernels.
+// ---------------------------------------------------------------------------
+__device__ __forceinline__ bool cert_pass(float v, float r, int t, double tol)
+{
+    if (!(r > -INFINITY) || tol == 0.0) return true;
+    const double dv = v, dr = r;
+    return dv - dr > tol * ((2.0 * t + 4.0) * 0x1p-23 * (fabs(dv) + fabs(dr)) + (2.0 * t + 2.0) * 0x1p-148);
+}
+
 // History slabs [K][64] (decode_small_fwd_kernel, decode_f32_fwd_kernel); the tile size is a compile-time constant
 // so that the load offsets become immediates.
 // T = double (exact, the reference's arithmetic) or float (cv_decode_batch_f32: the f32 history of decode_f32.cuh and
-// rn32(logA), same first-maximum rule on fl32 sums)
-template <int BT_CHUNK, int MINB, typename T = double>
+// rn32(logA), same first-maximum rule on fl32 sums).  CERT (T = float only): the certified backtrace described above.
+template <int BT_CHUNK, int MINB, typename T = double, bool CERT = false>
 __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const DecodeSmallParams p)
 {
+    static_assert(!CERT || sizeof(T) == 4, "the certified backtrace reads the f32 history");
     const T NEG = (T)neg_inf();
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int NS = 64;
     const int K = p.K, Kp = p.Kp;
     const int ATP = K | 1;                                   // odd pitch: rows of different states spread over banks
     T *sAT = reinterpret_cast<T *>(smem_raw);               // sAT[s*ATP + j] = logA[j][s]
-    for (int e = threadIdx.x; e < K * Kp; e += blockDim.x) {
-        const int j = e / Kp, s = e % Kp;
-        if (s < K) sAT[(size_t)s * ATP + j] = sizeof(T) == 4 ? (T)p.A32n[e] : (T)p.A[e];
+    if (CERT) {
+        // padding columns and the chunk padding behind the last row are zeros: they meet -inf operands only, and the
+        // runner-up must never see a NaN
+        for (int e = threadIdx.x; e < K * ATP + BT_CHUNK; e += blockDim.x) {
+            const int s = e / ATP, j = e % ATP;
+            sAT[e] = (s < K && j < K) ? (T)p.A32n[(size_t)j * Kp + s] : (T)0;
+        }
+    } else {
+        for (int e = threadIdx.x; e < K * Kp; e += blockDim.x) {
+            const int j = e / Kp, s = e % Kp;
+            if (s < K) sAT[(size_t)s * ATP + j] = sizeof(T) == 4 ? (T)p.A32n[e] : (T)p.A[e];
+        }
     }
     __syncthreads();
 
@@ -551,16 +606,45 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
         if (len <= 0 || p.tile_base[tile] + (long long)len > p.hist_cap_slabs) return my_chunk;   // tile refused by the forward kernel (status 7)
         const T *col = reinterpret_cast<const T *>(p.hist) + (size_t)p.tile_base[tile] * sl + (size_t)s;   // sequence s of slab 0
 
+        // certified backtrace: every decision passed its test so far (inf tolerance: none does)
+        bool ok = p.cert_tol < INFINITY;
+        // certified: the f64 score along the decoded path, or the sequence goes to the exact fallback
+        auto cert_finish = [&]() {
+            if (!ok) {
+                p.cert_list[atomicAdd(p.cert_count, 1u)] = b;
+                atomicMax(p.cert_count + 1, (unsigned int)len);
+                atomicAdd(reinterpret_cast<unsigned long long *>(p.cert_count + 2), (unsigned long long)len);
+                return;
+            }
+            if (!p.score) return;
+            double d = 0.0;                                   // viterbi.rs:6
+            uint32_t prev = load_path_at(p, off);
+#pragma unroll 4
+            for (int t = 1; t < len; t++) {
+                const uint32_t st = load_path_at(p, off + t);
+                uint32_t o = load_obs_at(p, off + t, false);
+                if ((int64_t)o >= p.M) o = 0;                    // reported by the forward kernel (status 3)
+                d = (d + __ldg(p.A + (size_t)prev * Kp + st)) + __ldg(p.BT + (size_t)o * Kp + st);   // viterbi.rs:17
+                prev = st;
+            }
+            p.score[b] = d;
+        };
+
         // end state: argmax of the last row (viterbi.rs:24)
         const T *row = col + (size_t)(len - 1) * sl;
-        T bv = bt_ld(row); int cur = 0;
+        T bv = bt_ld(row), br = NEG; int cur = 0;
         for (int j = 1; j < K; j++) {
             const T v = bt_ld(row + (size_t)j * NS);
+            if (CERT) br = max(br, min(v, bv));            // runner-up: the largest value that is not the first maximum
             if (v > bv) { bv = v; cur = j; }
         }
-        if (p.score) p.score[b] = (double)bv;
+        if (CERT) ok = ok && (!(bv > NEG) || cert_pass(bv, br, len - 1, p.cert_tol));
+        else if (p.score) p.score[b] = (double)bv;
         store_path_at(p, off + len - 1, (uint32_t)cur);
-        if (len == 1) return my_chunk;
+        if (len == 1) {
+            if (CERT) cert_finish();
+            return my_chunk;
+        }
 
         // walk back (viterbi.rs:27-30): steps tt = len-1 .. 1, each a scan of row tt-1 in chunks of BT_CHUNK predecessors;
         // the next chunk (of this step, or the first of the next step -- rows do not depend on the path) is always
@@ -579,18 +663,20 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
                 for (int k = 0; k < BT_CHUNK; k++) dst[k] = (k < ktail) ? bt_ld(q + (size_t)k * NS) : NEG;
             }
         };
-        T mv = 0; int mi = 0;
+        T mv = 0, rv = NEG; int mi = 0;
         const T *at = sAT;
         // chunk c of the current step: candidates fl(delta[tt-1][j] + logA[j][cur]), first maximum (viterbi.rs:15-16);
         // predecessors >= K hold -inf and can never be strictly greater (logA is read up to BT_CHUNK-1 doubles past
-        // K: padded)
+        // K: padded).  CERT: rv = the runner-up (the largest candidate other than the first maximum)
         auto reduce_chunk = [&](const T (&cu)[BT_CHUNK], int c) {
             const T *ac = at + c * BT_CHUNK;
             if (c == 0) {
                 mv = cu[0] + ac[0]; mi = 0;
+                if (CERT) rv = NEG;
 #pragma unroll
                 for (int k = 1; k < BT_CHUNK; k++) {
                     const T v = cu[k] + ac[k];
+                    if (CERT) rv = max(rv, min(v, mv));
                     if (v > mv) { mv = v; mi = k; }
                 }
             } else {
@@ -598,6 +684,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
 #pragma unroll
                 for (int k = 0; k < BT_CHUNK; k++) {
                     const T v = cu[k] + ac[k];
+                    if (CERT) rv = max(rv, min(v, mv));
                     if (v > mv) { mv = v; mi = j0 + k; }
                 }
             }
@@ -619,6 +706,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
                 reduce_chunk(X, c);
             }
             // psi = 0 when delta[tt][cur] = -inf (emission -inf or all candidates -inf; see header comment)
+            if (CERT && dcur > NEG) ok = ok && cert_pass(mv, rv, tt, p.cert_tol);
             cur = (dcur > NEG) ? mi : 0;
             dcur = __ldcg(rowp + (size_t)cur * NS);              // delta[tt-1][cur]
             store_path_at(p, pout, (uint32_t)cur);
@@ -632,6 +720,7 @@ __global__ void __launch_bounds__(128, MINB) backtrace_small_kernel(const Decode
         } else {
             for (int tt = len - 1; tt >= 1; tt--) step(bufA, bufB, tt);
         }
+        if (CERT) cert_finish();
         return my_chunk;
         }();
         bt_mark_done_warp(p, done_chunk);

@@ -104,7 +104,10 @@ int cv_decode_batch_keep(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq
  * that the status word is read back when `sync_status` != 0.
  * N = d_seq_off[B]; max_len = an upper bound on the sequence lengths (sizes the workspace, and the ordering of the
  * batch by length only looks at the bits such a length can have), <= 0 = not known (one extra synchronisation reads it
- * back).  A sequence longer than a positive max_len is CV_ERR_ARG. */
+ * back).  A sequence longer than a positive max_len is CV_ERR_ARG.
+ * K <= 64, more than 8192 sequences, a model of log-probabilities (every finite logA / logB entry <= 0, |x| <= 2^64):
+ * the call also waits once for `stream` -- the exact result comes from an f32 forward pass whose backpointers are
+ * certified against the f64 recurrence, and the host reads back how many sequences need an f64 re-decode. */
 int cv_decode_batch_dev(cv_hmm *h, const uint32_t *d_obs_flat, const int64_t *d_seq_off,
                         int64_t B, int64_t N, int64_t max_len, uint32_t *d_path_out,
                         double *d_score_out, void *stream, int sync_status);

@@ -48,6 +48,16 @@ void cv_debug_set_cp_leaf_batch(int on);
 /* cv_loglik_batch / cv_posterior_batch: cut the batch into chunks of n sequences (0 = automatic: chunks whose history
  * and device outputs fit half the free device memory) */
 void cv_debug_set_fb_chunk_seqs(int64_t n);
+/* exact decode, K <= 64, of a model of log-probabilities (every finite entry of logA / logB <= 0, |x| <= 2^64): 1 (default) =
+ * f32 forward pass, backtrace that certifies every backpointer against the f64 recurrence, exact f64 re-decode of the
+ * sequences it cannot certify; 0 = the f64 forward pass for every model */
+void cv_debug_set_certified(int on);
+/* scale of the certified backtrace's error bound: 1 (default) = the derived bound, 0 = certify every decision (the
+ * f32 path is taken as it is -- NOT exact), INFINITY = certify none (every sequence goes to the f64 fallback) */
+void cv_debug_set_cert_tolerance(double scale);
+/* sequences the last decode call on h re-decoded in f64 after the certified backtrace; -1 = that call did not take
+ * the certified path */
+int64_t cv_debug_last_flagged(const cv_hmm *h);
 
 /* Parity hooks for the CP path: after cv_cp_solve, copy out the final delta[N*K] / psi[N*K] state and the per-node
  * upper bounds (first `cap` nodes). */
