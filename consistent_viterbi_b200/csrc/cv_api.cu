@@ -201,7 +201,7 @@ extern "C" int cv_hmm_create(int K, int D, const uint64_t *bdims, const double *
     CUDA_TRY(cudaEventCreate(&h->ev0));
     CUDA_TRY(cudaEventCreate(&h->ev1));
     CUDA_TRY(cudaEventCreate(&h->ev2));
-    CUDA_TRY(cudaMallocHost(&h->pinned_status, 2048));     // [0, 64): status / bound words, [1024, 2048): leaf-batch bounds
+    CUDA_TRY(cudaMallocHost(&h->pinned_status, PIN_BYTES));     // laid out as PinnedAt (cv_internal.cuh)
     CUDA_TRY(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     CUDA_TRY(cudaStreamCreateWithFlags(&h->st_long, cudaStreamNonBlocking));
     CUDA_TRY(cudaEventCreateWithFlags(&h->ev_long_dep, cudaEventDisableTiming));
@@ -320,6 +320,23 @@ extern "C" void cv_host_free(void *p) { if (p) cudaFreeHost(p); }
 // ---------------------------------------------------------------------------
 // batched plain Viterbi
 // ---------------------------------------------------------------------------
+typedef cv_hmm::DecodeWs DecodeWs;
+
+// Options of one decode call.  Each public decode entry point builds one and passes it down, so that a function's
+// signature shows which precision and which formats it serves.
+struct DecodeCall {
+    bool f32;              // cv_decode_batch_f32 / cv_decode_batch_dev_f32
+    int64_t B;             // the call's batch size: the f32 mode picks its kernel once per call (chain_batch)
+    int obs16, path8;      // narrow formats: u16 observations (cv_decode_batch_u16u8), u8 states (and cv_decode_batch_dev_u8)
+    bool timing;           // cv_set_timing, read once when the call starts
+    size_t obs_bytes() const { return obs16 ? 2 : 4; }     // per element of the caller's host buffers
+    size_t path_bytes() const { return path8 ? 1 : 4; }
+};
+static DecodeCall decode_call(int64_t B, bool f32 = false, int obs16 = 0, int path8 = 0)
+{
+    return DecodeCall{f32, B, obs16, path8, g_timing.load() != 0};
+}
+
 // Long-sequence split (launch_decode_small): the tile kernel runs a tile in lock step for as many steps as its longest
 // sequence has, ~8 us per step, so in a SHORT batch (a slice of a sharded batch) a handful of very long sequences
 // are the critical path of the whole launch.  Sequences longer than `lstar` are taken out of the tiles: they get
@@ -365,6 +382,51 @@ static int key_bits(int64_t max_len)
     return b;
 }
 
+// stable descending radix sort of (keys_in, vals_in) on the key bits [0, end_bit): keys_out, order
+static int sort_desc(DecodeWs &w, int64_t n, int end_bit, cudaStream_t st)
+{
+    size_t tmp_bytes = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
+                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
+    if (int rc = w.cub_tmp.ensure(tmp_bytes)) return rc;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
+                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
+    return CV_OK;
+}
+
+// max_len <= 0 (not supplied): the longest length of the sorted batch is read back (one sync)
+static int read_max_len(const DecodeWs &w, int64_t &max_len, cudaStream_t st)
+{
+    if (max_len > 0) return CV_OK;
+    uint32_t L = 0;
+    CUDA_TRY(cudaMemcpyAsync(&L, w.keys_out.p, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    max_len = L;
+    return CV_OK;
+}
+
+// the buffers of workspace set w that ordering B sequences needs
+static int ensure_order_ws(DecodeWs &w, int64_t B)
+{
+    for (DevBuf *b : {&w.order, &w.keys_in, &w.keys_out, &w.vals_in})
+        if (int rc = b->ensure(sizeof(uint32_t) * (size_t)B)) return rc;
+    return w.misc.ensure(MISC_BYTES);
+}
+
+// Lengths of the sequences [b0, b1) from the host's offsets: their longest one, CV_ERR_ARG for offsets that are not
+// monotone, CV_ERR_EMPTY for an empty sequence (reference: usize underflow panic).
+static int scan_lengths(const int64_t *seq_off, int64_t b0, int64_t b1, int64_t &max_len)
+{
+    max_len = 0;
+    for (int64_t b = b0; b < b1; b++) {
+        const int64_t len = seq_off[b + 1] - seq_off[b];
+        if (len < 0) return fail(CV_ERR_ARG, "seq_off not monotone at %lld", (long long)b);
+        if (len == 0) return fail(CV_ERR_EMPTY, "sequence %lld is empty (reference: usize underflow panic)", (long long)b);
+        max_len = std::max(max_len, len);
+    }
+    return CV_OK;
+}
+
 // longest length of every tile of NS sequences (lengths are sorted descending)
 __global__ void tile_tmax_kernel(const uint32_t *sorted_len, int ntiles, int NS, long long *tmax)
 {
@@ -374,7 +436,6 @@ __global__ void tile_tmax_kernel(const uint32_t *sorted_len, int ntiles, int NS,
 
 // ---- streamed host path: keys = (chunk descending-coded, length) so that one descending sort orders the batch by
 // chunk (ascending) and, inside a chunk, by length (longest first); lengths must fit 24 bits
-constexpr int STREAM_MAX_CHUNKS = 16;
 // key = ordering group << shift | length.  promote_len > 0: the sequences of the chunks behind promote_to that are longer
 // than this are ordered with chunk promote_to (all observations have long arrived when that group is reached): every
 // group starts with its longest tiles, and a late, small group must not start tiles that outlast everything else.
@@ -429,9 +490,9 @@ struct StreamedIO {
 // Batches above the four-lane backtrace's range (launch_decode_small) are backtraced by one thread per sequence at
 // 6-9 us per step -- about as long again as the sequence's forward pass in a tile -- so there the limit is 45 %: at
 // 250 k sentences (a rank of a 4-GPU run) the slice holding a 191-step sentence ended 0.18 ms after the others.
-static uint32_t long_threshold(const cv_hmm *h, int64_t B, int64_t N, int64_t max_len)
+static uint32_t long_threshold(const cv_hmm *h, const DecodeCall &call, int64_t B, int64_t N, int64_t max_len)
 {
-    if (!g_tune.long_split || max_len <= 0 || h->K > SMALL_K_MAX || h->f32mode) return 0;   // (the warp-per-sequence kernel is f64)
+    if (!g_tune.long_split || max_len <= 0 || h->K > SMALL_K_MAX || call.f32) return 0;   // (the warp-per-sequence kernel is f64)
     const int64_t per_cta = (N / 64) / std::max<int64_t>(1, (int64_t)h->num_sms * 2);
     const int pct = g_tune.long_pct > 0 ? g_tune.long_pct : (g_tune.bt_split && B <= (int64_t)1300 * h->num_sms) ? 70 : 45;
     const int64_t l = std::max<int64_t>(64, per_cta * pct / 100);
@@ -440,10 +501,11 @@ static uint32_t long_threshold(const cv_hmm *h, int64_t B, int64_t N, int64_t ma
 constexpr uint32_t LONG_CAP = 4096;
 
 // binds the split's buffers for one launch (workspace set w) and zeroes the flags; ls.lstar = 0 when there is no split
-static int long_split_setup(cv_hmm *h, cv_hmm::DecodeWs &w, int64_t B, int64_t N, int64_t max_len, cudaStream_t st, LongSplit &ls)
+static int long_split_setup(cv_hmm *h, const DecodeCall &call, DecodeWs &w, int64_t B, int64_t N, int64_t max_len,
+                            cudaStream_t st, LongSplit &ls)
 {
     ls = LongSplit{0u, 0u, nullptr, nullptr, nullptr};
-    const uint32_t lstar = long_threshold(h, B, N, max_len);
+    const uint32_t lstar = long_threshold(h, call, B, N, max_len);
     if (!lstar) return CV_OK;
     int rc;
     const size_t row = (size_t)max_len * h->Kp;
@@ -454,30 +516,28 @@ static int long_split_setup(cv_hmm *h, cv_hmm::DecodeWs &w, int64_t B, int64_t N
     CUDA_TRY(cudaMemsetAsync(w.is_long.p, 0, (size_t)B, st));
     ls.lstar = lstar; ls.cap_long = cap;
     ls.is_long = (uint8_t *)w.is_long.p; ls.long_list = (uint32_t *)w.long_list.p;
-    ls.n_long = (unsigned int *)w.misc.p + 9;                // misc is zeroed by the caller before the keys kernel
+    ls.n_long = w.word(MISC_LONG_COUNT);                     // misc is zeroed by the caller before the keys kernel
     return CV_OK;
 }
 
-typedef cv_hmm::DecodeWs DecodeWs;
 #include "decode_large_host.inl"
 
-// cuStreamWaitValue32 through the runtime's driver entry-point lookup (no link-time dependency on libcuda):
-// lets a stream wait until a word in device memory reaches a value.  nullptr when unavailable.
-typedef int (*StreamWaitValue32Fn)(cudaStream_t, unsigned long long, unsigned int, unsigned int);
-static StreamWaitValue32Fn stream_wait_value32()
+// cuStreamWaitValue32 / cuStreamWriteValue32 through the runtime's driver entry-point lookup (no link-time dependency
+// on libcuda): a stream waits until a word in device memory reaches a value / writes a word once everything before it
+// in the stream is done.  nullptr when unavailable.
+typedef int (*StreamValue32Fn)(cudaStream_t, unsigned long long, unsigned int, unsigned int);
+static StreamValue32Fn driver_value32(const char *name)
 {
-    static StreamWaitValue32Fn fn = []() -> StreamWaitValue32Fn {
-        void *f = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuStreamWaitValue32", &f, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return (StreamWaitValue32Fn)f;
-    }();
-    return fn;
+    void *f = nullptr;
+    cudaDriverEntryPointQueryResult qr;
+    if (cudaGetDriverEntryPoint(name, &f, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess) {
+        cudaGetLastError();
+        return nullptr;
+    }
+    return (StreamValue32Fn)f;
 }
-
+static StreamValue32Fn stream_wait_value32() { static const StreamValue32Fn fn = driver_value32("cuStreamWaitValue32"); return fn; }
+static StreamValue32Fn stream_write_value32() { static const StreamValue32Fn fn = driver_value32("cuStreamWriteValue32"); return fn; }
 
 // the warp-per-sequence kernel with the instantiation that fits K (register-resident logA column for K <= 32)
 static int launch_chain_kernel(const cv_hmm *h, const DecodeChainParams &p, int grid, cudaStream_t st)
@@ -504,16 +564,37 @@ static int launch_chain_kernel(const cv_hmm *h, const DecodeChainParams &p, int 
     return CV_OK;
 }
 
-static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, int64_t B,
-                               int64_t N, uint32_t *d_path, double *d_score, unsigned int *d_counter, int *d_status,
-                               int64_t max_len, cudaStream_t st, bool timing, bool cert, const StreamedIO *sio = nullptr,
-                               const LongSplit *ls = nullptr)
+// Parameters of the warp-per-sequence kernel over the sequences order[0, B) with workspace set w: backpointer rows in
+// psi, tile counter in the misc word `counter`.  B_dev: the number of sequences is read on the device (at most B), and
+// the rows of list entry r start at row r * psi_stride.  sio: finished sequences are counted per chunk (streamed path).
+static DecodeChainParams chain_params(const cv_hmm *h, const DecodeCall &call, const DecodeWs &w, const uint32_t *d_obs,
+                                      const int64_t *d_off, uint32_t *d_path, double *d_score, const uint32_t *order,
+                                      void *psi, MiscWord counter, int64_t B, const unsigned int *B_dev = nullptr,
+                                      int64_t psi_stride = 0, const StreamedIO *sio = nullptr)
+{
+    DecodeChainParams q;
+    q.A = h->dA; q.BT = h->dBT; q.obs = d_obs; q.seq_off = d_off; q.order = order;
+    q.psi = (uint8_t *)psi; q.path = d_path; q.score = d_score; q.counter = w.word(counter); q.status = w.status();
+    q.M = h->M; q.B = B; q.K = h->K; q.Kp = h->Kp;
+    q.bt_in_smem = ((size_t)h->M * h->Kp * 8 <= CHAIN_BT_SMEM_MAX) ? 1 : 0;
+    q.obs16 = call.obs16; q.path8 = call.path8;
+    q.B_dev = B_dev; q.psi_stride = psi_stride;
+    q.chunk_done = sio ? sio->d_chunk_done : nullptr; q.nch = sio ? sio->cbs.nch : 0;
+    if (sio) for (int c = 0; c <= sio->cbs.nch; c++) q.cb[c] = sio->cbs.cb[c];
+    return q;
+}
+
+// The tile path of workspace set w: forward kernel over tiles of 64 sequences ordered longest first (w.order), then the
+// backtrace.  The tile counter and the status are w's misc words.
+static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off,
+                               int64_t B, int64_t N, uint32_t *d_path, double *d_score, int64_t max_len, cudaStream_t st,
+                               bool cert, const StreamedIO *sio = nullptr, const LongSplit *ls = nullptr)
 {
     const int G = h->G;
     const uint32_t *d_order = (const uint32_t *)w.order.p, *d_sorted_len = (const uint32_t *)w.keys_out.p;
     // optional f32 mode (decode_f32.cuh): its own forward kernel, f32 history, f32 backtrace.  cert: the same forward
     // kernel and history, then the certified backtrace (decode_small.cuh) -- the exact decode of an eligible model
-    const bool f32 = h->f32mode != 0 || cert;
+    const bool f32 = call.f32 || cert;
     // tiles of NS = 64 sequences (TP = 2 per lane), one warp per state group
     const int NS = 32 * TP, threads = 32 * G;
     size_t smem = f32 ? decode_f32_smem_bytes(h->K, h->Kp) : decode_small_smem_bytes(h->K, h->Kp, NS);
@@ -521,12 +602,7 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     if (ntiles64 > 0x7fffffffLL) return fail(CV_ERR_UNSUPPORTED, "batch too large");
     const int ntiles = (int)ntiles64;
     int rc;
-    if (max_len <= 0) {   // not supplied: read the longest length back (one sync)
-        uint32_t L = 0;
-        CUDA_TRY(cudaMemcpyAsync(&L, d_sorted_len, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        max_len = L;
-    }
+    if ((rc = read_max_len(w, max_len, st))) return rc;
     // history slabs: sum over tiles of NS * Tmax(tile) <= N + NS * max_len because lengths are sorted (per chunk, plus
     // the tiles that straddle two chunks, on the streamed path)
     // Streamed path: tiles are ordered by (chunk, length).  Inside a chunk the staircase bound above holds (one
@@ -554,17 +630,17 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     DecodeSmallParams p;
     p.A = h->dA; p.BT = h->dBT; p.obs = d_obs; p.seq_off = d_off; p.order = d_order;
     p.At = h->dA; p.BTt = h->dBT; p.nq_base = p.nq_rem = 0;
-    p.obs16 = h->obs16; p.path8 = h->path8; p.em_light = g_tune.em_light;
+    p.obs16 = call.obs16; p.path8 = call.path8; p.em_light = g_tune.em_light;
     p.is_long = (ls && ls->lstar) ? ls->is_long : nullptr;
     p.A32s = h->dA32f; p.A32n = h->dA32n; p.BT32 = h->dBT32;
     p.cert_list = cert ? (uint32_t *)w.cert_list.p : nullptr;
-    p.cert_count = cert ? (unsigned int *)w.misc.p + 10 : nullptr;      // zeroed by the caller with the rest of misc
+    p.cert_count = cert ? w.word(MISC_CERT) : nullptr;       // zeroed by the caller with the rest of misc
     p.cert_tol = g_tune.cert_tol;
     if ((f32 || g_tune.balanced_split) && h->dAb) {
         p.At = h->dAb; p.BTt = h->dBTb; p.nq_base = h->K / G; p.nq_rem = h->K % G;
     }
     p.tile_base = (const long long *)w.base.p;
-    p.hist = (double *)w.hist.p; p.hist_cap_slabs = (long long)(hist_rows / (size_t)NS); p.path = d_path; p.score = d_score; p.tile_counter = d_counter; p.status = d_status;
+    p.hist = (double *)w.hist.p; p.hist_cap_slabs = (long long)(hist_rows / (size_t)NS); p.path = d_path; p.score = d_score; p.tile_counter = w.word(MISC_COUNTER); p.status = w.status();
     p.M = h->M; p.B = B; p.K = h->K; p.Kp = h->Kp; p.G = G; p.NS = NS; p.ntiles = ntiles;
     p.tile_tmax = nullptr; p.tile_chunk = nullptr; p.arrived = nullptr; p.chunk_done = nullptr; p.nch = 0;
     if (sio) {
@@ -599,8 +675,8 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     // it tile by tile (tile_done flags).  It is released only when every forward CTA is resident (stream wait on
     // the `started` counter), so its spinning CTAs can never keep a forward CTA off an SM; it then lives on the
     // registers / shared memory the forward CTAs leave free.
-    StreamWaitValue32Fn wait32 = stream_wait_value32();
-    const bool concurrent = !timing && g_tune.bt_concurrent && wait32 != nullptr && w.st_bt != nullptr;
+    StreamValue32Fn wait32 = stream_wait_value32();
+    const bool concurrent = !call.timing && g_tune.bt_concurrent && wait32 != nullptr && w.st_bt != nullptr;
     if (sio && !concurrent) return fail(CV_ERR_UNSUPPORTED, "the streamed path needs the concurrent backtrace");
     p.tile_done = nullptr; p.started = nullptr;
     if (concurrent) {
@@ -614,16 +690,8 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     // stream of its own; it is launched first so that its few CTAs are resident before the persistent forward CTAs.
     bool long_launched = false;
     if (ls && ls->lstar) {
-        DecodeChainParams q;
-        q.A = h->dA; q.BT = h->dBT; q.obs = d_obs; q.seq_off = d_off; q.order = ls->long_list;
-        q.psi = (uint8_t *)w.long_psi.p; q.path = d_path; q.score = d_score;
-        q.counter = (unsigned int *)w.misc.p + 8; q.status = d_status;
-        q.M = h->M; q.B = (int64_t)ls->cap_long; q.K = h->K; q.Kp = h->Kp;
-        q.bt_in_smem = ((size_t)h->M * h->Kp * 8 <= CHAIN_BT_SMEM_MAX) ? 1 : 0;
-        q.obs16 = h->obs16; q.path8 = h->path8;
-        q.B_dev = ls->n_long; q.psi_stride = max_len;
-        q.chunk_done = sio ? sio->d_chunk_done : nullptr; q.nch = sio ? sio->cbs.nch : 0;
-        if (sio) for (int c = 0; c <= sio->cbs.nch; c++) q.cb[c] = sio->cbs.cb[c];
+        const DecodeChainParams q = chain_params(h, call, w, d_obs, d_off, d_path, d_score, ls->long_list, w.long_psi.p,
+                                                 MISC_LONG_COUNTER, (int64_t)ls->cap_long, ls->n_long, max_len, sio);
         CUDA_TRY(cudaEventRecord(h->ev_long_dep, st));                        // keys kernel (list, count) and the offsets are done
         CUDA_TRY(cudaStreamWaitEvent(h->st_long, h->ev_long_dep, 0));
         if (sio) CUDA_TRY(cudaStreamWaitEvent(h->st_long, sio->all_in, 0));   // streamed: all observations on the device
@@ -633,11 +701,11 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
         long_launched = true;
     }
     const bool bt_prof = g_tune.bt_prof != 0;   // prints forward / forward+backtrace times of the concurrent mode
-    if (timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev0, st));
+    if (call.timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev0, st));
     kern<<<std::max(1, grid), threads, smem, st>>>(p);
     g_launches++;
     CUDA_TRY(cudaGetLastError());
-    if (timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev1, st));
+    if (call.timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev1, st));
     // end state + backtrace with lazy backpointers: one thread per sequence
     const size_t smem_bt = (size_t)h->K * (h->K | 1) * 8 + 16 * 8;      // + one chunk of padding behind the last row
     void (*bt_seq)(DecodeSmallParams) = cert ? backtrace_small_kernel<16, 4, float, true>
@@ -686,7 +754,7 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
     bt_seq<<<grid_bt, 128, smem_bt_use, st>>>(p);
     g_launches++;
     CUDA_TRY(cudaGetLastError());
-    if (timing) CUDA_TRY(cudaEventRecord(h->ev2, st));
+    if (call.timing) CUDA_TRY(cudaEventRecord(h->ev2, st));
     if (long_launched) CUDA_TRY(cudaStreamWaitEvent(st, h->ev_long_done, 0));
     return CV_OK;
 }
@@ -696,9 +764,9 @@ static int launch_decode_small(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, co
 // not to one chunk: cv_b200.h promises such calls the exact f64 kernel, and every larger call the f32 kernels in all
 // its chunks (a forced small chunk count must not hand part of an f32 call to the f64 kernel).
 constexpr int64_t CHAIN_BATCH_MAX = 8192;
-static bool chain_batch(const cv_hmm *h, int64_t B)
+static bool chain_batch(const cv_hmm *h, const DecodeCall &call, int64_t B)
 {
-    if (h->f32mode) return h->K <= SMALL_K_MAX && h->f32_call_B <= CHAIN_BATCH_MAX;
+    if (call.f32) return h->K <= SMALL_K_MAX && call.B <= CHAIN_BATCH_MAX;
     const long long bound = g_tune.chain_max_b < 0 ? CHAIN_BATCH_MAX : g_tune.chain_max_b;
     return h->K <= SMALL_K_MAX && B <= bound;
 }
@@ -717,12 +785,11 @@ __global__ void listed_len_keys_kernel(const int64_t *seq_off, const uint32_t *l
 // paths and scores are overwritten.  This is the one host round trip of a certified call: the flagged count, their
 // longest length and their elements are read back, and decide the kernel -- the warp-per-sequence kernel for as many
 // sequences as a batch would give it (chain_batch), else the f64 tile path over the flagged sequences ordered by length.
-static int certified_fallback(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, uint32_t *d_path,
-                              double *d_score, int *d_status, cudaStream_t st)
+static int certified_fallback(cv_hmm *h, const DecodeCall &call, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off,
+                              uint32_t *d_path, double *d_score, cudaStream_t st)
 {
-    unsigned int *d_count = (unsigned int *)w.misc.p + 10;                  // cert_count of launch_decode_small
-    unsigned int *hc = (unsigned int *)((char *)h->pinned_status + 64);
-    CUDA_TRY(cudaMemcpyAsync(hc, d_count, 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
+    unsigned int *hc = h->pinned<unsigned int>(PIN_CERT);
+    CUDA_TRY(cudaMemcpyAsync(hc, w.word(MISC_CERT), 4 * sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     const int64_t n = hc[0], lmax = hc[1];
     const int64_t nel = (int64_t)*reinterpret_cast<const unsigned long long *>(hc + 2);
@@ -733,100 +800,70 @@ static int certified_fallback(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, con
     if (n <= CHAIN_BATCH_MAX) {
         // the f32 history is no longer needed: its buffer takes the backpointer rows
         if ((rc = w.hist.ensure((size_t)n * (size_t)lmax * h->Kp + 64))) return rc;
-        DecodeChainParams q;
-        q.A = h->dA; q.BT = h->dBT; q.obs = d_obs; q.seq_off = d_off; q.order = list;
-        q.psi = (uint8_t *)w.hist.p; q.path = d_path; q.score = d_score;
-        q.counter = (unsigned int *)w.misc.p + 14; q.status = d_status;
-        q.M = h->M; q.B = n; q.K = h->K; q.Kp = h->Kp;
-        q.bt_in_smem = ((size_t)h->M * h->Kp * 8 <= CHAIN_BT_SMEM_MAX) ? 1 : 0;
-        q.obs16 = h->obs16; q.path8 = h->path8;
-        q.B_dev = d_count; q.psi_stride = lmax;
-        q.chunk_done = nullptr; q.nch = 0;
+        const DecodeChainParams q = chain_params(h, call, w, d_obs, d_off, d_path, d_score, list, w.hist.p, MISC_CERT_COUNTER,
+                                                 n, w.word(MISC_CERT), lmax);
         const int grid = (int)std::min<int64_t>((n + DC_WARPS - 1) / DC_WARPS, (int64_t)h->num_sms * 8);
         return launch_chain_kernel(h, q, grid, st);
     }
     listed_len_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, list, n, (uint32_t *)w.keys_in.p, (uint32_t *)w.vals_in.p);
     g_launches++;
-    const int end_bit = key_bits(lmax);
-    size_t tmp_bytes = 0;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
-                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
-    if ((rc = w.cub_tmp.ensure(tmp_bytes))) return rc;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
-                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)n, 0, end_bit, st));
-    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, sizeof(unsigned int), st));        // tile counter
-    return launch_decode_small(h, w, d_obs, d_off, n, nel, d_path, d_score, (unsigned int *)w.misc.p, d_status, lmax, st,
-                               false, false);
+    if ((rc = sort_desc(w, n, key_bits(lmax), st))) return rc;
+    CUDA_TRY(cudaMemsetAsync(w.word(MISC_COUNTER), 0, sizeof(unsigned int), st));
+    DecodeCall exact = call;
+    exact.timing = false;                     // the call's kernel times stay those of the certified pass
+    return launch_decode_small(h, exact, w, d_obs, d_off, n, nel, d_path, d_score, lmax, st, false);
 }
 
 // One chunk of sequences [0, B) of d_off (offsets are absolute into d_obs / d_path): order by length,
 // forward, backtrace; everything enqueued on `st` with workspace set `w`.  can_certify: the chunk is the whole call
 // (certified_fallback's host round trip is made once per call).
-static int decode_chunk(cv_hmm *h, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                        int64_t max_len, uint32_t *d_path, double *d_score, cudaStream_t st, bool timing, bool can_certify)
+static int decode_chunk(cv_hmm *h, const DecodeCall &call, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off,
+                        int64_t B, int64_t N, int64_t max_len, uint32_t *d_path, double *d_score, cudaStream_t st,
+                        bool can_certify)
 {
     int rc;
     if (B > 0x7fffffffLL) return fail(CV_ERR_UNSUPPORTED, "more than 2^31 sequences in one chunk");
-    if ((rc = w.order.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
-    if ((rc = w.keys_in.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
-    if ((rc = w.keys_out.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
-    if ((rc = w.vals_in.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
-    if ((rc = w.misc.ensure(256))) return rc;
-    unsigned int *d_counter = (unsigned int *)w.misc.p;
-    int *d_status = (int *)w.misc.p + 16;
-    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, 256, st));
-    const bool chain_all = chain_batch(h, B);
+    if ((rc = ensure_order_ws(w, B))) return rc;
+    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, MISC_BYTES, st));
+    const bool chain_all = chain_batch(h, call, B);
     LongSplit ls{0u, 0u, nullptr, nullptr, nullptr};
-    if (!chain_all && (rc = long_split_setup(h, w, B, N, max_len, st, ls))) return rc;
+    if (!chain_all && (rc = long_split_setup(h, call, w, B, N, max_len, st, ls))) return rc;
     // order sequences by length, longest first (stable radix sort => deterministic)
     seq_len_keys_kernel<<<(unsigned)((B + 255) / 256), 256, 0, st>>>(d_off, B, (uint32_t *)w.keys_in.p,
-                                                                    (uint32_t *)w.vals_in.p, d_status, ls, max_len);
+                                                                    (uint32_t *)w.vals_in.p, w.status(), ls, max_len);
     g_launches++;
     // the radix sort only visits the bits a length can have (one 8-bit pass for lengths up to 255 instead of four)
-    const int end_bit = max_len > 0 ? key_bits(max_len) : 32;
-    size_t tmp_bytes = 0;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, (uint32_t *)w.keys_in.p,
-                                                       (uint32_t *)w.keys_out.p, (uint32_t *)w.vals_in.p,
-                                                       (uint32_t *)w.order.p, (int)B, 0, end_bit, st));
-    if ((rc = w.cub_tmp.ensure(tmp_bytes))) return rc;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p,
-                                                       (uint32_t *)w.keys_out.p, (uint32_t *)w.vals_in.p,
-                                                       (uint32_t *)w.order.p, (int)B, 0, end_bit, st));
+    if ((rc = sort_desc(w, B, max_len > 0 ? key_bits(max_len) : 32, st))) return rc;
     if (chain_all) {
         // few sequences: one warp per sequence (latency-oriented), backpointers as u8 rows
         if ((rc = w.hist.ensure((size_t)N * h->Kp + 64))) return rc;
-        DecodeChainParams p;
-        p.A = h->dA; p.BT = h->dBT; p.obs = d_obs; p.seq_off = d_off; p.order = (const uint32_t *)w.order.p;
-        p.psi = (uint8_t *)w.hist.p; p.path = d_path; p.score = d_score; p.counter = d_counter; p.status = d_status;
-        p.M = h->M; p.B = B; p.K = h->K; p.Kp = h->Kp;
-        p.bt_in_smem = ((size_t)h->M * h->Kp * 8 <= CHAIN_BT_SMEM_MAX) ? 1 : 0;
-        p.obs16 = h->obs16; p.path8 = h->path8;
-        p.B_dev = nullptr; p.psi_stride = 0; p.chunk_done = nullptr; p.nch = 0;
+        const DecodeChainParams p = chain_params(h, call, w, d_obs, d_off, d_path, d_score, (const uint32_t *)w.order.p,
+                                                 w.hist.p, MISC_COUNTER, B);
         const int grid = (int)std::min<int64_t>((B + DC_WARPS - 1) / DC_WARPS, (int64_t)h->num_sms * 8);
-        if (timing) CUDA_TRY(cudaEventRecord(h->ev0, st));
+        if (call.timing) CUDA_TRY(cudaEventRecord(h->ev0, st));
         if ((rc = launch_chain_kernel(h, p, grid, st))) return rc;
-        if (timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
+        if (call.timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
         return CV_OK;
     }
     if (h->K <= SMALL_K_MAX) {
-        const bool cert = can_certify && h->cert_ok && !h->f32mode && g_tune.certified;
+        const bool cert = can_certify && h->cert_ok && !call.f32 && g_tune.certified;
         if (cert && (rc = w.cert_list.ensure(sizeof(uint32_t) * (size_t)B))) return rc;
-        if ((rc = launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, st, timing, cert, nullptr, &ls)))
-            return rc;
+        if ((rc = launch_decode_small(h, call, w, d_obs, d_off, B, N, d_path, d_score, max_len, st, cert, nullptr, &ls))) return rc;
         if (!cert) return CV_OK;
-        if ((rc = certified_fallback(h, w, d_obs, d_off, d_path, d_score, d_status, st))) return rc;
-        if (timing) CUDA_TRY(cudaEventRecord(h->ev2, st));               // backtrace time = backtrace + fallback
+        if ((rc = certified_fallback(h, call, w, d_obs, d_off, d_path, d_score, st))) return rc;
+        if (call.timing) CUDA_TRY(cudaEventRecord(h->ev2, st));               // backtrace time = backtrace + fallback
         return CV_OK;
     }
-    if (timing) CUDA_TRY(cudaEventRecord(h->ev0, st));
-    if ((rc = launch_decode_large(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, st))) return rc;
-    if (timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
+    if (call.timing) CUDA_TRY(cudaEventRecord(h->ev0, st));
+    if ((rc = launch_decode_large(h, w, d_obs, d_off, B, d_path, d_score, max_len, st))) return rc;
+    if (call.timing) { CUDA_TRY(cudaEventRecord(h->ev1, st)); CUDA_TRY(cudaEventRecord(h->ev2, st)); }
     return CV_OK;
 }
 
-static int chunk_count(const cv_hmm *h, int64_t B, bool timing, bool host_buffers)
+static int chunk_count(const cv_hmm *h, const DecodeCall &call, bool host_buffers)
 {
-    if (timing || h->K > SMALL_K_MAX) return 1;          // kernel timing wants one launch for the whole batch
+    const int64_t B = call.B;
+    if (call.timing || h->K > SMALL_K_MAX) return 1;     // kernel timing wants one launch for the whole batch
     if (g_tune.chunks > 0) return (int)std::min<int64_t>(g_tune.chunks, std::max<int64_t>(B, 1));
     // >= ~6 tiles per resident CTA per chunk keeps the dynamic tile scheduler balanced.  Host buffers: six
     // chunks so that H2D / D2H copies hide behind the kernels (measured at the POS shape: 2 chunks 16.5 ms,
@@ -847,10 +884,21 @@ static int chunk_count(const cv_hmm *h, int64_t B, bool timing, bool host_buffer
     return (int)std::max<int64_t>(1, std::min<int64_t>(host_buffers ? 6 : dev_chunks, B / per_chunk));
 }
 
-static int report_status(const int *status_words, int n)
+// The end of a call that used workspace sets [0, nws): their status words are read back behind the work on st[k], the
+// kernel times are taken when the call is timed, and the first error status is reported.
+static int finish_call(cv_hmm *h, const DecodeCall &call, int nws, cudaStream_t st0, cudaStream_t st1 = nullptr)
 {
-    for (int i = 0; i < n; i++) {
-        const int s = status_words[i];
+    const cudaStream_t st[2] = {st0, st1};
+    int *hs = h->pinned<int>(PIN_STATUS);
+    for (int k = 0; k < nws; k++) CUDA_TRY(cudaMemcpyAsync(hs + k, h->ws[k].status(), sizeof(int), cudaMemcpyDeviceToHost, st[k]));
+    for (int k = 0; k < nws; k++) CUDA_TRY(cudaStreamSynchronize(st[k]));
+    if (call.timing) {
+        float ms = 0.f;
+        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_ms = ms; else cudaGetLastError();
+        if (cudaEventElapsedTime(&ms, h->ev1, h->ev2) == cudaSuccess) h->last_bt_ms = ms; else cudaGetLastError();
+    }
+    for (int k = 0; k < nws; k++) {
+        const int s = hs[k];
         if (s == CV_ERR_EMPTY) return fail(CV_ERR_EMPTY, "empty sequence in batch (reference: usize underflow panic)");
         if (s == CV_ERR_ARG) return fail(CV_ERR_ARG, "observation index >= M (reference: ndarray index panic)");
         if (s) return fail(s, "device status %d", s);
@@ -858,41 +906,10 @@ static int report_status(const int *status_words, int n)
     return CV_OK;
 }
 
-static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                                 int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status);
-
-extern "C" int cv_decode_batch_dev(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                                   int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
+static int decode_batch_dev(cv_hmm *h, const DecodeCall &call, const uint32_t *d_obs, const int64_t *d_off, int64_t N,
+                            int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
 {
-    return decode_batch_dev_impl(h, d_obs, d_off, B, N, max_len, d_path, d_score, stream, sync_status);
-}
-
-extern "C" int cv_decode_batch_dev_u8(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                                      int64_t max_len, uint8_t *d_path, double *d_score, void *stream, int sync_status)
-{
-    if (!h) return fail(CV_ERR_ARG, "NULL model");
-    if (h->K > SMALL_K_MAX) return fail(CV_ERR_UNSUPPORTED, "u8 paths are implemented for K <= %d", SMALL_K_MAX);
-    h->path8 = 1;
-    const int rc = decode_batch_dev_impl(h, d_obs, d_off, B, N, max_len, reinterpret_cast<uint32_t *>(d_path), d_score, stream, sync_status);
-    h->path8 = 0;
-    return rc;
-}
-
-extern "C" int cv_decode_batch_dev_f32(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                                       int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
-{
-    if (!h) return fail(CV_ERR_ARG, "NULL model");
-    if (!h->dA32f) return fail(CV_ERR_UNSUPPORTED, "the f32 mode is implemented for K <= %d", SMALL_K_MAX);
-    if (!h->f32_range_ok) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs every finite model entry within |x| <= 2^64");
-    h->f32mode = 1; h->f32_call_B = B;
-    const int rc = decode_batch_dev_impl(h, d_obs, d_off, B, N, max_len, d_path, d_score, stream, sync_status);
-    h->f32mode = 0;
-    return rc;
-}
-
-static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
-                                 int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
-{
+    const int64_t B = call.B;
     if (!h) return fail(CV_ERR_ARG, "NULL model");
     if (B < 0 || N < 0) return fail(CV_ERR_ARG, "negative size");
     if (B == 0) return CV_OK;
@@ -900,11 +917,10 @@ static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t
     CUDA_TRY(cudaSetDevice(h->device));
     h->last_flagged = -1;
     cudaStream_t user = (cudaStream_t)stream;
-    const bool timing = g_timing.load() != 0;
-    const int nch = chunk_count(h, B, timing, false);
+    const int nch = chunk_count(h, call, false);
     int rc;
     if (nch == 1) {
-        if ((rc = decode_chunk(h, h->ws[0], d_obs, d_off, B, N, max_len, d_path, d_score, user, timing, true))) return rc;
+        if ((rc = decode_chunk(h, call, h->ws[0], d_obs, d_off, B, N, max_len, d_path, d_score, user, true))) return rc;
     } else {
         // fork: chunk k runs on internal stream k % 2 so that backtrace(k) overlaps forward(k+1)
         if (max_len <= 0) return fail(CV_ERR_ARG, "max_len is required for the chunked device path");
@@ -913,8 +929,8 @@ static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t
         for (int k = 0; k < nch; k++) {
             const int64_t b0 = B * k / nch, b1 = B * (k + 1) / nch;
             DecodeWs &w = h->ws[k & 1];
-            if ((rc = decode_chunk(h, w, d_obs, d_off + b0, b1 - b0, N, max_len, d_path,
-                                   d_score ? d_score + b0 : nullptr, w.st, false, false)))
+            if ((rc = decode_chunk(h, call, w, d_obs, d_off + b0, b1 - b0, N, max_len, d_path,
+                                   d_score ? d_score + b0 : nullptr, w.st, false)))
                 return rc;
         }
         for (int k = 0; k < 2; k++) {
@@ -922,38 +938,39 @@ static int decode_batch_dev_impl(cv_hmm *h, const uint32_t *d_obs, const int64_t
             CUDA_TRY(cudaStreamWaitEvent(user, h->ws[k].done, 0));
         }
     }
-    if (sync_status || timing) {
-        int *hs = (int *)h->pinned_status + 8;
-        for (int k = 0; k < 2; k++)
-            if (h->ws[k].misc.p) CUDA_TRY(cudaMemcpyAsync(hs + k, (int *)h->ws[k].misc.p + 16, sizeof(int), cudaMemcpyDeviceToHost, user));
-            else hs[k] = 0;
-        CUDA_TRY(cudaStreamSynchronize(user));
-        if (timing) {
-            float ms = 0.f;
-            CUDA_TRY(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
-            h->last_ms = ms;
-            CUDA_TRY(cudaEventElapsedTime(&ms, h->ev1, h->ev2));
-            h->last_bt_ms = ms;
-        }
-        return report_status(hs, 2);
-    }
+    if (!sync_status && !call.timing) return CV_OK;
+    return finish_call(h, call, nch == 1 ? 1 : 2, user, user);
+}
+
+extern "C" int cv_decode_batch_dev(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
+                                   int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
+{
+    return decode_batch_dev(h, decode_call(B), d_obs, d_off, N, max_len, d_path, d_score, stream, sync_status);
+}
+
+extern "C" int cv_decode_batch_dev_u8(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
+                                      int64_t max_len, uint8_t *d_path, double *d_score, void *stream, int sync_status)
+{
+    if (!h) return fail(CV_ERR_ARG, "NULL model");
+    if (h->K > SMALL_K_MAX) return fail(CV_ERR_UNSUPPORTED, "u8 paths are implemented for K <= %d", SMALL_K_MAX);
+    return decode_batch_dev(h, decode_call(B, false, 0, 1), d_obs, d_off, N, max_len, reinterpret_cast<uint32_t *>(d_path),
+                            d_score, stream, sync_status);
+}
+
+// preconditions of the f32 entry points
+static int check_f32(const cv_hmm *h)
+{
+    if (!h) return fail(CV_ERR_ARG, "NULL model");
+    if (!h->dA32f) return fail(CV_ERR_UNSUPPORTED, "the f32 mode is implemented for K <= %d", SMALL_K_MAX);
+    if (!h->f32_range_ok) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs every finite model entry within |x| <= 2^64");
     return CV_OK;
 }
 
-// cuStreamWriteValue32: a stream writes a word once everything before it in the stream is done
-typedef int (*StreamWriteValue32Fn)(cudaStream_t, unsigned long long, unsigned int, unsigned int);
-static StreamWriteValue32Fn stream_write_value32()
+extern "C" int cv_decode_batch_dev_f32(cv_hmm *h, const uint32_t *d_obs, const int64_t *d_off, int64_t B, int64_t N,
+                                       int64_t max_len, uint32_t *d_path, double *d_score, void *stream, int sync_status)
 {
-    static StreamWriteValue32Fn fn = []() -> StreamWriteValue32Fn {
-        void *f = nullptr;
-        cudaDriverEntryPointQueryResult qr;
-        if (cudaGetDriverEntryPoint("cuStreamWriteValue32", &f, cudaEnableDefault, &qr) != cudaSuccess || qr != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return (StreamWriteValue32Fn)f;
-    }();
-    return fn;
+    if (int rc = check_f32(h)) return rc;
+    return decode_batch_dev(h, decode_call(B, true), d_obs, d_off, N, max_len, d_path, d_score, stream, sync_status);
 }
 
 // Streamed host path (K <= 64, large batches): ONE forward + backtrace launch over the whole batch while the
@@ -962,28 +979,23 @@ static StreamWriteValue32Fn stream_write_value32()
 // the backtrace has counted the chunk's sequences done (stream wait on chunk_done[c]).  The batch is ordered by
 // (chunk, length), so the kernels consume the chunks in arrival order.  Against one launch per chunk this
 // removes the per-chunk sort / launch / ramp costs: the copies hide behind 13 ms of kernels instead of 6 x 2.3 ms.
-static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B, uint32_t *path_out,
-                           double *score_out, int nch, bool *handled, uint32_t *d_path, double *d_score)
+static int decode_streamed(cv_hmm *h, const DecodeCall &call, const uint32_t *obs_flat, const int64_t *seq_off,
+                           uint32_t *path_out, double *score_out, int nch, bool *handled, uint32_t *d_path, double *d_score)
 {
     *handled = false;
-    const size_t ob = h->obs16 ? 2 : 4, pb = h->path8 ? 1 : 4;       // bytes per observation / per path element on the host side
-    StreamWaitValue32Fn wait32 = stream_wait_value32();
-    StreamWriteValue32Fn write32 = stream_write_value32();
+    const int64_t B = call.B;
+    const size_t ob = call.obs_bytes(), pb = call.path_bytes();
+    StreamValue32Fn wait32 = stream_wait_value32(), write32 = stream_write_value32();
     if (!g_tune.streamed || !g_tune.bt_concurrent || !wait32 || !write32 || nch < 2 || nch > STREAM_MAX_CHUNKS) return CV_OK;
-    if (h->K > SMALL_K_MAX || chain_batch(h, B) || B > 0x7fffffffLL) return CV_OK;
+    if (h->K > SMALL_K_MAX || chain_batch(h, call, B) || B > 0x7fffffffLL) return CV_OK;
     const int64_t N = seq_off[B];
     DecodeWs &w = h->ws[0];
     cudaStream_t sk = w.st, s_in = h->ws[1].st, s_out = h->ws[1].st_bt;
     uint32_t *d_obs = (uint32_t *)h->obs.p;
     int64_t *d_off = (int64_t *)h->seq_off.p;
     int rc;
-    if ((rc = w.order.ensure(sizeof(uint32_t) * (size_t)B)) || (rc = w.keys_in.ensure(sizeof(uint32_t) * (size_t)B)) ||
-        (rc = w.keys_out.ensure(sizeof(uint32_t) * (size_t)B)) || (rc = w.vals_in.ensure(sizeof(uint32_t) * (size_t)B)) ||
-        (rc = w.misc.ensure(256)))
-        return rc;
-    unsigned int *d_counter = (unsigned int *)w.misc.p;
-    int *d_status = (int *)w.misc.p + 16;
-    unsigned int *d_maxlen = (unsigned int *)w.misc.p + 17, *d_arrived = (unsigned int *)w.misc.p + 32, *d_chunk_done = d_arrived + 1;
+    if ((rc = ensure_order_ws(w, B))) return rc;
+    unsigned int *d_arrived = w.word(MISC_ARRIVED), *d_chunk_done = w.word(MISC_CHUNK_DONE);
     StreamedIO sio;
     sio.cbs.nch = nch;
     // Chunk sizes.  The forward kernel cannot start before chunk 0 is on the device and the last chunk's paths leave after
@@ -1020,10 +1032,9 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     double hm_scan = 0.0, hm_enq = 0.0;
     if (prof) { for (auto &e : pe) cudaEventCreate(&e); cudaEventRecord(pe[0], sk); }
     // offsets first (the ordering needs nothing else), then the observations chunk by chunk on the copy stream
-    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, 256, sk));
+    CUDA_TRY(cudaMemsetAsync(w.misc.p, 0, MISC_BYTES, sk));
     CUDA_TRY(cudaMemcpyAsync(d_off, seq_off, sizeof(int64_t) * (size_t)(B + 1), cudaMemcpyHostToDevice, sk));
     CUDA_TRY(cudaEventRecord(w.ev_pre, sk));
-    int *hs = (int *)h->pinned_status + 8;
     // `arrived` is zeroed first -- and the offsets have the link to themselves: the ordering (keys, sort) waits for them,
     // and two host-to-device copies in flight share the bandwidth (offsets + keys done at 0.5 instead of 0.25 ms)
     CUDA_TRY(cudaStreamWaitEvent(s_in, w.ev_pre, 0));
@@ -1040,19 +1051,14 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     LongSplit ls{0u, 0u, nullptr, nullptr, nullptr};
     int64_t max_len_host = 0;
     if (B <= (1 << 18)) {
-        for (int64_t b = 0; b < B; b++) {
-            const int64_t len = seq_off[b + 1] - seq_off[b];
-            if (len <= 0) return len == 0 ? fail(CV_ERR_EMPTY, "empty sequence in batch (reference: usize underflow panic)")
-                                          : fail(CV_ERR_ARG, "seq_off not monotone");
-            max_len_host = std::max(max_len_host, len);
-        }
-        if (max_len_host <= 0xffffffLL && (rc = long_split_setup(h, w, B, N, max_len_host, sk, ls))) return rc;
+        if ((rc = scan_lengths(seq_off, 0, B, max_len_host))) return rc;
+        if (max_len_host <= 0xffffffLL && (rc = long_split_setup(h, call, w, B, N, max_len_host, sk, ls))) return rc;
     }
     // sort key = chunk field << shift | length: 24 bits of length when the longest one is not known yet, else just the
     // bits it needs (the sort then takes one or two 8-bit passes instead of four)
     sio.cbs.shift = (max_len_host > 0 && max_len_host <= 0xffffffLL) ? key_bits(max_len_host) : 24;
     seq_chunk_keys_kernel<<<(unsigned)((B + 255) / 256), 256, 0, sk>>>(d_off, B, sio.cbs, (uint32_t *)w.keys_in.p,
-                                                                      (uint32_t *)w.vals_in.p, d_status, d_maxlen, ls);
+                                                                      (uint32_t *)w.vals_in.p, w.status(), w.word(MISC_MAX_LEN), ls);
     g_launches++;
     // Lengths are checked and the longest one is found before the launch (the history is sized from it).  Small
     // batches (a slice of a sharded batch): on the HOST while the first copies fly -- 0.1 ms per 100 k sequences and no
@@ -1060,7 +1066,8 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     // thread would need ~0.7 ms for a million offsets, which delays the launch past the arrival of chunk 0).
     int64_t max_len = max_len_host;
     if (B > (1 << 18)) {
-        CUDA_TRY(cudaMemcpyAsync(hs, d_status, 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));  // status, longest length
+        int *hs = h->pinned<int>(PIN_STATUS);
+        CUDA_TRY(cudaMemcpyAsync(hs, w.status(), 2 * sizeof(int), cudaMemcpyDeviceToHost, sk));  // MISC_STATUS, MISC_MAX_LEN
         CUDA_TRY(cudaStreamSynchronize(sk));
         if (hs[0] == CV_ERR_EMPTY) return fail(CV_ERR_EMPTY, "empty sequence in batch (reference: usize underflow panic)");
         if (hs[0] == CV_ERR_ARG) return fail(CV_ERR_ARG, "seq_off not monotone");
@@ -1070,15 +1077,9 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
     if (max_len > 0xffffffLL) { *handled = false; return CV_OK; }                              // does not fit the 24-bit sort key: chunked path
     if (prof) { hm_scan = host_ms(); cudaEventRecord(pe[1], sk); cudaEventRecord(pe[4], s_in); }
 
-    const int end_bit = std::min(32, sio.cbs.shift + key_bits(nch - 1));
-    size_t tmp_bytes = 0;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
-                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)B, 0, end_bit, sk));
-    if ((rc = w.cub_tmp.ensure(tmp_bytes))) return rc;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(w.cub_tmp.p, tmp_bytes, (uint32_t *)w.keys_in.p, (uint32_t *)w.keys_out.p,
-                                                       (uint32_t *)w.vals_in.p, (uint32_t *)w.order.p, (int)B, 0, end_bit, sk));
+    if ((rc = sort_desc(w, B, std::min(32, sio.cbs.shift + key_bits(nch - 1)), sk))) return rc;
     if (prof) cudaEventRecord(pe[2], sk);
-    if ((rc = launch_decode_small(h, w, d_obs, d_off, B, N, d_path, d_score, d_counter, d_status, max_len, sk, false, false, &sio, &ls))) return rc;
+    if ((rc = launch_decode_small(h, call, w, d_obs, d_off, B, N, d_path, d_score, max_len, sk, false, &sio, &ls))) return rc;
     if (prof) cudaEventRecord(pe[3], sk);
     // paths / scores of chunk c leave as soon as the backtrace has counted all its sequences
     CUDA_TRY(cudaStreamWaitEvent(s_out, w.ev_pre, 0));
@@ -1090,10 +1091,8 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
         CUDA_TRY(cudaMemcpyAsync((char *)path_out + pb * e0, (const char *)d_path + pb * e0, pb * (size_t)(e1 - e0), cudaMemcpyDeviceToHost, s_out));
         if (score_out) CUDA_TRY(cudaMemcpyAsync(score_out + b0, d_score + b0, sizeof(double) * (size_t)(b1 - b0), cudaMemcpyDeviceToHost, s_out));
     }
-    CUDA_TRY(cudaMemcpyAsync(hs, d_status, sizeof(int), cudaMemcpyDeviceToHost, sk));
-    hs[1] = 0;
     if (prof) { hm_enq = host_ms(); cudaEventRecord(pe[5], s_out); }
-    CUDA_TRY(cudaStreamSynchronize(sk));
+    const int status = finish_call(h, call, 1, sk);
     CUDA_TRY(cudaStreamSynchronize(s_out));
     CUDA_TRY(cudaStreamSynchronize(s_in));
     if (prof) {
@@ -1106,54 +1105,13 @@ static int decode_streamed(cv_hmm *h, const uint32_t *obs_flat, const int64_t *s
         for (auto &e : pe) cudaEventDestroy(e);
     }
     *handled = true;
-    return report_status(hs, 1);
+    return status;
 }
 
-static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B, uint32_t *path_out,
-                             double *score_out, uint32_t *d_path_keep, double *d_score_keep);
-
-extern "C" int cv_decode_batch(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
-                               uint32_t *path_out, double *score_out)
+static int decode_batch_host(cv_hmm *h, const DecodeCall &call, const uint32_t *obs_flat, const int64_t *seq_off,
+                             uint32_t *path_out, double *score_out, uint32_t *d_path_keep = nullptr, double *d_score_keep = nullptr)
 {
-    return decode_batch_host(h, obs_flat, seq_off, B, path_out, score_out, nullptr, nullptr);
-}
-
-extern "C" int cv_decode_batch_keep(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
-                                    uint32_t *path_out, double *score_out, uint32_t *d_path_keep, double *d_score_keep)
-{
-    if (!d_path_keep || !d_score_keep) return fail(CV_ERR_ARG, "NULL device buffer");
-    return decode_batch_host(h, obs_flat, seq_off, B, path_out, score_out, d_path_keep, d_score_keep);
-}
-
-extern "C" int cv_decode_batch_f32(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
-                                   uint32_t *path_out, double *score_out)
-{
-    if (!h) return fail(CV_ERR_ARG, "NULL model");
-    if (!h->dA32f) return fail(CV_ERR_UNSUPPORTED, "the f32 mode is implemented for K <= %d", SMALL_K_MAX);
-    if (!h->f32_range_ok) return fail(CV_ERR_UNSUPPORTED, "the f32 mode needs every finite model entry within |x| <= 2^64");
-    h->f32mode = 1; h->f32_call_B = B;
-    const int rc = decode_batch_host(h, obs_flat, seq_off, B, path_out, score_out, nullptr, nullptr);
-    h->f32mode = 0;
-    return rc;
-}
-
-extern "C" int cv_decode_batch_u16u8(cv_hmm *h, const uint16_t *obs_flat, const int64_t *seq_off, int64_t B,
-                                     uint8_t *path_out, double *score_out)
-{
-    if (!h) return fail(CV_ERR_ARG, "NULL model");
-    if (h->M > 65536) return fail(CV_ERR_UNSUPPORTED, "u16 observations need M <= 65536 (M = %lld)", (long long)h->M);
-    if (h->K > 256) return fail(CV_ERR_UNSUPPORTED, "u8 paths need K <= 256 (K = %d)", h->K);
-    if (h->K > SMALL_K_MAX) return fail(CV_ERR_UNSUPPORTED, "the narrow host formats are implemented for K <= %d", SMALL_K_MAX);
-    h->obs16 = 1; h->path8 = 1;
-    const int rc = decode_batch_host(h, reinterpret_cast<const uint32_t *>(obs_flat), seq_off, B,
-                                     reinterpret_cast<uint32_t *>(path_out), score_out, nullptr, nullptr);
-    h->obs16 = 0; h->path8 = 0;
-    return rc;
-}
-
-static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B, uint32_t *path_out,
-                             double *score_out, uint32_t *d_path_keep, double *d_score_keep)
-{
+    const int64_t B = call.B;
     if (!h) return fail(CV_ERR_ARG, "NULL model");
     if (B < 0) return fail(CV_ERR_ARG, "negative B");
     if (B == 0) return CV_OK;
@@ -1171,12 +1129,11 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
     uint32_t *d_obs = (uint32_t *)h->obs.p, *d_path = d_path_keep ? d_path_keep : (uint32_t *)h->path.p;
     int64_t *d_off = (int64_t *)h->seq_off.p;
     double *d_score = d_score_keep ? d_score_keep : (double *)h->score.p;
-    const bool timing = g_timing.load() != 0;
-    const int nch = chunk_count(h, B, timing, true);
-    const size_t ob = h->obs16 ? 2 : 4, pb = h->path8 ? 1 : 4;
-    if (!timing) {
+    const int nch = chunk_count(h, call, true);
+    const size_t ob = call.obs_bytes(), pb = call.path_bytes();
+    if (!call.timing) {
         bool handled = false;
-        if ((rc = decode_streamed(h, obs_flat, seq_off, B, path_out, score_out, nch, &handled, d_path, d_score))) return rc;
+        if ((rc = decode_streamed(h, call, obs_flat, seq_off, path_out, score_out, nch, &handled, d_path, d_score))) return rc;
         if (handled) return CV_OK;
     }
     // Chunk k: H2D of its observations -> order/forward/backtrace -> D2H of its paths, on stream k % 2, so the
@@ -1191,12 +1148,7 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
     for (int k = 0; k < nck; k++) {
         const int64_t b0 = cb[k], b1 = cb[k + 1];
         int64_t max_len = 0;
-        for (int64_t b = b0; b < b1; b++) {
-            const int64_t len = seq_off[b + 1] - seq_off[b];
-            if (len < 0) return fail(CV_ERR_ARG, "seq_off not monotone at %lld", (long long)b);
-            if (len == 0) return fail(CV_ERR_EMPTY, "sequence %lld is empty (reference: usize underflow panic)", (long long)b);
-            max_len = std::max(max_len, len);
-        }
+        if ((rc = scan_lengths(seq_off, b0, b1, max_len))) return rc;
         DecodeWs &w = h->ws[k & 1];
         cudaStream_t st = nch == 1 ? h->stream : w.st;
         const int64_t e0 = seq_off[b0], e1 = seq_off[b1];
@@ -1204,7 +1156,7 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
         mark(st);
         CUDA_TRY(cudaMemcpyAsync((char *)d_obs + ob * e0, (const char *)obs_flat + ob * e0, ob * (size_t)(e1 - e0), cudaMemcpyHostToDevice, st));
         mark(st);
-        if ((rc = decode_chunk(h, w, d_obs, d_off + b0, b1 - b0, e1 - e0, max_len, d_path, d_score + b0, st, timing, nck == 1))) return rc;
+        if ((rc = decode_chunk(h, call, w, d_obs, d_off + b0, b1 - b0, e1 - e0, max_len, d_path, d_score + b0, st, nck == 1))) return rc;
         mark(st);
         CUDA_TRY(cudaMemcpyAsync((char *)path_out + pb * e0, (const char *)d_path + pb * e0, pb * (size_t)(e1 - e0), cudaMemcpyDeviceToHost, st));
         if (score_out)
@@ -1220,22 +1172,36 @@ static int decode_batch_host(cv_hmm *h, const uint32_t *obs_flat, const int64_t 
         }
         for (cudaEvent_t e : pev) cudaEventDestroy(e);
     }
-    int *hs = (int *)h->pinned_status + 8;
-    hs[0] = hs[1] = 0;
-    if (nch == 1) {
-        CUDA_TRY(cudaMemcpyAsync(hs, (int *)h->ws[0].misc.p + 16, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-        CUDA_TRY(cudaStreamSynchronize(h->stream));
-    } else {
-        for (int k = 0; k < 2; k++) {
-            CUDA_TRY(cudaMemcpyAsync(hs + k, (int *)h->ws[k].misc.p + 16, sizeof(int), cudaMemcpyDeviceToHost, h->ws[k].st));
-            CUDA_TRY(cudaStreamSynchronize(h->ws[k].st));
-        }
-    }
-    if (timing) {
-        float ms = 0.f;
-        if (cudaEventElapsedTime(&ms, h->ev0, h->ev1) == cudaSuccess) h->last_ms = ms; else cudaGetLastError();
-        if (cudaEventElapsedTime(&ms, h->ev1, h->ev2) == cudaSuccess) h->last_bt_ms = ms; else cudaGetLastError();
-    }
-    return report_status(hs, 2);
+    return nch == 1 ? finish_call(h, call, 1, h->stream) : finish_call(h, call, 2, h->ws[0].st, h->ws[1].st);
 }
 
+extern "C" int cv_decode_batch(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                               uint32_t *path_out, double *score_out)
+{
+    return decode_batch_host(h, decode_call(B), obs_flat, seq_off, path_out, score_out);
+}
+
+extern "C" int cv_decode_batch_keep(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                                    uint32_t *path_out, double *score_out, uint32_t *d_path_keep, double *d_score_keep)
+{
+    if (!d_path_keep || !d_score_keep) return fail(CV_ERR_ARG, "NULL device buffer");
+    return decode_batch_host(h, decode_call(B), obs_flat, seq_off, path_out, score_out, d_path_keep, d_score_keep);
+}
+
+extern "C" int cv_decode_batch_f32(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B,
+                                   uint32_t *path_out, double *score_out)
+{
+    if (int rc = check_f32(h)) return rc;
+    return decode_batch_host(h, decode_call(B, true), obs_flat, seq_off, path_out, score_out);
+}
+
+extern "C" int cv_decode_batch_u16u8(cv_hmm *h, const uint16_t *obs_flat, const int64_t *seq_off, int64_t B,
+                                     uint8_t *path_out, double *score_out)
+{
+    if (!h) return fail(CV_ERR_ARG, "NULL model");
+    if (h->M > 65536) return fail(CV_ERR_UNSUPPORTED, "u16 observations need M <= 65536 (M = %lld)", (long long)h->M);
+    if (h->K > 256) return fail(CV_ERR_UNSUPPORTED, "u8 paths need K <= 256 (K = %d)", h->K);
+    if (h->K > SMALL_K_MAX) return fail(CV_ERR_UNSUPPORTED, "the narrow host formats are implemented for K <= %d", SMALL_K_MAX);
+    return decode_batch_host(h, decode_call(B, false, 1, 1), reinterpret_cast<const uint32_t *>(obs_flat), seq_off,
+                             reinterpret_cast<uint32_t *>(path_out), score_out);
+}

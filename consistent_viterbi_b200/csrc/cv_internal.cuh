@@ -8,6 +8,8 @@
 
 #include <cuda_runtime.h>
 
+#include "common.cuh"
+
 #include <algorithm>
 #include <atomic>
 #include <cmath>
@@ -85,6 +87,38 @@ struct DevBuf {
     void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
 };
 
+// ---- fixed layouts: the words of a decode workspace's misc buffer and the handle's pinned host block -----------------
+constexpr int STREAM_MAX_CHUNKS = 16;   // chunks of the streamed host path (cv_api.cu, decode_streamed)
+
+// u32 words of cv_hmm::DecodeWs::misc (MISC_BYTES, zeroed before the keys kernel of every chunk)
+enum MiscWord : int {
+    MISC_COUNTER = 0,         // tile counter of the forward / warp-per-sequence kernel; words 0-1: the large-K item counter (u64)
+    MISC_LONG_COUNTER = 8,    // tile counter of the long-sequence split's warp-per-sequence kernel
+    MISC_LONG_COUNT = 9,      // sequences the long-sequence split moved (LongSplit::n_long)
+    MISC_CERT = 10,           // [4] certified backtrace: flagged sequences, their longest length, their elements (u64)
+    MISC_CERT_COUNTER = 14,   // tile counter of certified_fallback's warp-per-sequence kernel
+    MISC_STATUS = 16,         // device status (int)
+    MISC_MAX_LEN = 17,        // longest length, found by the streamed path's keys kernel
+    MISC_ARRIVED = 32,        // streamed path: chunks whose observations have arrived
+    MISC_CHUNK_DONE = 33,     // streamed path: [STREAM_MAX_CHUNKS] finished sequences per chunk
+};
+constexpr size_t MISC_BYTES = 256;
+static_assert(MISC_CERT % 2 == 0, "the certified element count at MISC_CERT + 2 is a u64");
+static_assert(MISC_MAX_LEN == MISC_STATUS + 1, "decode_streamed reads the status and the longest length in one copy");
+static_assert(sizeof(unsigned int) * (MISC_CHUNK_DONE + STREAM_MAX_CHUNKS) <= MISC_BYTES, "chunk_done lies inside misc");
+
+// byte offsets into cv_hmm::pinned_status (PIN_BYTES of pinned host memory)
+enum PinnedAt : size_t {
+    PIN_CP_BOUND = 8,     // double[3] constrained solver: a node's bound, the peer-timeout flag, the node's sequence number
+    PIN_STATUS = 32,      // int[2] decode status words of the two workspace sets (decode_streamed: status, longest length)
+    PIN_CERT = 64,        // u32[4] the MISC_CERT words (certified_fallback)
+    PIN_LEAF_UB = 1024,   // double[K] leaf-batch bounds of the constrained solver, K <= SMALL_K_MAX
+    PIN_BYTES = 2048,
+};
+static_assert(PIN_CP_BOUND + 3 * sizeof(double) <= PIN_STATUS && PIN_STATUS + 2 * sizeof(int) <= PIN_CERT &&
+              PIN_CERT + 4 * sizeof(unsigned int) <= PIN_LEAF_UB && PIN_LEAF_UB + SMALL_K_MAX * sizeof(double) <= PIN_BYTES,
+              "the pinned words do not overlap");
+
 }  // namespace cvb
 
 // ---- model handle (opaque in the ABI) ------------------------------------------------------------------------------
@@ -99,8 +133,6 @@ struct cv_hmm {
     double *dAb = nullptr, *dBTb = nullptr;
     // f32 mode (decode_f32.cuh): rn32(logA) natural [K][Kp] and slot-permuted [K][Kp], rn32(logB^T) slot-permuted [M][Kp]
     float *dA32n = nullptr, *dA32f = nullptr, *dBT32 = nullptr;
-    int f32mode = 0;                          // the call in progress is cv_decode_batch_f32 / cv_decode_batch_dev_f32
-    int64_t f32_call_B = 0;                   // its batch size: the kernel choice is made once per call (chain_batch)
     bool f32_range_ok = false;                // every finite model entry has |x| <= 2^64 (cv_hmm_create)
     // the exact decode may run the f32 forward pass and certify it (decode_small.cuh, certified backtrace): K <= 64,
     // f32_range_ok and every finite entry of logA / logB <= 0
@@ -131,6 +163,8 @@ struct cv_hmm {
         cudaEvent_t done = nullptr;
         cudaStream_t st_bt = nullptr;                      // concurrent backtrace (launch_decode_small)
         cudaEvent_t ev_pre = nullptr, ev_bt = nullptr;
+        unsigned int *word(cvb::MiscWord i) const { return (unsigned int *)misc.p + i; }
+        int *status() const { return (int *)word(cvb::MISC_STATUS); }
     } ws[2];
     cudaEvent_t ev_fork = nullptr;
     cudaStream_t st_long = nullptr;                        // warp-per-sequence kernel for the long sequences of a tile launch
@@ -139,9 +173,9 @@ struct cv_hmm {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr, ev2 = nullptr;
     double last_ms = 0.0, last_bt_ms = 0.0;   // forward kernel / backtrace kernel
-    int obs16 = 0, path8 = 0;                 // host formats of the call in progress (cv_decode_batch_u16u8), else 0
     // CP debug state
     int64_t cp_N = 0;
     std::vector<double> cp_ub;
-    void *pinned_status = nullptr;
+    void *pinned_status = nullptr;            // cvb::PIN_BYTES, laid out as cvb::PinnedAt
+    template <class T> T *pinned(cvb::PinnedAt at) const { return (T *)((char *)pinned_status + at); }
 };
