@@ -91,6 +91,7 @@ SIGNATURES = {
 DEBUG_SIGNATURES = {
     "cv_debug_cp_last_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "cv_debug_cp_last_ub": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, _u64p]),
+    "cv_debug_cp_last_paths": (C.c_uint32, [C.c_void_p]),
     "cv_debug_ordered_sum": (C.c_int, [C.c_void_p, C.c_int64, C.c_int, _dp]),
     "cv_debug_set_chunks": (None, [C.c_int]),
     "cv_debug_set_chain_max_batch": (None, [C.c_longlong]),

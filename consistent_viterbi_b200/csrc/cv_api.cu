@@ -549,14 +549,14 @@ static int launch_chain_kernel(const cv_hmm *h, const DecodeChainParams &p, int 
         kern<<<grid, 32 * DC_WARPS, smem, st>>>(p);
         return CV_OK;
     };
-    const bool regs = h->Kp == 8 * ((h->K + 7) / 8);     // register-resident logA column needs Kp = 4 * KQ
+    // every model has Kp = 8 G (cv_hmm_create), so K <= 32 always fits the register-resident column of 4 KQ = Kp
     int rc;
-    switch (regs ? (h->K + 7) / 8 : 9) {
+    switch (h->G) {
         case 1: rc = go(decode_chain_kernel<1, 2>); break;
         case 2: rc = go(decode_chain_kernel<1, 4>); break;
         case 3: rc = go(decode_chain_kernel<1, 6>); break;
         case 4: rc = go(decode_chain_kernel<1, 8>); break;
-        default: rc = h->K <= 32 ? go(decode_chain_kernel<1, 0>) : go(decode_chain_kernel<2, 0>);
+        default: rc = go(decode_chain_kernel<2, 0>);
     }
     if (rc) return rc;
     g_launches++;

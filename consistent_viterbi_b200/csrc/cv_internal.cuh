@@ -176,6 +176,7 @@ struct cv_hmm {
     // CP debug state
     int64_t cp_N = 0;
     std::vector<double> cp_ub;
+    uint32_t cp_paths = 0;                    // CV_CP_PATH_* bits of the last solve (cv_debug_cp_last_paths)
     void *pinned_status = nullptr;            // cvb::PIN_BYTES, laid out as cvb::PinnedAt
     template <class T> T *pinned(cvb::PinnedAt at) const { return (T *)((char *)pinned_status + at); }
 };

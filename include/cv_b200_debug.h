@@ -64,6 +64,28 @@ int64_t cv_debug_last_flagged(const cv_hmm *h);
 int cv_debug_cp_last_state(cv_hmm *h, double *delta_out, uint64_t *psi_out);
 int cv_debug_cp_last_ub(cv_hmm *h, double *ub_out, uint64_t cap, uint64_t *n_out);
 
+/* Launch paths the last cv_cp_solve / cv_cp_solve_dist on h took: an OR of the CV_CP_PATH_* bits below, cleared on
+ * entry and set by the host at each launch site.  Tests assert them so that a case cannot drift off the path it is
+ * meant to cover when a selection rule changes. */
+uint32_t cv_debug_cp_last_paths(const cv_hmm *h);
+#define CV_CP_PATH_SWEEP_1_2_16   (1u << 0)   /* warp-per-segment sweep, K <= 8, two segments per warp */
+#define CV_CP_PATH_SWEEP_1_4_16   (1u << 1)   /* K = 9..16, two segments per warp */
+#define CV_CP_PATH_SWEEP_1_6      (1u << 2)   /* K = 17..24 */
+#define CV_CP_PATH_SWEEP_1_8      (1u << 3)   /* K = 25..32 */
+#define CV_CP_PATH_SWEEP_2_0      (1u << 4)   /* K = 33..64, two states per lane, logA column from shared memory */
+#define CV_CP_PATH_SWEEP_GENERIC  (1u << 5)   /* K > 64 */
+#define CV_CP_PATH_SWEEP_FW_1_2   (1u << 6)   /* CV_CP_FULLWARP: K <= 8, one segment per warp */
+#define CV_CP_PATH_SWEEP_FW_1_4   (1u << 7)   /* CV_CP_FULLWARP: K = 9..16, one segment per warp */
+#define CV_CP_PATH_BT_IN_SMEM     (1u << 8)   /* logB^T staged in shared memory by the warp-per-segment sweep */
+#define CV_CP_PATH_BTR_ROWS_GMEM  (1u << 9)   /* backtrack maps / fill walk psi in global memory (K too large to stage) */
+#define CV_CP_PATH_BTR_CHAIN_GMEM (1u << 10)  /* backtrack entry chain walked by one thread from global memory */
+#define CV_CP_PATH_SUM_LOOP       (1u << 11)  /* bound sum: one-thread loop */
+#define CV_CP_PATH_SUM_BLOCKS     (1u << 12)  /* bound sum: block-structured exact-order kernels */
+#define CV_CP_PATH_SUM_PREFIX     (1u << 13)  /* bound sum: block-structured, block prefixes from their own kernel */
+#define CV_CP_PATH_SUM_ONE_CTA    (1u << 14)  /* bound sum: single-CTA binade scan */
+#define CV_CP_PATH_LEAF_BATCH     (1u << 15)  /* the siblings of the last component evaluated as one batch */
+#define CV_CP_PATH_BOUND_COPY     (1u << 16)  /* CV_CP_HOSTPOLL=0: a node's bound copied back and the stream synchronised */
+
 /* Parity hook for the bound sum of solve_r (cp.rs:103-116): ((0.0 + v[0]) + v[1]) + ... of n host values,
  * mode 0 = one-thread loop, mode 1 = the parallel exact-order kernel; both must agree bit for bit. */
 int cv_debug_ordered_sum(const double *values, int64_t n, int mode, double *out);

@@ -5,12 +5,13 @@ import pytest
 
 import consistent_viterbi_b200 as cv
 from oracle import pyoracle as po
-from util import random_hmm, random_superseq
+from util import cp_path_bits, random_hmm, random_superseq
 
 pytestmark = pytest.mark.gpu
 
 
 def _check(A, B, pi, obs, start, comp, ncomp, max_nodes=0):
+    """Returns the solve's launch path bits (cv_debug_cp_last_paths), 0 when both sides raised."""
     h = cv.HMM(A, B, pi)
     try:
         ref = po.cp_solve(A, B, pi, obs, start, comp, ncomp, max_nodes=max_nodes, trace_nodes=1 << 16, want_state=True)
@@ -25,7 +26,7 @@ def _check(A, B, pi, obs, start, comp, ncomp, max_nodes=0):
     assert ref_err == got_err, (ref_err, got_err)
     if ref_err is not None:
         h.close()
-        return
+        return 0
     assert got["explored"] == ref["explored"]
     assert got["steps"] == ref["steps"]
     n = min(len(got["ub"]), int(ref["explored"]))
@@ -34,7 +35,9 @@ def _check(A, B, pi, obs, start, comp, ncomp, max_nodes=0):
     assert (got["sol"] == ref["sol"]).all()
     assert got["delta"].tobytes() == ref["delta"].tobytes(), "final delta state differs"
     assert (got["psi"] == ref["psi"]).all(), "final psi state differs"
+    paths = cv._lib.lib().cv_debug_cp_last_paths(h.device_handle())
     h.close()
+    return paths
 
 
 @pytest.mark.parametrize("seed", range(8))
@@ -47,13 +50,18 @@ def test_cp_random_small(seed):
         _check(A, B, pi, obs, start, comp, ncomp)
 
 
-@pytest.mark.parametrize("K", [8, 9, 12, 16, 24, 45])
+@pytest.mark.parametrize("K", [8, 9, 12, 16, 24, 25, 28, 32, 34, 45, 57, 63, 64])
 def test_cp_mid_k(K):
+    """Every warp-per-segment sweep shape: its path bit (include/cv_b200_debug.h) must be the one K selects."""
     rng = np.random.default_rng(600 + K)
     M = 12
     A, B, pi = random_hmm(rng, K, M, zero_frac=0.1)
     obs, start, comp, ncomp = random_superseq(rng, 30, M, 3, 0.08, 5, 60)
-    _check(A, B, pi, obs, start, comp, ncomp, max_nodes=60)
+    paths = _check(A, B, pi, obs, start, comp, ncomp, max_nodes=60)
+    P = cp_path_bits()
+    want = ["SWEEP_1_2_16", "SWEEP_1_4_16", "SWEEP_1_6", "SWEEP_1_8"][(K + 7) // 8 - 1] if K <= 32 else "SWEEP_2_0"
+    sweeps = P["SWEEP_1_2_16"] | P["SWEEP_1_4_16"] | P["SWEEP_1_6"] | P["SWEEP_1_8"] | P["SWEEP_2_0"]
+    assert paths & sweeps == P[want], hex(paths)
 
 
 @pytest.mark.parametrize("K", [65, 100, 130, 300])

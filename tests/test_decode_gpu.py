@@ -48,15 +48,33 @@ def test_large_k_random(K, Bn, tmax):
     _check(A, B, pi, obs, off)
 
 
-def test_large_k_batch_groups(monkeypatch):
+def test_large_k_batch_groups():
     """The delta history of a large-K batch is processed in groups of row blocks when it does not fit in HBM;
-    force groups of one and two row blocks."""
+    force groups of one and two row blocks.  B = 300 is five row blocks of 64: 5, 3 and 1 groups, and every group
+    launches three kernels (items per step, forward, backtrace)."""
     rng = np.random.default_rng(3200)
     A, B, pi = random_hmm(rng, 140, 9, zero_frac=0.3)
     obs, off = random_batch(rng, 300, 9, 1, 14)
-    for rb in ("1", "2"):
-        monkeypatch.setenv("CV_LARGE_GROUP_RB", rb)
-        _check(A, B, pi, obs, off)
+    rp, rs = po.decode_batch(A, B, obs, off, nthreads=8)
+    h = cv.HMM(A, B, pi)
+    L = cv._lib.lib()
+    launches = {}
+    L.cv_debug_set_chunks(1)
+    try:
+        cv.decode_batch(h, obs, off)                              # the model's device set-up launches kernels too
+        for rb in (0, 1, 2):
+            L.cv_debug_set_large_group_rb(rb)
+            n0 = L.cv_launch_count()
+            paths, scores = cv.decode_batch(h, obs, off)
+            launches[rb] = L.cv_launch_count() - n0
+            assert (paths == rp).all(), f"rb={rb}: path mismatches"
+            assert scores.tobytes() == rs.tobytes(), f"rb={rb}: scores differ"
+    finally:
+        L.cv_debug_set_large_group_rb(0)
+        L.cv_debug_set_chunks(-1)
+        h.close()
+    assert launches[1] - launches[0] == 3 * (5 - 1), launches
+    assert launches[2] - launches[0] == 3 * (3 - 1), launches
 
 
 def test_large_k_ties():

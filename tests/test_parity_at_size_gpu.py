@@ -11,6 +11,7 @@ import pytest
 
 import consistent_viterbi_b200 as cv
 from oracle import pyoracle as po
+from test_cp_paths_gpu import _check, _expect, _superseq_n
 from util import random_hmm
 
 pytestmark = pytest.mark.gpu
@@ -159,3 +160,19 @@ def test_chain_kernel_on_a_multi_chunk_call(K):
         L.cv_debug_set_chunks(-1)
         L.cv_debug_set_pipeline(1, 1)
     h.close()
+
+
+@pytest.mark.parametrize("N", [402945, 402946])
+def test_backtrack_chain_smem_edge(N):
+    """K = 64: the chunk maps of N - 1 = 402 944 rows (1574 chunks) fit the entry chain's shared memory, one row more
+    (1575 chunks) and one thread walks them in global memory.  The only component sits in the last rows, so the
+    oracle's cost is the unconstrained prefix, N K^2 = 1.7e9 cell updates, once (about a minute per case)."""
+    rng = np.random.default_rng(7700 + N)
+    K, M = 64, 20
+    A, B, pi = random_hmm(rng, K, M, zero_frac=0.0)
+    obs, start, comp = _superseq_n(rng, N, M, 5, 40)
+    comp[[N - 180, N - 120, N - 61, N - 1]] = 0
+    paths, got = _check(A, B, pi, obs, start, comp, 1, state=False)
+    assert got["obj"] > -np.inf
+    _expect(paths, on=["SWEEP_2_0", "LEAF_BATCH"] + (["BTR_CHAIN_GMEM"] if N > 402945 else []),
+            off=["BTR_ROWS_GMEM"] + ([] if N > 402945 else ["BTR_CHAIN_GMEM"]))

@@ -1,7 +1,17 @@
 """Shared generators for the parity tests (seeded, numpy only)."""
 from __future__ import annotations
 
+import os
+import re
+
 import numpy as np
+
+
+def cp_path_bits():
+    """{name: bit} of the CV_CP_PATH_* launch-path bits of include/cv_b200_debug.h (cv_debug_cp_last_paths)."""
+    with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "cv_b200_debug.h")) as f:
+        text = f.read()
+    return {m.group(1): 1 << int(m.group(2)) for m in re.finditer(r"#define CV_CP_PATH_(\w+)\s+\(1u << (\d+)\)", text)}
 
 
 def random_hmm(rng, K, M, zero_frac=0.2, alpha=0.5, ties=False):
