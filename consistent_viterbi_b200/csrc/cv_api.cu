@@ -564,6 +564,46 @@ static int launch_chain_kernel(const cv_hmm *h, const DecodeChainParams &p, int 
     return CV_OK;
 }
 
+// Residency budget of a forward kernel that a backtrace kernel runs beside (launch_decode_small, concurrent mode): the
+// most forward CTAs per SM, at most occ, that leave room on the SM for at least one backtrace CTA (bt, bt_threads,
+// bt_smem) -- registers, shared memory with the per-CTA reservation, threads and CTA slots, from the device's
+// per-SM limits and the kernels' attributes.  The block scheduler puts as many forward CTAs on an SM as its resources
+// allow, so a grid of n CTAs per SM alone does not keep the room free: when n < occ, fwd_smem is padded to the
+// smallest size at which n + 1 forward CTAs no longer fit on an SM.  Returns n (fwd_smem updated), or 0 when not even
+// one forward CTA leaves room (fwd_smem unchanged; the backtrace then waits for forward CTAs to exit).
+static int residency_budget(int dev, void (*fwd)(DecodeSmallParams), int fwd_threads, size_t &fwd_smem,
+                            void (*bt)(DecodeSmallParams), int bt_threads, size_t bt_smem, int occ)
+{
+    int regs_sm = 0, smem_sm = 0, resv = 0, threads_sm = 0, ctas_sm = 0;
+    cudaFuncAttributes af, ab;
+    if (cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&resv, cudaDevAttrReservedSharedMemoryPerBlock, dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&threads_sm, cudaDevAttrMaxThreadsPerMultiProcessor, dev) != cudaSuccess ||
+        cudaDeviceGetAttribute(&ctas_sm, cudaDevAttrMaxBlocksPerMultiprocessor, dev) != cudaSuccess ||
+        cudaFuncGetAttributes(&af, fwd) != cudaSuccess || cudaFuncGetAttributes(&ab, bt) != cudaSuccess) {
+        cudaGetLastError();
+        return 0;
+    }
+    // registers are allocated per warp in units of 256, shared memory per CTA in units of 128 bytes
+    auto regs_cta = [](const cudaFuncAttributes &a, int threads) -> int64_t {
+        return (int64_t)((threads + 31) / 32) * ((a.numRegs * 32 + 255) / 256 * 256);
+    };
+    auto smem_cta = [&](const cudaFuncAttributes &a, size_t dyn) -> int64_t {
+        return (int64_t)((a.sharedSizeBytes + dyn + 127) / 128 * 128) + resv;
+    };
+    const int64_t rf = regs_cta(af, fwd_threads), rb = regs_cta(ab, bt_threads), sb = smem_cta(ab, bt_smem);
+    for (int n = occ; n >= 1; n--) {
+        if (n * rf + rb > regs_sm || n * fwd_threads + bt_threads > threads_sm || n + 1 > ctas_sm) continue;
+        int64_t sf = smem_cta(af, fwd_smem);
+        if (n < occ) sf = std::max(sf, ((int64_t)smem_sm / (n + 1) + 1 + 127) / 128 * 128);
+        if (n * sf + sb > smem_sm) continue;
+        fwd_smem = (size_t)(sf - resv - (int64_t)af.sharedSizeBytes);
+        return n;
+    }
+    return 0;
+}
+
 // Parameters of the warp-per-sequence kernel over the sequences order[0, B) with workspace set w: backpointer rows in
 // psi, tile counter in the misc word `counter`.  B_dev: the number of sequences is read on the device (at most B), and
 // the rows of list entry r start at row r * psi_stride.  sio: finished sequences are counted per chunk (streamed path).
@@ -648,7 +688,13 @@ static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, c
         p.arrived = sio->d_arrived; p.chunk_done = sio->d_chunk_done; p.nch = sio->cbs.nch;
         for (int c = 0; c <= sio->cbs.nch; c++) p.cb[c] = sio->cbs.cb[c];
     }
-    void (*kern)(DecodeSmallParams) = f32 ? decode_f32_fwd_kernel : decode_small_fwd_kernel<0>;
+    // f32: the 64-register build of the forward kernel leaves room for the concurrent backtrace and hides it behind a
+    // long batch's forward pass (1 M POS sentences: 7.3 -> 6.6 ms per certified step); a short batch -- a few tiles per
+    // CTA, the same bound as the four-lane backtrace's -- cannot hide it and runs the faster 78-register build
+    // (125 k sentences: 1.58 ms per step with it, 1.71 ms with the 64-register build).
+    const bool long_batch = B > (int64_t)1300 * h->num_sms;
+    void (*kern)(DecodeSmallParams) = !f32 ? decode_small_fwd_kernel<0>
+                                    : long_batch ? decode_f32_fwd_kernel<4> : decode_f32_fwd_kernel<3>;
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     int occ = 1;
@@ -667,10 +713,6 @@ static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, c
         }
         if (occ_c >= occ) { kern = kc; smem = smem_c; }
     }
-    const int grid = (int)std::min<int64_t>((int64_t)h->num_sms * occ, ntiles);
-    if (g_tune.debug)
-        fprintf(stderr, "[cv] decode_small: K=%d G=%d f32=%d cert=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
-                h->K, G, (int)f32, (int)cert, threads, smem, occ, grid, ntiles);
     // Concurrent backtrace: the backtrace kernel runs next to the forward kernel on a second stream and follows
     // it tile by tile (tile_done flags).  It is released only when every forward CTA is resident (stream wait on
     // the `started` counter), so its spinning CTAs can never keep a forward CTA off an SM; it then lives on the
@@ -678,6 +720,24 @@ static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, c
     StreamValue32Fn wait32 = stream_wait_value32();
     const bool concurrent = !call.timing && g_tune.bt_concurrent && wait32 != nullptr && w.st_bt != nullptr;
     if (sio && !concurrent) return fail(CV_ERR_UNSUPPORTED, "the streamed path needs the concurrent backtrace");
+    // end state + backtrace with lazy backpointers: one thread per sequence
+    const size_t smem_bt = (size_t)h->K * (h->K | 1) * 8 + 16 * 8;      // + one chunk of padding behind the last row
+    void (*bt_seq)(DecodeSmallParams) = cert ? backtrace_small_kernel<16, 4, float, true>
+                                      : f32 ? backtrace_small_kernel<16, 4, float> : backtrace_small_kernel<16, 4>;
+    void (*bt_con)(DecodeSmallParams) = cert ? backtrace_small_kernel<8, 8, float, true>
+                                      : f32 ? backtrace_small_kernel<8, 8, float> : backtrace_small_kernel<8, 8>;
+    // The f32 forward kernel alone fills an SM's registers (four CTAs at K = 45): make room for the backtrace
+    if (f32 && concurrent) {
+        if (int n = residency_budget(h->device, kern, threads, smem, bt_con, 128, smem_bt, occ)) {
+            CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem));
+            if (occ != n) return fail(CV_ERR_CUDA, "forward CTAs per SM: %d, budget %d", occ, n);
+        }
+    }
+    const int grid = (int)std::min<int64_t>((int64_t)h->num_sms * occ, ntiles);
+    if (g_tune.debug)
+        fprintf(stderr, "[cv] decode_small: K=%d G=%d f32=%d cert=%d threads=%d smem=%zu occ=%d grid=%d tiles=%d\n",
+                h->K, G, (int)f32, (int)cert, threads, smem, occ, grid, ntiles);
     p.tile_done = nullptr; p.started = nullptr;
     if (concurrent) {
         if ((rc = w.lg_done.ensure(sizeof(int) * ((size_t)ntiles + 8)))) return rc;
@@ -706,12 +766,6 @@ static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, c
     g_launches++;
     CUDA_TRY(cudaGetLastError());
     if (call.timing || bt_prof) CUDA_TRY(cudaEventRecord(h->ev1, st));
-    // end state + backtrace with lazy backpointers: one thread per sequence
-    const size_t smem_bt = (size_t)h->K * (h->K | 1) * 8 + 16 * 8;      // + one chunk of padding behind the last row
-    void (*bt_seq)(DecodeSmallParams) = cert ? backtrace_small_kernel<16, 4, float, true>
-                                      : f32 ? backtrace_small_kernel<16, 4, float> : backtrace_small_kernel<16, 4>;
-    void (*bt_con)(DecodeSmallParams) = cert ? backtrace_small_kernel<8, 8, float, true>
-                                      : f32 ? backtrace_small_kernel<8, 8, float> : backtrace_small_kernel<8, 8>;
     // Four lanes per sequence (backtrace_split_kernel, f64 only) -- for batches that do
     // not fill the GPU for long (a rank's slice of a sharded batch): there the one-thread-per-sequence kernel is latency
     // bound and most of its work is still open when the forward kernel ends.  Measured, device step with the concurrent

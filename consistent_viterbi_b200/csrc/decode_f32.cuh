@@ -14,6 +14,11 @@
 // of <= 8 target states of the balanced split, emission rows by TMA, one TMA bulk store of the [K][64] slab per step),
 // at half the shared memory (46 KB at K = 45: four CTAs per SM).
 //
+// MINB = 4 caps the kernel at 64 registers (78 uncapped; the 8 + 24 bytes of spills are in the per-tile prologue and
+// epilogue, none in the step loop): then four forward CTAs of six warps (K = 45) and two CTAs of the concurrent
+// backtrace share an SM's registers, and the backtrace of a long batch runs beside the forward pass instead of after it.
+// The cap costs the kernel ~10 % alone, so short batches run the uncapped build (MINB = 3; launch_decode_small).
+//
 // The exact decode of an eligible model (cv_hmm_create: every finite entry <= 0 and |x| <= 2^64) runs this kernel as
 // well: backtrace_small_kernel<.., float, true> then certifies every backpointer against the f64 recurrence (the
 // bound is derived above that kernel) and the sequences it cannot certify are decoded again in f64.
@@ -38,7 +43,8 @@ __host__ __device__ inline size_t decode_f32_smem_bytes(int K, int Kp)
     return (size_t)K * Kp * 4 + (size_t)2 * K * 64 * 4 + (size_t)64 * f32_em_pitch(Kp) * 4 + 64 * (8 + 4) + 32 + 16;
 }
 
-__global__ void __launch_bounds__(256, 3) decode_f32_fwd_kernel(const DecodeSmallParams p)
+template <int MINB>
+__global__ void __launch_bounds__(256, MINB) decode_f32_fwd_kernel(const DecodeSmallParams p)
 {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr int NS = 64;
