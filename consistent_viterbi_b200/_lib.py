@@ -108,6 +108,8 @@ DEBUG_SIGNATURES = {
     "cv_debug_set_certified": (None, [C.c_int]),
     "cv_debug_set_cert_tolerance": (None, [C.c_double]),
     "cv_debug_last_flagged": (C.c_int64, [C.c_void_p]),
+    "cv_debug_set_fallback": (None, [C.c_int, C.c_longlong]),
+    "cv_debug_last_fallback_chain": (C.c_int64, [C.c_void_p]),
 }
 
 

@@ -624,14 +624,14 @@ static DecodeChainParams chain_params(const cv_hmm *h, const DecodeCall &call, c
     return q;
 }
 
-// The tile path of workspace set w: forward kernel over tiles of 64 sequences ordered longest first (w.order), then the
-// backtrace.  The tile counter and the status are w's misc words.
+// The tile path of workspace set w: forward kernel over tiles of 64 sequences ordered longest first (w.order from rank
+// `first` on), then the backtrace.  The tile counter and the status are w's misc words.
 static int launch_decode_small(cv_hmm *h, const DecodeCall &call, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off,
                                int64_t B, int64_t N, uint32_t *d_path, double *d_score, int64_t max_len, cudaStream_t st,
-                               bool cert, const StreamedIO *sio = nullptr, const LongSplit *ls = nullptr)
+                               bool cert, const StreamedIO *sio = nullptr, const LongSplit *ls = nullptr, int64_t first = 0)
 {
     const int G = h->G;
-    const uint32_t *d_order = (const uint32_t *)w.order.p, *d_sorted_len = (const uint32_t *)w.keys_out.p;
+    const uint32_t *d_order = (const uint32_t *)w.order.p + first, *d_sorted_len = (const uint32_t *)w.keys_out.p + first;
     // optional f32 mode (decode_f32.cuh): its own forward kernel, f32 history, f32 backtrace.  cert: the same forward
     // kernel and history, then the certified backtrace (decode_small.cuh) -- the exact decode of an eligible model
     const bool f32 = call.f32 || cert;
@@ -835,10 +835,39 @@ __global__ void listed_len_keys_kernel(const int64_t *seq_off, const uint32_t *l
     vals[i] = b;
 }
 
+// How many of the n flagged sequences (longest lmax) certified_fallback gives the warp-per-sequence kernel.
+// - Up to CHAIN_BATCH_MAX: all of them, as a batch of n would go there (chain_batch).
+// - Up to two tiles per SM: the tile path is one wave of about one tile per CTA, in lock step for as many steps as its
+//   longest tile, and flagged sequences are the long ones (the certificate's bound grows with the step).  The
+//   FB_CHAIN_PER_SM * num_sms longest go to the warp-per-sequence kernel beside it, one warp each.  Measured on one
+//   NVIDIA B200 (148 SMs), fallback with its host round trip: 1 M POS sentences (17 369 flagged) 1.34-1.46 ms on the
+//   tiles alone, 0.81-0.89 ms with 296-592 on the warp kernel, 1.35 ms with 4736 and 1.36 ms with all of them (a warp
+//   then decodes several sequences, at 1-2 us per step beside the tile kernel); 500 k (8494 flagged) 1.08 ms on the
+//   tiles, 0.59-0.66 ms with 148-296, 0.74 ms with all of them.
+// - More: the tile scheduler balances several waves of tiles, and the warp kernel beside them only takes issue slots
+//   (tie-heavy model, 124 952 flagged: 1.45 ms on the tiles, 1.50 ms with 296 on the warp kernel).
+constexpr int64_t FB_CHAIN_PER_SM = 2;
+static int64_t fallback_chain_count(const cv_hmm *h, int64_t n, int64_t lmax)
+{
+    int64_t k;
+    switch (g_tune.fb_route) {
+        case 1: k = 0; break;
+        case 2: k = n; break;
+        case 3: k = g_tune.fb_chain; break;
+        default:
+            if (n <= CHAIN_BATCH_MAX) return n;
+            if (n > (int64_t)2 * 64 * h->num_sms) return 0;
+            // backpointer rows of the moved sequences: at most 512 MB
+            k = std::min<int64_t>(FB_CHAIN_PER_SM * h->num_sms, ((int64_t)512 << 20) / (lmax * h->Kp));
+    }
+    return std::max<int64_t>(0, std::min(k, n));
+}
+
 // Exact f64 re-decode of the sequences the certified backtrace could not certify (launch_decode_small with cert): their
 // paths and scores are overwritten.  This is the one host round trip of a certified call: the flagged count, their
-// longest length and their elements are read back, and decide the kernel -- the warp-per-sequence kernel for as many
-// sequences as a batch would give it (chain_batch), else the f64 tile path over the flagged sequences ordered by length.
+// longest length and their elements are read back, and decide the kernels (fallback_chain_count): the warp-per-sequence
+// kernel for all of them, or the flagged sequences ordered by length with the longest on the warp-per-sequence kernel
+// (stream st_long) and the rest on the f64 tile path beside it.
 static int certified_fallback(cv_hmm *h, const DecodeCall &call, DecodeWs &w, const uint32_t *d_obs, const int64_t *d_off,
                               uint32_t *d_path, double *d_score, cudaStream_t st)
 {
@@ -848,10 +877,13 @@ static int certified_fallback(cv_hmm *h, const DecodeCall &call, DecodeWs &w, co
     const int64_t n = hc[0], lmax = hc[1];
     const int64_t nel = (int64_t)*reinterpret_cast<const unsigned long long *>(hc + 2);
     h->last_flagged = n;
+    h->last_fb_chain = 0;
     if (n == 0) return CV_OK;
     const uint32_t *list = (const uint32_t *)w.cert_list.p;
+    const int64_t n_chain = fallback_chain_count(h, n, lmax);
+    h->last_fb_chain = n_chain;
     int rc;
-    if (n <= CHAIN_BATCH_MAX) {
+    if (n_chain == n) {
         // the f32 history is no longer needed: its buffer takes the backpointer rows
         if ((rc = w.hist.ensure((size_t)n * (size_t)lmax * h->Kp + 64))) return rc;
         const DecodeChainParams q = chain_params(h, call, w, d_obs, d_off, d_path, d_score, list, w.hist.p, MISC_CERT_COUNTER,
@@ -863,9 +895,34 @@ static int certified_fallback(cv_hmm *h, const DecodeCall &call, DecodeWs &w, co
     g_launches++;
     if ((rc = sort_desc(w, n, key_bits(lmax), st))) return rc;
     CUDA_TRY(cudaMemsetAsync(w.word(MISC_COUNTER), 0, sizeof(unsigned int), st));
+    if (n_chain > 0) {
+        // the n_chain longest (w.order[0, n_chain)) on the warp-per-sequence kernel; its backpointer rows go to long_psi
+        // because the tile path writes its history to w.hist at the same time.  Its count is read on the device: the
+        // flagged count is at least n_chain.
+        if ((rc = w.long_psi.ensure((size_t)n_chain * (size_t)lmax * h->Kp + 64))) return rc;
+        const DecodeChainParams q = chain_params(h, call, w, d_obs, d_off, d_path, d_score, (const uint32_t *)w.order.p,
+                                                 w.long_psi.p, MISC_CERT_COUNTER, n_chain, w.word(MISC_CERT), lmax);
+        CUDA_TRY(cudaEventRecord(h->ev_long_dep, st));                        // the sorted order is done
+        CUDA_TRY(cudaStreamWaitEvent(h->st_long, h->ev_long_dep, 0));
+        const int grid = (int)std::min<int64_t>((n_chain + DC_WARPS - 1) / DC_WARPS, (int64_t)h->num_sms);
+        if ((rc = launch_chain_kernel(h, q, grid, h->st_long))) return rc;
+        CUDA_TRY(cudaEventRecord(h->ev_long_done, h->st_long));
+    }
     DecodeCall exact = call;
     exact.timing = false;                     // the call's kernel times stay those of the certified pass
-    return launch_decode_small(h, exact, w, d_obs, d_off, n, nel, d_path, d_score, lmax, st, false);
+    if ((rc = launch_decode_small(h, exact, w, d_obs, d_off, n - n_chain, nel, d_path, d_score, lmax, st, false, nullptr,
+                                  nullptr, n_chain)))
+        return rc;
+    if (n_chain > 0) CUDA_TRY(cudaStreamWaitEvent(st, h->ev_long_done, 0));
+    if (g_tune.bt_prof) {
+        CUDA_TRY(cudaEventRecord(h->ev2, st));
+        CUDA_TRY(cudaStreamSynchronize(st));
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, h->ev0, h->ev2);
+        fprintf(stderr, "[cv] fallback: %lld flagged, %lld on the warp kernel, tiles + warp kernel %.3f ms\n",
+                (long long)n, (long long)n_chain, ms);
+    }
+    return CV_OK;
 }
 
 // One chunk of sequences [0, B) of d_off (offsets are absolute into d_obs / d_path): order by length,

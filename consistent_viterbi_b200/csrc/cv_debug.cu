@@ -25,6 +25,8 @@ extern "C" void cv_debug_set_fb_chunk_seqs(int64_t n) { g_tune.fb_chunk_seqs = n
 extern "C" void cv_debug_set_certified(int on) { g_tune.certified = on; }
 extern "C" void cv_debug_set_cert_tolerance(double scale) { g_tune.cert_tol = scale; }
 extern "C" int64_t cv_debug_last_flagged(const cv_hmm *h) { return h ? h->last_flagged : -1; }
+extern "C" void cv_debug_set_fallback(int route, long long n_chain) { g_tune.fb_route = route; g_tune.fb_chain = n_chain; }
+extern "C" int64_t cv_debug_last_fallback_chain(const cv_hmm *h) { return h ? h->last_fb_chain : 0; }
 
 // ---------------------------------------------------------------------------
 // FP64 probe

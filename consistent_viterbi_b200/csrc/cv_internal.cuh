@@ -61,6 +61,8 @@ struct Tuning {
     int cp_fullwarp = 0, cp_prof = 0, cp_sum = -1, cp_hostpoll = 1, cp_leaf_batch = 1;   // constrained solver (CV_CP_*)
     int certified = 1;             // eligible models: f32 forward pass + certified backtrace + exact fallback (cv_debug_set_certified)
     double cert_tol = 1.0;         // scale of the certified backtrace's error bound (cv_debug_set_cert_tolerance)
+    int fb_route = 0;              // certified fallback: 0 = automatic, 1 = tiles, 2 = warp kernel, 3 = the fb_chain longest on the warp kernel (cv_debug_set_fallback)
+    long long fb_chain = 0;
 };
 extern Tuning g_tune;
 
@@ -138,6 +140,7 @@ struct cv_hmm {
     // f32_range_ok and every finite entry of logA / logB <= 0
     bool cert_ok = false;
     int64_t last_flagged = -1;                // sequences the last decode call re-decoded in f64; -1: not certified
+    int64_t last_fb_chain = 0;                // of those, the ones the warp-per-sequence kernel decoded (the rest: tiles)
     // large-K layout
     int Kl = 0;              // K padded to a multiple of LARGE_BN
     double *dAl = nullptr;   // [Kl][Kl]

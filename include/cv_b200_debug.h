@@ -58,6 +58,13 @@ void cv_debug_set_cert_tolerance(double scale);
 /* sequences the last decode call on h re-decoded in f64 after the certified backtrace; -1 = that call did not take
  * the certified path */
 int64_t cv_debug_last_flagged(const cv_hmm *h);
+/* route of the certified decode's f64 re-decode: 0 (default) = automatic, 1 = every flagged sequence on the tile path,
+ * 2 = every one on the warp-per-sequence kernel, 3 = the n_chain longest on the warp-per-sequence kernel beside the
+ * tile path, which takes the rest (n_chain is clipped to [0, flagged]) */
+void cv_debug_set_fallback(int route, long long n_chain);
+/* of the sequences cv_debug_last_flagged counts, the ones the warp-per-sequence kernel decoded; the rest went to the
+ * tile path */
+int64_t cv_debug_last_fallback_chain(const cv_hmm *h);
 
 /* Parity hooks for the CP path: after cv_cp_solve, copy out the final delta[N*K] / psi[N*K] state and the per-node
  * upper bounds (first `cap` nodes). */

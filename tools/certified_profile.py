@@ -3,6 +3,10 @@ certification, how many sequences were flagged and what their f64 re-decode cost
 f64 path; the results checked byte for byte against that path.
 
   python tools/certified_profile.py [--nseq 1000000 125000] [--steps 10] [--out profile.json]
+                                    [--routes tile chain 1184 2368 4736 ...]
+
+--routes also times the step with the fallback's route forced (cv_debug_set_fallback): `tile`, `chain`, or a number of
+the longest flagged sequences given to the warp-per-sequence kernel beside the tile path (route_step_ms).
 
 Per workload (the POS shape of bench.py at each size, and the POS lengths on a tie-heavy model of dyadic values with
 +-0.0, where most decisions are exact ties):
@@ -11,6 +15,7 @@ Per workload (the POS shape of bench.py at each size, and the POS lengths on a t
   bt_fb_ms      backtrace + certification + host round trip + fallback, default bound
   fallback_ms   bt_fb_ms - bt_ms
   flagged       sequences re-decoded in f64
+  fallback_chain  of those, the ones the warp-per-sequence kernel decoded (the rest went to the f64 tile path)
   step_ms       device step as bench.py times it (concurrent backtrace), certified / forced f64
 The forward kernel's bound is its issue rate, not bench.py's FP64 peak (bench.py's roofline.frac still divides by the
 FP64 DADD+DSETP rate): a cell is one FADD2 or FMNMX3 issue slot (two cells each for an add and a max), so at most
@@ -41,7 +46,7 @@ def gpu_info():
         return {"error": repr(e)}
 
 
-def profile(cv, torch, wl, steps):
+def profile(cv, torch, wl, steps, routes=()):
     L = cv._lib.lib()
     K = wl["K"]
     hmm = cv.HMM(wl["A"], wl["B"], np.zeros(K))
@@ -93,6 +98,7 @@ def profile(cv, torch, wl, steps):
         L.cv_debug_set_certified(1)
     r["step_ms"] = step_ms()
     r["flagged"] = int(L.cv_debug_last_flagged(h))
+    r["fallback_chain"] = int(L.cv_debug_last_fallback_chain(h))
     r["paths_equal_f64"] = bool((d_path.cpu().numpy() == ref_p).all())
     r["score_bits_equal_f64"] = d_score.cpu().numpy().tobytes() == ref_s.tobytes()
     r["fwd_ms"], r["bt_fb_ms"] = timed()
@@ -102,6 +108,20 @@ def profile(cv, torch, wl, steps):
     finally:
         L.cv_debug_set_cert_tolerance(1.0)
     r["fallback_ms"] = r["bt_fb_ms"] - r["bt_ms"]
+    if routes:
+        r["route_step_ms"], r["route_fallback_ms"] = {}, {}
+        for rt in routes:
+            route, k = {"tile": (1, 0), "chain": (2, 0)}.get(rt, (3, int(rt) if rt.isdigit() else 0))
+            L.cv_debug_set_fallback(route, k)
+            try:
+                ms = step_ms()
+                same = bool((d_path.cpu().numpy() == ref_p).all()) and d_score.cpu().numpy().tobytes() == ref_s.tobytes()
+                _, bt_fb = timed()
+            finally:
+                L.cv_debug_set_fallback(0, 0)
+            r["route_step_ms"][rt] = ms
+            r["route_fallback_ms"][rt] = bt_fb - r["bt_ms"]
+            r["paths_equal_f64"] = r["paths_equal_f64"] and same
     hmm.close()
     return r
 
@@ -111,6 +131,7 @@ def main():
     ap.add_argument("--nseq", type=int, nargs="+", default=[1_000_000, 125_000])
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--routes", nargs="*", default=[])
     args = ap.parse_args()
     import torch
 
@@ -123,11 +144,11 @@ def main():
     sms = torch.cuda.get_device_properties(0).multi_processor_count
     res = {"gpu": info, "sms": sms, "runs": []}
     for n in args.nseq:
-        res["runs"].append(profile(cv, torch, workload_pos(0, n), args.steps))
+        res["runs"].append(profile(cv, torch, workload_pos(0, n), args.steps, args.routes))
     wl = workload_pos(0, args.nseq[-1])
     wl["A"], wl["B"], _ = random_hmm(np.random.default_rng(3019), wl["K"], wl["M"], ties=True)
     wl["name"] = "pos_lengths_tie_heavy_model"
-    res["runs"].append(profile(cv, torch, wl, args.steps))
+    res["runs"].append(profile(cv, torch, wl, args.steps, args.routes))
     clk = info.get("clocks_max_sm_mhz")
     for r in res["runs"]:
         if clk:
