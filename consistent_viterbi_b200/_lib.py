@@ -52,6 +52,7 @@ SIGNATURES = {
     "cv_hmm_nstates": (C.c_int, [C.c_void_p]),
     "cv_hmm_nobs": (C.c_int64, [C.c_void_p]),
     "cv_decode_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
+    "cv_decode_batch_kbest": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p, C.c_void_p]),
     "cv_decode_batch_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]),
     "cv_decode_batch_dev_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_int64,
                                           C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
@@ -105,6 +106,7 @@ DEBUG_SIGNATURES = {
     "cv_debug_set_large_group_rb": (None, [C.c_longlong]),
     "cv_debug_set_cp_leaf_batch": (None, [C.c_int]),
     "cv_debug_set_fb_chunk_seqs": (None, [C.c_int64]),
+    "cv_debug_set_kbest_chunk_seqs": (None, [C.c_int64]),
     "cv_debug_set_certified": (None, [C.c_int]),
     "cv_debug_set_cert_tolerance": (None, [C.c_double]),
     "cv_debug_last_flagged": (C.c_int64, [C.c_void_p]),

@@ -22,6 +22,7 @@ extern "C" void cv_debug_set_uneven_chunks(int on) { g_tune.uneven_chunks = on; 
 extern "C" void cv_debug_set_large_group_rb(long long rb) { g_tune.large_group_rb = rb; }
 extern "C" void cv_debug_set_cp_leaf_batch(int on) { g_tune.cp_leaf_batch = on; }
 extern "C" void cv_debug_set_fb_chunk_seqs(int64_t n) { g_tune.fb_chunk_seqs = n; }
+extern "C" void cv_debug_set_kbest_chunk_seqs(int64_t n) { g_tune.kbest_chunk_seqs = n; }
 extern "C" void cv_debug_set_certified(int on) { g_tune.certified = on; }
 extern "C" void cv_debug_set_cert_tolerance(double scale) { g_tune.cert_tol = scale; }
 extern "C" int64_t cv_debug_last_flagged(const cv_hmm *h) { return h ? h->last_flagged : -1; }

@@ -58,6 +58,7 @@ struct Tuning {
     int bt_prof = 0, e2e_prof = 0; // print pipeline timelines                                    (CV_BT_PROF, CV_E2E_PROF)
     long long large_group_rb = 0;  // row blocks per group of the large-K kernel, 0 = automatic    (CV_LARGE_GROUP_RB)
     long long fb_chunk_seqs = 0;   // sequences per chunk of cv_loglik_batch / cv_posterior_batch, 0 = automatic (cv_debug_set_fb_chunk_seqs)
+    long long kbest_chunk_seqs = 0; // sequences per chunk of cv_decode_batch_kbest, 0 = automatic (cv_debug_set_kbest_chunk_seqs)
     int cp_fullwarp = 0, cp_prof = 0, cp_sum = -1, cp_hostpoll = 1, cp_leaf_batch = 1;   // constrained solver (CV_CP_*)
     int certified = 1;             // eligible models: f32 forward pass + certified backtrace + exact fallback (cv_debug_set_certified)
     double cert_tol = 1.0;         // scale of the certified backtrace's error bound (cv_debug_set_cert_tolerance)

@@ -67,6 +67,35 @@ def decode_batch_narrow(hmm: HMM, obs_flat, seq_off, device: int = -1):
     return paths, scores
 
 
+def decode_batch_kbest(hmm: HMM, obs_flat, seq_off, k: int, device: int = -1):
+    """The k highest-scoring state paths of every sequence (cv_decode_batch_kbest, contract in include/cv_b200.h).
+
+    obs_flat u32[N], seq_off i64[B+1].  Returns (paths u32[k, N], scores f64[k, B]): row r holds rank r laid out as
+    decode_batch's outputs, and row 0 is decode_batch's result byte for byte.  A sequence of T elements has
+    min(k, K^T) paths; a rank beyond that is "no path": score -inf, every path element 0xFFFFFFFF.  K <= 64, k <= 32."""
+    obs_flat = np.ascontiguousarray(obs_flat, dtype=np.uint32)
+    seq_off = np.ascontiguousarray(seq_off, dtype=np.int64)
+    B, N = seq_off.shape[0] - 1, obs_flat.shape[0]
+    if B > 0 and int(seq_off[-1]) != N:
+        raise ValueError("seq_off[-1] != len(obs_flat)")
+    kk = max(int(k), 0)
+    paths = np.zeros((kk, N), dtype=np.uint32)
+    scores = np.zeros((kk, max(B, 0)), dtype=np.float64)
+    rc = _lib.lib().cv_decode_batch_kbest(hmm.device_handle(device), obs_flat.ctypes.data, seq_off.ctypes.data, B,
+                                          int(k), paths.ctypes.data, scores.ctypes.data)
+    _lib.check(rc)
+    return paths, scores
+
+
+def decode_kbest(sequence, hmm: HMM, k: int, device: int = -1) -> list:
+    """The k best state paths of one sequence as a list of (path u64[T], score), best first; fewer than k when the
+    sequence has fewer than k paths."""
+    obs = hmm.flatten_obs(sequence) if len(sequence) else np.zeros(0, dtype=np.uint32)
+    off = np.array([0, len(obs)], dtype=np.int64)
+    paths, scores = decode_batch_kbest(hmm, obs, off, k, device=device)
+    return [(paths[r].astype(np.uint64), float(scores[r, 0])) for r in range(paths.shape[0]) if paths[r, 0] != 0xFFFFFFFF]
+
+
 def decode(sequence, hmm: HMM, device: int = -1) -> np.ndarray:
     """viterbi::decode(sequence, hmm) -> Array1<usize> (viterbi.rs:5). `sequence` is a
     list of D-dimensional observations (Vec<[usize; D]>)."""

@@ -70,6 +70,34 @@ int64_t cv_hmm_nobs(const cv_hmm *h);          /* M = prod(bdims)               
 int cv_decode_batch(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off,
                     int64_t B, uint32_t *path_out, double *score_out);
 
+/* ---- k-best (list) Viterbi, batched ------------------------------------------
+ * The k highest-scoring state paths of every sequence under the recurrence of cv_decode_batch (pi and o_0 ignored,
+ * every fl one binary64 add).  The score of a path s_0 .. s_{T-1} is the left-to-right rounded sum
+ *   v_0 = 0,  v_t = fl(fl(v_{t-1} + a[s_{t-1}][s_t]) + b[s_t][o_t]),  score = v_{T-1}.
+ * The list at (t, i) holds at most k entries, each a value and a backpointer (j, r).  At t = 0 every state has one
+ * entry, value 0.0.  For t >= 1 the candidates are every entry (j, r) of row t-1, with c = fl(L[t-1][j][r] + a[j][i]):
+ *   - b[i][o_t] > -inf: the first min(k, #candidates) candidates in the order (c descending, j ascending, r ascending),
+ *     compared with IEEE > (-0.0 and +0.0 tie); each entry's value is fl(c + b[i][o_t]);
+ *   - b[i][o_t] = -inf: the first min(k, #candidates) candidates in (j ascending, r ascending) order, every value -inf
+ *     (the psi = 0 rule of the plain decode).
+ * Ranks 0 .. k-1 of a sequence are the first k entries (i, r) of row T-1 in the order (value descending, i ascending,
+ * r ascending), each backtraced through the stored (j, r).  Hence:
+ *   - rank 0 is cv_decode_batch's path and score, byte for byte (fl(x + a) is monotone, so (j, r > 0) never beats
+ *     (j, 0)), including sequences whose every path is -inf and exact ties;
+ *   - every score is its path's rounded sum, scores do not increase with rank, the paths are pairwise distinct, and
+ *     the multiset of the scores is the top k of the scores of all K^T paths;
+ *   - a sequence has min(k, K^T) paths; a rank at or beyond that count is "no path": score -inf and every path
+ *     element 0xFFFFFFFF.
+ *   path_out[k*N]   rank-major: plane r (path_out + r*N) is laid out as cv_decode_batch's path_out
+ *   score_out[k*B]  rank-major: plane r (score_out + r*B) as cv_decode_batch's score_out (may be NULL)
+ * A sequence's outputs do not depend on the batch it is in, its place there or how the call cuts the batch into
+ * chunks; two calls with the same inputs return the same bytes.  Any model cv_hmm_create accepts.
+ *   B = 0: CV_OK, nothing written   CV_ERR_ARG NULL h / obs_flat / seq_off / path_out, seq_off[0] != 0, an observation
+ *   >= M or k < 1 (checked on the host before any launch)   CV_ERR_EMPTY an empty sequence   CV_ERR_UNSUPPORTED K > 64
+ *   or k > 32   CV_ERR_CUDA no device.  HOST pointers, as for cv_decode_batch. */
+int cv_decode_batch_kbest(cv_hmm *h, const uint32_t *obs_flat, const int64_t *seq_off, int64_t B, int k,
+                          uint32_t *path_out /* [k*N] */, double *score_out /* [k*B], may be NULL */);
+
 /* Same call with narrow HOST formats: u16 observations (needs M <= 65536) and u8 states (needs K <= 256; implemented
  * for K <= 64).  A third of the bytes cross PCIe (POS shape: 216 MB -> 75 MB per million sentences); the kernels read
  * and write the narrow types directly.  cv_decode_batch stays the reference-shaped entry. */

@@ -48,6 +48,9 @@ void cv_debug_set_cp_leaf_batch(int on);
 /* cv_loglik_batch / cv_posterior_batch: cut the batch into chunks of n sequences (0 = automatic: chunks whose history
  * and device outputs fit half the free device memory) */
 void cv_debug_set_fb_chunk_seqs(int64_t n);
+/* cv_decode_batch_kbest: cut the batch into chunks of n sequences (0 = automatic: chunks whose backpointers, inputs
+ * and device outputs fit half the free device memory) */
+void cv_debug_set_kbest_chunk_seqs(int64_t n);
 /* exact decode, K <= 64, of a model of log-probabilities (every finite entry of logA / logB <= 0, |x| <= 2^64): 1 (default) =
  * f32 forward pass, backtrace that certifies every backpointer against the f64 recurrence, exact f64 re-decode of the
  * sequences it cannot certify; 0 = the f64 forward pass for every model */
